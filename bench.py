@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the TopoWx interpolation hot path (BASELINE.json metric: interpolated cell-days/sec).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload = BASELINE.json configs[4] (C5): the CONUS 30-arcsec grid (3250 x 7000 cells, synthetic land mask, ~56 % land),
 10 000 synthetic stations per variable, one year (365 days) of daily Tmin+Tmax (12 monthly-normal regression krigings +
@@ -12,6 +12,7 @@ sample of 64 of the 255 tiles that contain land, evenly spaced over the list (TW
 shared counter the way the reference's workers pull chunks from the coordinator rank
 (scripts/step25_mpi_interp_tair.py:293-305); stations are replicated, there is no collective on the data path.
 Prints ONE JSON line on rank 0; secondary figures (configs[1] tile, C3 leave-one-out, C4 normals only) ride in the same line.
+--dump-outputs DIR writes what the last timed step computed, for comparing two builds output for output (OutputDump).
 """
 import argparse
 import ctypes as C
@@ -138,6 +139,44 @@ class ClockSampler(threading.Thread):
                 "reasons": reasons, "samples": len(sm)}
 
 
+DUMP_BYTES = 64 * 10 ** 6
+DUMP_SEED = 2024
+
+
+class OutputDump(object):
+    """--dump-outputs: what twxi_interp_chunk returned for every tile of the last timed step, at a fixed seeded sample of
+    cells (the same row-major cell indices in every tile; as many as fit DUMP_BYTES).  Gathered on the stream right after
+    each tile, before its result buffers are reused.  Files: <key>.npy of shape (tiles in list order, ..., cells), the
+    int16 / uint8 results as float32 and ninvalid as float64 (exact)."""
+    KEYS = ("tmin", "tmax", "tmin_norm", "tmax_norm", "tmin_se", "tmax_se", "ninvalid", "status")
+
+    def __init__(self, ntiles):
+        import torch
+        per_cell = (2 * NDAYS + 4 * 12 + 1) * 4 + 8
+        n = min(TILE * TILE, (DUMP_BYTES - len(self.KEYS) * 4096) // (ntiles * per_cell))
+        cells = np.sort(np.random.default_rng(DUMP_SEED).choice(TILE * TILE, n, replace=False))
+        self.cells = torch.from_numpy(cells).cuda()
+        lead = dict(tmin=(NDAYS,), tmax=(NDAYS,), ninvalid=(), status=())
+        self.buf = {k: torch.zeros((ntiles,) + lead.get(k, (12,)) + (n,), device="cuda",
+                                   dtype=torch.float64 if k == "ninvalid" else torch.float32) for k in self.KEYS}
+
+    def take(self, i, out):
+        for k, b in self.buf.items():
+            v = out[k]
+            b[i] = v.reshape(v.shape[:-2] + (-1,)).index_select(-1, self.cells)
+
+    def save(self, path, world, rank):
+        """Every rank holds the tiles it pulled (zeros elsewhere): a sum over ranks assembles the whole list exactly."""
+        import torch.distributed as dist
+        if world > 1:
+            for b in self.buf.values():
+                dist.all_reduce(b)
+        if rank == 0:
+            os.makedirs(path, exist_ok=True)
+            for k, b in self.buf.items():
+                np.save(os.path.join(path, k + ".npy"), b.cpu().numpy())
+
+
 def sample_cells(wrk, n, seed=7):
     r = np.random.default_rng(seed)
     land = np.nonzero(wrk[2].ravel() != 0)[0]
@@ -261,7 +300,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true")
     ap.add_argument("--cpu-cells", type=int, default=int(os.environ.get("TWX_CPU_CELLS", "2048")))
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a fixed sample of the last timed step's results to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the CUDA path's results; --impl reference has none")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -311,6 +355,7 @@ def main():
                     status=torch.empty((TILE, TILE), dtype=torch.uint8, **kw))
     out_d = [mk(True) for _ in range(2)]
     out_h = [mk(False) for _ in range(3)]       # one set of pinned result buffers per chunk in flight (async contract: 3)
+    dump = OutputDump(NT) if args.dump_outputs else None
     t_setup = time.perf_counter() - t_setup
     puller = Puller(world)
 
@@ -321,16 +366,17 @@ def main():
 
     pass_id = [0]
 
-    def run_pass(kind, nsteps):
+    def run_pass(kind, nsteps, dump=None):
         """nsteps passes over the tile list, tiles pulled from the shared counter.  kind 'resident': device buffers, at
         most two tiles in flight per rank; 'e2e': pinned host buffers through twxi_interp_chunk_async (host->device copy of
-        the next tile and device->host copy of the previous one overlap the kernels; the library lets two run ahead)."""
+        the next tile and device->host copy of the previous one overlap the kernels; the library lets two run ahead).
+        dump (resident only): takes every tile's results of the last pass."""
         ntile = 0
         with torch.cuda.stream(stream):
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record(stream)
             ring = [None, None]
-            for _ in range(nsteps):
+            for step in range(nsteps):
                 key = "p%d" % pass_id[0]
                 pass_id[0] += 1
                 while True:
@@ -342,6 +388,8 @@ def main():
                         if ring[s] is not None:
                             ring[s].synchronize()               # throttle: a rank never holds more than two tiles
                         interp_chunk(ctx[0], ctx[1], wrk_d[i], out=out_d[s])
+                        if dump is not None and step == nsteps - 1:
+                            dump.take(i, out_d[s])
                         ev = torch.cuda.Event()
                         ev.record(stream)
                         ring[s] = ev
@@ -363,7 +411,7 @@ def main():
         sampler.start()
     lib.twxi_launch_count(1)
     t_wall = time.perf_counter()
-    ms_res, nt_res = run_pass("resident", args.steps)
+    ms_res, nt_res = run_pass("resident", args.steps, dump)
     barrier()
     t_wall = time.perf_counter() - t_wall
     launches = int(lib.twxi_launch_count(0))
@@ -382,6 +430,8 @@ def main():
         allst = stats.cpu().numpy()[None, :]
     tot_ms, tot_e2e_ms = float(allst[:, 0].max()), float(allst[:, 1].max())
     launches_all = int(allst[:, 2].sum())
+    if dump is not None:
+        dump.save(args.dump_outputs, world, rank)
 
     # ---- per-kernel rooflines: a separate pass with stage events over the first (full-land) tiles of the list ----------
     nroof = min(4, NT)

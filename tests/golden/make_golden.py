@@ -68,10 +68,12 @@ def main():
             idx_all.append(np.array([stn_da.stn_idxs[x] for x in ids]))
             d_all.append(ss_rm0.ngh_dists.copy()); w_all.append(ss_rm0.ngh_wgt.copy())
             meta.append((st[db.LAT], st[db.LON], nn, s, 1))
-    # obs loading order (station_select.py:184-185 -> DB order)
+    # obs loading order (station_select.py:184-185 -> DB order); the station table's obs are stored for January-August
+    # only (the case reads March), which keeps the file under 1 MB
     ss.set_ngh_stns(pts_lat[0], pts_lon[0], 40, load_obs=True, obs_mth=3)
+    month = np.asarray(stn_da.days[db.MONTH])
     out.update(obs_case_idx=np.array([stn_da.stn_idxs[s] for s in ss.ngh_stns[db.STN_ID]]),
-               obs_case=ss.ngh_obs, obs_all=stn_da.var, month=np.asarray(stn_da.days[db.MONTH]))
+               obs_case=ss.ngh_obs, obs_all=stn_da.var[month <= 8], month=month[month <= 8])
     K = max(len(a) for a in idx_all)
     pad = lambda a, fill: np.array([np.concatenate([x, np.full(K - len(x), fill)]) for x in a])
     out.update(meta=np.array(meta, dtype=np.float64), idx=pad(idx_all, -1).astype(np.int64),

@@ -1,13 +1,11 @@
 """Pin the numpy oracle against golden vectors produced by the reference's own code
 (tests/golden/make_golden.py executes util_geo.py / station_select.py / _gwr_series / tmin_tmax_fixer
-verbatim from /root/reference).  CPU only."""
+verbatim from the original TopoWx sources).  CPU only."""
 import os
 
 import numpy as np
-import pytest
 
 from oracle import twx_oracle as o
-from oracle import ref_loader
 
 
 def _mini_db(g):
@@ -75,22 +73,3 @@ def test_fixer_matches_reference(golden_dir):
         assert n == int(g["ninv%d" % c])
         assert np.array_equal(a, g["otmin%d" % c]) and np.array_equal(b, g["otmax%d" % c])
     assert int(g["ninv0"]) == 0 and int(g["ninv4"]) >= 5
-
-
-@pytest.mark.skipif(not ref_loader.available(), reason="reference tree only exists in the build container")
-def test_oracle_vs_live_reference_station_select():
-    """Belt and braces in the container: random points against the live reference class."""
-    from topowx_b200 import synth, db
-    ref = ref_loader.load()
-    sd = synth.make_station_db(0, 500, synth.tile_bbox(buf=1.0), synth.Fields())
-    good = np.isnan(sd.stns[db.BAD])
-    r_ss = ref.StationSelect(sd, good)
-    o_ss = o.StationSelect(o.StationDb(sd.stns, sd.var, sd.days), good)
-    rng = np.random.default_rng(3)
-    for _ in range(10):
-        la, lo, nn = rng.uniform(39.6, 41.6), rng.uniform(-100, -98), int(rng.integers(35, 148))
-        r_ss.set_ngh_stns(la, lo, nn, load_obs=True, obs_mth=7)
-        o_ss.set_ngh_stns(la, lo, nn, load_obs=True, obs_mth=7)
-        assert np.array_equal(r_ss.ngh_stns[db.STN_ID], o_ss.ngh_stns[db.STN_ID])
-        assert np.array_equal(r_ss.ngh_wgt, o_ss.ngh_wgt)
-        assert np.array_equal(r_ss.ngh_obs, o_ss.ngh_obs)
