@@ -273,6 +273,31 @@ int twxi_interp_chunk_async(twxi_ctx* ctx_tmin, twxi_ctx* ctx_tmax, const double
 int twxi_interp_chunk_wait(twxi_ctx* ctx_tmin, int host_sync);
 
 /*
+ * One work chunk over a long record in day windows (multi-decade records: twxi_interp_chunk holds the chunk's whole
+ * daily record on the device, 12.4 GB per variable for a 250 x 250 tile over 1948-2015).
+ *   twxi_tile_begin  everything of twxi_interp_chunk that does not depend on the day: unpack, kNN, neighbour counts,
+ *                    kriging of the 12 normals and the 12 GWR hat rows of both variables.  Opens a "tile" on the pair
+ *                    (state owned by ctx_tmin: 288 kh + 1 624 bytes per cell, kh = the largest neighbour count;
+ *                    2.75 GB for a 250 x 250 tile at kh = 147; kept for the next tile until the context is destroyed); a new begin discards an open tile.  `mem` is the memory space of
+ *                    wrk_chk.
+ *   twxi_tile_days   the next `ndays` days of the record (windows are consecutive, any length >= 1, chronological):
+ *                    tmin, tmax int16 [ndays][ny][nx], quantised exactly like twxi_interp_chunk.
+ *   twxi_tile_end    after the last day: normals (recomputed from the fixed 1981-2010 dailies when any day was fixed),
+ *                    se, ninvalid and status in the layouts of twxi_interp_chunk.  Closes the tile.
+ * Concatenated in order, the windows' outputs and the end's outputs are byte-identical to twxi_interp_chunk's for every
+ * partition of the record.  The tile shares no workspace with the other entry points, so other calls on the same contexts
+ * may run between windows.  Errors: days / end without an open tile, end before every day was emitted, or either after
+ * twxi_ctx_set_obs on one of the pair -> TWXI_ERR_STATE; more days than remain, or another ctx_tmax than at begin ->
+ * TWXI_ERR_ARG.  With host buffers the call returns once the results are in them; with device buffers after enqueueing.
+ * With twxi_set_stage_timing(1), twxi_get_stage_ms after twxi_tile_days holds the window's GWR apply (slot 3) and fixer /
+ * quantisation (slot 4) times.
+ */
+int twxi_tile_begin(twxi_ctx* ctx_tmin, twxi_ctx* ctx_tmax, const double* wrk_chk, int ny, int nx, int mem);
+int twxi_tile_days(twxi_ctx* ctx_tmin, twxi_ctx* ctx_tmax, int ndays, int16_t* tmin, int16_t* tmax, int mem);
+int twxi_tile_end(twxi_ctx* ctx_tmin, twxi_ctx* ctx_tmax, float* tmin_norm, float* tmax_norm, float* tmin_se,
+                  float* tmax_se, int32_t* ninvalid, uint8_t* status, int mem);
+
+/*
  * Instrumentation for bench.py: number of kernels this library launched on the calling thread's contexts
  * since the last reset, and per-stage device time (ms) of the most recent twxi_interp_chunk /
  * twxi_interp_cells / twxi_interp_points call when timing was enabled (stage order: knn, nngh_params, krig,

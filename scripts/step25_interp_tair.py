@@ -3,6 +3,7 @@
 Gridded interpolation driver: the Python-3 / GPU counterpart of scripts/step25_mpi_interp_tair.py.
 
     python scripts/step25_interp_tair.py --out /tmp/twx_out [--rows 500 --cols 750] [--format nc|raw]
+                                         [--year0 1948 --years 68 --window year]
     torchrun --nproc-per-node N scripts/step25_interp_tair.py ...     (one process per GPU)
 
 The reference runs an MPI task farm: rank 0 reads every 50x50 work chunk's 27 predictor windows from netCDF and hands it
@@ -13,6 +14,10 @@ background thread reads each tile's windows once into pinned memory (TileFeed), 
 PtInterpTair.interp_chunk(wait=False) = twxi_interp_chunk_async with three sets of pinned result buffers in flight, and a
 writer pool writes the reference's netCDF tiles (TileWriter; raw .npy with --format raw).  Without rasters at --rasters a
 synthetic window of the CONUS grid is generated first (topowx_b200.synth).
+The synthetic station record covers --years calendar years from --year0.  --window record (default) computes each tile's
+whole record in one call; --window year goes through PtInterpTair.interp_chunk_stream instead: kriging and GWR hat rows
+once per tile, then one calendar year at a time, so a multi-decade record never sits whole on the device or in pinned
+memory.  Each year is written as it comes (TileWriter.open_tile_stream; --format raw: one .npy per year window).
 '''
 import argparse
 import os
@@ -25,7 +30,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 
 from topowx_b200 import synth                                     # noqa: E402
 from topowx_b200.interp import (PtInterpTair, Tiler, partition_chunks, PredictorStore, TileFeed,     # noqa: E402
-                                AsyncTileWriter)
+                                AsyncTileWriter, TileWriter)
 
 P_TILESIZE = 250                                                  # step25_mpi_interp_tair.py:349-352
 
@@ -40,6 +45,10 @@ def main():
     ap.add_argument("--cols", type=int, default=2 * P_TILESIZE)
     ap.add_argument("--nstns", type=int, default=4000)
     ap.add_argument("--format", default="nc", choices=["nc", "raw"])
+    ap.add_argument("--year0", type=int, default=1995, help="first year of the synthetic station record")
+    ap.add_argument("--years", type=int, default=1, help="calendar years of the synthetic station record")
+    ap.add_argument("--window", default="record", choices=["record", "year"],
+                    help="whole record per tile in one call, or one calendar year at a time")
     args = ap.parse_args()
     import torch
     rank = int(os.environ.get("RANK", "0"))
@@ -48,7 +57,7 @@ def main():
     torch.cuda.set_device(local_rank)
 
     f = synth.Fields()
-    days = synth.make_days(1995, 1)
+    days = synth.make_days(args.year0, args.years)
     rpath = args.rasters or os.path.join(args.out, "rasters")
     if not os.path.exists(os.path.join(rpath, "mask.npy")):
         if rank == 0:
@@ -66,6 +75,9 @@ def main():
 
     mine = partition_chunks(tiler.tile_chks, tiler.mask, P_TILESIZE, P_TILESIZE, world, rank)
     nd = days.size
+    if args.window == "year":
+        return by_year(args, pt_interp, TileFeed(tiler, chunks=mine, depth=4), TileWriter(info, args.out), days, rank, world,
+                       len(mine))
     pin = lambda shape, dt: torch.empty(shape, dtype=dt).pin_memory()
     outs = [dict(tmin=pin((nd, P_TILESIZE, P_TILESIZE), torch.int16), tmax=pin((nd, P_TILESIZE, P_TILESIZE), torch.int16),
                  tmin_norm=pin((12, P_TILESIZE, P_TILESIZE), torch.float32), tmax_norm=pin((12, P_TILESIZE, P_TILESIZE), torch.float32),
@@ -99,6 +111,37 @@ def main():
           "tiles on disk (%.1f MB)" % (rank, world, len(mine), ncells, nd, dt, ncells * nd / max(dt, 1e-9),
                                        feed.bytes_read / 1e6, writer.tw.format if args.format == "nc" else "raw .npy",
                                        nbytes / 1e6))
+
+
+def by_year(args, pt_interp, feed, tw, days, rank, world, ntiles):
+    t0 = time.time()
+    ncells, nbytes = 0, 0
+    for k, tid, wrk in feed:
+        s = pt_interp.interp_chunk_stream(wrk)
+        d = os.path.join(args.out, tid)
+        os.makedirs(d, exist_ok=True)
+        hs = {v: tw.open_tile_stream(tid, v, days) for v in ("tmin", "tmax")} if args.format == "nc" else None
+        for d0, o in s.years():
+            for v in ("tmin", "tmax"):
+                if hs:
+                    hs[v].write_days(d0, o[v])
+                else:
+                    np.save(os.path.join(d, "%s_%s_%05d.npy" % (tid, v, d0)), o[v])
+                    nbytes += o[v].nbytes
+        fin = s.finish()
+        for v in ("tmin", "tmax"):
+            if hs:
+                hs[v].close(fin[v + "_norm"], fin[v + "_se"], fin["ninvalid"])
+                nbytes += os.path.getsize(tw._fpath(tid, v))
+        if not hs:
+            for key, a in fin.items():
+                np.save(os.path.join(d, "%s_%s.npy" % (tid, key)), a)
+                nbytes += a.nbytes
+        ncells += int((fin["status"] == 0).sum())
+    dt = time.time() - t0
+    print("rank %d/%d: %d tiles, %d cells x %d days in %.2f s = %.3g cell-days/s in year windows to %s tiles on disk "
+          "(%.1f MB)" % (rank, world, ntiles, ncells, days.size, dt, ncells * days.size / max(dt, 1e-9),
+                         tw.format if args.format == "nc" else "raw .npy", nbytes / 1e6))
 
 
 if __name__ == "__main__":

@@ -16,7 +16,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libtwxi.so")
-SOURCES = ["api.cu", "knn.cu", "setup.cu", "ked.cu", "gwr.cu", "fixer.cu", "peak.cu", "vario.cu", "xval.cu"]
+SOURCES = ["api.cu", "knn.cu", "setup.cu", "ked.cu", "gwr.cu", "fixer.cu", "peak.cu", "vario.cu", "xval.cu", "record.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-O2"]          # never fast-math: FP64 parity
 

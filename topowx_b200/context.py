@@ -292,3 +292,71 @@ def interp_chunk(ctx_tmin, ctx_tmax, wrk_chk, out=None, daily=True, wait=True):
 def interp_chunk_wait(ctx_tmin, host_sync=True):
     """Completion of the chunks submitted with ``interp_chunk(..., wait=False)`` (twxi_interp_chunk_wait)."""
     check(lib.twxi_interp_chunk_wait(ctx_tmin.handle, 1 if host_sync else 0))
+
+
+def _check_wrk_chk(wrk_chk):
+    if len(wrk_chk.shape) != 3 or wrk_chk.shape[0] != 32:
+        raise ValueError("wrk_chk must be [32, ny, nx] (planes of tiling.py:205-213 / step25:273-279), got %r"
+                         % (tuple(wrk_chk.shape),))
+    if _dtype_name(wrk_chk) != "float64":
+        raise ValueError("wrk_chk must be float64, got %s" % _dtype_name(wrk_chk))
+    return int(wrk_chk.shape[1]), int(wrk_chk.shape[2])
+
+
+def _result_buffers(want, out, device):
+    """Result buffers {name: (dtype, shape)}: allocated when ``out`` is None (numpy on the host, or torch tensors on the CUDA
+    ``device``), otherwise checked like interp_chunk's (dtype, shape, one memory space).  Returns (buffers, on_device)."""
+    if out is None:
+        if device is None:
+            return {k: np.empty(shp, dtype=dt) for k, (dt, shp) in want.items()}, False
+        import torch
+        return {k: torch.empty(shp, dtype=getattr(torch, dt), device=device) for k, (dt, shp) in want.items()}, True
+    dev = None
+    for k, (dt, shp) in want.items():
+        b = out.get(k)
+        if b is None:
+            raise ValueError("out[%r] is missing" % k)
+        if _dtype_name(b) != dt or tuple(b.shape) != shp:
+            raise ValueError("out[%r] must be %s %r, got %s %r" % (k, dt, shp, _dtype_name(b), tuple(b.shape)))
+        if dev is None:
+            dev = _lib.is_device(b)
+        elif _lib.is_device(b) != dev:
+            raise ValueError("out[%r] must live in the same memory space as the other result buffers" % k)
+    return out, dev
+
+
+def tile_begin(ctx_tmin, ctx_tmax, wrk_chk):
+    """twxi_tile_begin: everything of interp_chunk that does not depend on the day (kNN, neighbour counts, kriging, GWR hat
+    rows) for the work chunk ``wrk_chk`` f8[32, ny, nx]; opens a tile on the context pair.  Returns (ny, nx)."""
+    ny, nx = _check_wrk_chk(wrk_chk)
+    if ctx_tmin.ndays != ctx_tmax.ndays:
+        raise ValueError("tmin and tmax contexts hold observation records of different length")
+    check(lib.twxi_tile_begin(ctx_tmin.handle, ctx_tmax.handle, ptr(wrk_chk), ny, nx,
+                              MEM_DEVICE if _lib.is_device(wrk_chk) else MEM_HOST))
+    return ny, nx
+
+
+def tile_days(ctx_tmin, ctx_tmax, ndays, shape, out=None, device=None):
+    """twxi_tile_days: the next ``ndays`` days of the open tile of ``shape`` = (ny, nx) -> {tmin, tmax} int16
+    [ndays, ny, nx], byte-identical to the same days of interp_chunk.  ``out`` may carry the two buffers; otherwise they are
+    allocated on the host, or on the CUDA ``device`` (a torch device) when given."""
+    ny, nx = shape
+    want = dict(tmin=("int16", (int(ndays), ny, nx)), tmax=("int16", (int(ndays), ny, nx)))
+    out, dev = _result_buffers(want, out, device)
+    check(lib.twxi_tile_days(ctx_tmin.handle, ctx_tmax.handle, int(ndays), ptr(out["tmin"]), ptr(out["tmax"]),
+                             MEM_DEVICE if dev else MEM_HOST))
+    return out
+
+
+def tile_end(ctx_tmin, ctx_tmax, shape, out=None, device=None):
+    """twxi_tile_end after the last day: {tmin_norm, tmax_norm, tmin_se, tmax_se, ninvalid, status} of interp_chunk
+    (normals recomputed from the fixed 1981-2010 dailies when a day was fixed); closes the tile."""
+    ny, nx = shape
+    want = dict(tmin_norm=("float32", (12, ny, nx)), tmax_norm=("float32", (12, ny, nx)),
+                tmin_se=("float32", (12, ny, nx)), tmax_se=("float32", (12, ny, nx)),
+                ninvalid=("int32", (ny, nx)), status=("uint8", (ny, nx)))
+    out, dev = _result_buffers(want, out, device)
+    check(lib.twxi_tile_end(ctx_tmin.handle, ctx_tmax.handle, ptr(out["tmin_norm"]), ptr(out["tmax_norm"]),
+                            ptr(out["tmin_se"]), ptr(out["tmax_se"]), ptr(out["ninvalid"]), ptr(out["status"]),
+                            MEM_DEVICE if dev else MEM_HOST))
+    return out

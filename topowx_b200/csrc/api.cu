@@ -203,6 +203,24 @@ static int copy_out_on(cudaStream_t s, T* dst, const T* src, size_t count) {
     return TWXI_OK;
 }
 
+// Lay out the per-tile arrays of TileState in one allocation (256-byte aligned pieces).
+static int tile_alloc(TileState& t) {
+    const size_t nc = (size_t)t.ncell, nh = (size_t)2 * nc * 12 * t.kh;
+    const size_t sizes[] = {2 * nc * 12 * 4, nh * 4, nh * 8, 2 * nc * 12 * 8, 2 * nc * 12 * 8, 2 * nc * 12 * 8, nc * 4,
+                            nc * 4, 2 * nc * 15 * 8, 2 * nc * 32 * 8, 2 * nc * 12 * 8};
+    size_t off[11], tot = 0;
+    for (int i = 0; i < 11; ++i) { off[i] = tot; tot += (sizes[i] + 255) & ~(size_t)255; }
+    char* p;
+    TWXI_TRY(t.fixed.get((void**)&p, tot));
+    t.hk = reinterpret_cast<int32_t*>(p + off[0]); t.hidx = reinterpret_cast<int32_t*>(p + off[1]);
+    t.hz = reinterpret_cast<double*>(p + off[2]); t.hoff = reinterpret_cast<double*>(p + off[3]);
+    t.mean = reinterpret_cast<double*>(p + off[4]); t.var = reinterpret_cast<double*>(p + off[5]);
+    t.status = reinterpret_cast<int32_t*>(p + off[6]); t.ninv = reinterpret_cast<int32_t*>(p + off[7]);
+    t.carry = reinterpret_cast<double*>(p + off[8]); t.gpart = reinterpret_cast<double*>(p + off[9]);
+    t.gacc = reinterpret_cast<double*>(p + off[10]);
+    return TWXI_OK;
+}
+
 static bool is_device_ptr(const void* p) {
     cudaPointerAttributes at;
     if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { cudaGetLastError(); return false; }
@@ -356,6 +374,7 @@ int twxi_ctx_destroy(twxi_ctx* c) {
     free_batch(c->b);
     for (auto& sc : c->scratch) sc.release();
     c->async.destroy();
+    c->tile.release();
     ked_work_free(c->ked);
     knn_work_free(c->knn);
     delete c;
@@ -398,6 +417,7 @@ int twxi_ctx_set_obs(twxi_ctx* c, const float* obs, int ndays, const int32_t* mo
     for (void* p : c->obs_owned) cudaFree(p);
     c->obs_owned.clear();
     c->has_obs = false;
+    ++c->obs_gen;
     const int n = c->n;
     ObsTable& ob = c->ob;
     ob.ndays = ndays;
@@ -443,6 +463,9 @@ int twxi_ctx_set_obs(twxi_ctx* c, const float* obs, int ndays, const int32_t* mo
     TWXI_TRY(dev_upload(*c, c->obs_owned, &d_gl, glen.data(), glen.size()));
     TWXI_CUDA(cudaStreamSynchronize(c->stream));
     ob.obsT = d_obsT; ob.day_of_pos = d_dop; ob.grp_start = d_gs; ob.grp_len = d_gl;
+    c->h_day_of_pos = std::move(day_of_pos);
+    c->h_grp_start = std::move(gstart);
+    c->h_grp_len = std::move(glen);
     c->has_obs = true;
     return TWXI_OK;
 }
@@ -950,6 +973,185 @@ int twxi_interp_chunk_async(twxi_ctx* cmin, twxi_ctx* cmax, const double* wrk_ch
                             int32_t* ninvalid, uint8_t* status, int mem) {
     return interp_chunk_impl(cmin, cmax, wrk_chk, ny, nx, tmin, tmax, tmin_norm, tmax_norm, tmin_se, tmax_se, ninvalid,
                              status, mem, true);
+}
+
+static int tile_begin_impl(twxi_ctx* cmin, twxi_ctx* cmax, const double* wrk_chk, int ny, int nx, int mem) {
+    const int ncell = ny * nx;
+    TWXI_TRY(ensure_batch(*cmin, ncell, default_k1(*cmin), false));
+    TWXI_TRY(ensure_batch(*cmax, ncell, default_k1(*cmax), false));
+    Ctx* cs[2] = {cmin, cmax};
+    for (Ctx* c : cs) {
+        c->b.n_rm = 0; c->b.rm_zero = 0;
+        c->b.gy = ny; c->b.gx = nx;
+    }
+    const double* d_wrk = wrk_chk;
+    if (mem != TWXI_MEM_DEVICE) {
+        double* w;
+        const size_t wrk_bytes = (size_t)32 * ncell * 8;
+        TWXI_TRY(cmin->scratch[2].get((void**)&w, wrk_bytes));
+        TWXI_CUDA(cudaMemcpyAsync(w, wrk_chk, wrk_bytes, cudaMemcpyHostToDevice, cmin->stream));
+        d_wrk = w;
+    }
+    TileState& t = cmin->tile;
+    t.ny = ny; t.nx = nx; t.ncell = ncell;
+    t.kh = std::max(cmin->b.k1, cmax->b.k1) - 1;              // k_anom < k1 of its context
+    TWXI_TRY(tile_alloc(t));
+    StageTimer tm[2];
+    tm[0].begin(cmin->stream);
+    TWXI_TRY(launch_unpack_chunk(cmin->stream, d_wrk, ny, nx, cmin->climdivs, cmin->n_climdivs, cmax->climdivs,
+                                 cmax->n_climdivs, cmin->b, cmax->b));
+    for (int v = 0; v < 2; ++v) {                             // run_variable with hat rows instead of the daily apply
+        Ctx& c = *cs[v];
+        if (v) tm[1].begin(cmin->stream);
+        TWXI_TRY(run_knn(c));
+        tm[v].mark(1);
+        TWXI_TRY(launch_nngh_params(c, c.b, nullptr, nullptr, 0, 1, 1, 1));
+        tm[v].mark(2);
+        TWXI_TRY(launch_krig(c, c.b, 0, nullptr));
+        tm[v].mark(3);
+        const size_t n12 = (size_t)v * ncell * 12;
+        TWXI_TRY(launch_gwr_hat_rows(c, c.b, t.kh, t.hk + n12, t.hidx + n12 * t.kh, t.hz + n12 * t.kh, t.hoff + n12));
+        tm[v].mark(4);
+        if (v) TWXI_TRY(launch_tile_init(cmin->stream, t, cmin->b, cmax->b));
+        tm[v].mark(5);
+    }
+    tm[0].end(false);
+    tm[1].end(true);
+    t.cmax = cmax;
+    t.gen_min = cmin->obs_gen; t.gen_max = cmax->obs_gen;
+    t.ndays = cmin->ob.ndays;
+    t.next_day = 0;
+    TWXI_TRY(finish(*cmin, mem));
+    t.open = true;
+    return TWXI_OK;
+}
+
+// The calls after begin: an open tile of this pair whose observation records have not been replaced since.
+static int tile_check(twxi_ctx* cmin, twxi_ctx* cmax) {
+    TWXI_ARG(cmin && cmax, "null ctx");
+    const TileState& t = cmin->tile;
+    if (!t.open) { set_error("no open tile on this context pair (twxi_tile_begin)"); return TWXI_ERR_STATE; }
+    TWXI_ARG(t.cmax == cmax, "ctx_tmax differs from the one the tile was begun with");
+    if (!cmin->has_obs || !cmax->has_obs || cmin->obs_gen != t.gen_min || cmax->obs_gen != t.gen_max) {
+        set_error("the observation record was replaced after twxi_tile_begin");
+        return TWXI_ERR_STATE;
+    }
+    return TWXI_OK;
+}
+
+// Month-major positions of the days [d0, d1) of month m: one contiguous run, days of a month are chronological.
+static void month_positions(const Ctx& c, int m, int d0, int d1, int* p0, int* cnt) {
+    const int* b = c.h_day_of_pos.data() + c.ob.moff[m];
+    const int* e = c.h_day_of_pos.data() + c.ob.moff[m + 1];
+    const int* lo = std::lower_bound(b, e, d0);
+    const int* hi = std::lower_bound(lo, e, d1);
+    *p0 = (int)(lo - c.h_day_of_pos.data());
+    *cnt = (int)(hi - lo);
+}
+
+static int tile_days_impl(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, int16_t* tmin, int16_t* tmax, int mem) {
+    TileState& t = cmin->tile;
+    WindowSpan w;
+    w.w0 = t.next_day; w.nwin = ndays;
+    const int w1 = w.w0 + ndays;
+    w.la = std::min(15, t.ndays - w1);
+    const Ctx* cs[2] = {cmin, cmax};
+    for (int v = 0; v < 2; ++v)
+        for (int m = 0; m < 12; ++m) month_positions(*cs[v], m, w.w0, w1 + w.la, &w.p0[v][m], &w.cnt[v][m]);
+    w.g0 = w.g1 = 0;
+    for (int g = 0; g < cmin->ob.ngroups; ++g) {
+        const int gs = cmin->h_grp_start[g], len = cmin->h_grp_len[g];
+        if (len == 0 || gs >= w1 || gs + len <= w.w0) continue;
+        if (w.g0 == w.g1) w.g0 = g;
+        w.g1 = g + 1;
+    }
+    const size_t nq = (size_t)ndays * t.ncell;
+    int16_t *d_qmin = tmin, *d_qmax = tmax;
+    if (mem != TWXI_MEM_DEVICE) {
+        TWXI_TRY(t.out.get((void**)&d_qmin, 2 * nq * 2));
+        d_qmax = d_qmin + nq;
+    }
+    cudaEvent_t ev[3];
+    const bool timing = stage_timing_on();
+    if (timing) {
+        for (auto& e : ev) cudaEventCreate(&e);
+        cudaEventRecord(ev[0], cmin->stream);
+    }
+    TWXI_TRY(launch_tile_window(cmin->stream, t, *cmin, *cmax, w, d_qmin, d_qmax, timing ? ev[1] : nullptr));
+    if (timing) {                                             // stage slots 3 (GWR daily apply) and 4 (fixer / quantise)
+        cudaEventRecord(ev[2], cmin->stream);
+        cudaEventSynchronize(ev[2]);
+        g_stage_ms[0] = g_stage_ms[1] = g_stage_ms[2] = 0.0f;
+        cudaEventElapsedTime(&g_stage_ms[3], ev[0], ev[1]);
+        cudaEventElapsedTime(&g_stage_ms[4], ev[1], ev[2]);
+        for (auto& e : ev) cudaEventDestroy(e);
+    }
+    if (mem != TWXI_MEM_DEVICE) {
+        TWXI_TRY(copy_out(*cmin, tmin, d_qmin, nq));
+        TWXI_TRY(copy_out(*cmin, tmax, d_qmax, nq));
+    }
+    t.next_day = w1;
+    return finish(*cmin, mem);
+}
+
+static int tile_end_impl(twxi_ctx* cmin, float* tmin_norm, float* tmax_norm, float* tmin_se, float* tmax_se,
+                         int32_t* ninvalid, uint8_t* status, int mem) {
+    TileState& t = cmin->tile;
+    const size_t nc = (size_t)t.ncell, f = 12 * nc;
+    float *d_fnmin = tmin_norm, *d_fnmax = tmax_norm, *d_fsemin = tmin_se, *d_fsemax = tmax_se;
+    int32_t* d_ninv = ninvalid;
+    uint8_t* d_st = status;
+    if (mem != TWXI_MEM_DEVICE) {
+        char* o;
+        TWXI_TRY(t.out.get((void**)&o, 4 * f * 4 + nc * 5));
+        d_fnmin = reinterpret_cast<float*>(o); d_fnmax = d_fnmin + f; d_fsemin = d_fnmax + f; d_fsemax = d_fsemin + f;
+        d_ninv = reinterpret_cast<int32_t*>(d_fsemax + f);
+        d_st = reinterpret_cast<uint8_t*>(d_ninv + nc);
+    }
+    TWXI_TRY(launch_tile_end(cmin->stream, t, *cmin, d_fnmin, d_fnmax, d_fsemin, d_fsemax, d_ninv, d_st));
+    if (mem != TWXI_MEM_DEVICE) {
+        TWXI_TRY(copy_out(*cmin, tmin_norm, d_fnmin, f));
+        TWXI_TRY(copy_out(*cmin, tmax_norm, d_fnmax, f));
+        TWXI_TRY(copy_out(*cmin, tmin_se, d_fsemin, f));
+        TWXI_TRY(copy_out(*cmin, tmax_se, d_fsemax, f));
+        TWXI_TRY(copy_out(*cmin, ninvalid, d_ninv, nc));
+        TWXI_TRY(copy_out(*cmin, status, d_st, nc));
+    }
+    t.open = false;
+    return finish(*cmin, mem);
+}
+
+int twxi_tile_begin(twxi_ctx* cmin, twxi_ctx* cmax, const double* wrk_chk, int ny, int nx, int mem) {
+    TWXI_ARG(wrk_chk, "null argument");
+    TWXI_ARG(ny >= 1 && nx >= 1 && (long long)ny * nx <= (1 << 24), "bad chunk size");
+    TWXI_TRY(check_pair(cmin, cmax, true));
+    TWXI_CUDA(cudaSetDevice(cmin->device));
+    cmin->tile.open = false;                                  // a new begin discards an open tile
+    cudaStream_t saved = cmax->stream;
+    cmax->stream = cmin->stream;
+    const int rc = tile_begin_impl(cmin, cmax, wrk_chk, ny, nx, mem);
+    cmax->stream = saved;
+    return rc;
+}
+
+int twxi_tile_days(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, int16_t* tmin, int16_t* tmax, int mem) {
+    TWXI_TRY(tile_check(cmin, cmax));
+    TWXI_ARG(tmin && tmax, "null argument");
+    TWXI_ARG(ndays >= 1 && ndays <= cmin->tile.ndays - cmin->tile.next_day, "ndays must be 1 .. the days that remain");
+    TWXI_CUDA(cudaSetDevice(cmin->device));
+    return tile_days_impl(cmin, cmax, ndays, tmin, tmax, mem);
+}
+
+int twxi_tile_end(twxi_ctx* cmin, twxi_ctx* cmax, float* tmin_norm, float* tmax_norm, float* tmin_se, float* tmax_se,
+                  int32_t* ninvalid, uint8_t* status, int mem) {
+    TWXI_TRY(tile_check(cmin, cmax));
+    TWXI_ARG(tmin_norm && tmax_norm && tmin_se && tmax_se && ninvalid && status, "null argument");
+    if (cmin->tile.next_day != cmin->tile.ndays) {
+        set_error("twxi_tile_end before every day of the record was emitted");
+        return TWXI_ERR_STATE;
+    }
+    TWXI_CUDA(cudaSetDevice(cmin->device));
+    return tile_end_impl(cmin, tmin_norm, tmax_norm, tmin_se, tmax_se, ninvalid, status, mem);
 }
 
 int twxi_interp_chunk_wait(twxi_ctx* cmin, int host_sync) {

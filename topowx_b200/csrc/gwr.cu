@@ -50,9 +50,13 @@ struct GwrArgs {
     const int32_t* xv_self;    // [npts] station index of the point, or null
     double* xv_out;            // [npts][xv_nc][12][3]
     int xv_nc, xv_ci;
+    double* hat_off;           // HAT instance: [npts][12] pt_norm - z . norm
 };
 
-template <bool XVAL, bool PACKED>
+// HAT: hat rows of every (point, month) to hat_k / hat_off [npts][12] and hat_idx / hat_z [npts][12][kmax], no daily
+// values (the day windows of twxi_tile_days apply them).  A separate instance, so that the production kernel carries no
+// branch for it: z and the offset are bitwise what the production instance applies to the days.
+template <bool XVAL, bool PACKED, bool HAT = false>
 __global__ void __launch_bounds__(GWR_THREADS, TWXI_GWR_MINB) gwr_kernel(GwrArgs a) {
     __shared__ __align__(16) double s_z[GWR_WARPS][GWR_MAXK];
     __shared__ __align__(16) int s_off[GWR_WARPS][GWR_MAXK];                // station * ndays: row offset into obsT
@@ -166,12 +170,24 @@ __global__ void __launch_bounds__(GWR_THREADS, TWXI_GWR_MINB) gwr_kernel(GwrArgs
         s_z[warp][j] = zj;
         s_off[warp][j] = s * (int)nd;
         zn += zj * nrm;
-        if (a.hat_z && j < a.kmax) {                          // (device-resident overrides are not scanned on the host)
+        if constexpr (HAT) {
+            const size_t o = ((size_t)q * 12 + m) * a.kmax + j;
+            a.hat_z[o] = zj;
+            a.hat_idx[o] = s;
+        } else if (a.hat_z && j < a.kmax) {                   // (device-resident overrides are not scanned on the host)
             a.hat_z[(size_t)q * a.kmax + j] = zj;
             a.hat_idx[(size_t)q * a.kmax + j] = s;
         }
     }
     zn = warp_sum(zn);
+    if constexpr (HAT) {
+        if (lane == 0) {
+            const double ptn = a.pt_norm[(size_t)q * 12 + m];
+            a.hat_k[(size_t)q * 12 + m] = k;
+            a.hat_off[(size_t)q * 12 + m] = ptn - zn;
+        }
+        return;
+    }
     if (a.hat_k && lane == 0) a.hat_k[q] = k;
     __syncwarp();
     if (!XVAL && !a.daily && !a.out_month) return;
@@ -268,7 +284,7 @@ static void gwr_fill(GwrArgs& a, Ctx& c, Batch& b, int mth) {
     a.qlon = b.lon; a.qlat = b.lat; a.qelev = b.elev; a.qtdi = b.tdi; a.qlst = b.lst;
     a.pt_norm = b.mean; a.pt_norm_single = 0; a.daily = nullptr; a.out_month = nullptr;
     a.kmax = 0; a.hat_k = nullptr; a.hat_idx = nullptr; a.hat_z = nullptr; a.status = b.status;
-    a.k_fixed = 0; a.xv_self = nullptr; a.xv_out = nullptr; a.xv_nc = 0; a.xv_ci = 0;
+    a.k_fixed = 0; a.xv_self = nullptr; a.xv_out = nullptr; a.xv_nc = 0; a.xv_ci = 0; a.hat_off = nullptr;
 }
 
 int launch_gwr(Ctx& c, Batch& b, int mth, const double* pt_norm_override, int write_daily, double* out_month,
@@ -289,6 +305,19 @@ int launch_gwr(Ctx& c, Batch& b, int mth, const double* pt_norm_override, int wr
     const unsigned grid = (unsigned)((items + GWR_WARPS - 1) / GWR_WARPS);
     if (a.st.n > TWXI_GWR_PACKED_MIN_N) gwr_kernel<false, true><<<grid, GWR_THREADS, 0, c.stream>>>(a);
     else gwr_kernel<false, false><<<grid, GWR_THREADS, 0, c.stream>>>(a);
+    TWXI_LAUNCH_CHECK();
+    return TWXI_OK;
+}
+
+int launch_gwr_hat_rows(Ctx& c, Batch& b, int kh, int32_t* hk, int32_t* hidx, double* hz, double* hoff) {
+    if (b.npts <= 0) return TWXI_OK;
+    GwrArgs a;
+    gwr_fill(a, c, b, 0);
+    a.kmax = kh; a.hat_k = hk; a.hat_idx = hidx; a.hat_z = hz; a.hat_off = hoff;
+    const long long items = (long long)b.npts * 12;
+    const unsigned grid = (unsigned)((items + GWR_WARPS - 1) / GWR_WARPS);
+    if (a.st.n > TWXI_GWR_PACKED_MIN_N) gwr_kernel<false, true, true><<<grid, GWR_THREADS, 0, c.stream>>>(a);
+    else gwr_kernel<false, false, true><<<grid, GWR_THREADS, 0, c.stream>>>(a);
     TWXI_LAUNCH_CHECK();
     return TWXI_OK;
 }

@@ -135,11 +135,35 @@ struct AsyncOut {
     void destroy();
 };
 
+struct Ctx;
+
+// A work chunk interpolated over its record in day windows (twxi_tile_begin / _days / _end), owned by the tmin context of
+// the pair.  Everything the windows need is copied here at begin, so other calls on the same contexts (which reuse Batch)
+// may run between windows.  Per-variable arrays are [2][...]: tmin, then tmax.
+struct TileState {
+    bool open = false;
+    const Ctx* cmax = nullptr;
+    long long gen_min = 0, gen_max = 0;  // obs generations of the pair at begin: twxi_ctx_set_obs invalidates the tile
+    int ny = 0, nx = 0, ncell = 0, kh = 0, ndays = 0, next_day = 0;
+    int32_t* hk = nullptr;     // [2][ncell][12] k_anom
+    int32_t* hidx = nullptr;   // [2][ncell][12][kh] neighbour station indices (distance order)
+    double* hz = nullptr;      // [2][ncell][12][kh] hat row z in neighbour order
+    double* hoff = nullptr;    // [2][ncell][12] pt_norm - z . norm
+    double* mean = nullptr;    // [2][ncell][12] kriged normals
+    double* var = nullptr;     // [2][ncell][12] kriging variances
+    int32_t* status = nullptr; // [ncell] status of the pair (TWXI_ST_FIXER_EMPTY is set by the first window)
+    int32_t* ninv = nullptr;   // [ncell] running count of Tmin >= Tmax days
+    double* carry = nullptr;   // [2][ncell][15] the last 15 fixed dailies before the next window
+    double* gpart = nullptr;   // [2][ncell][32] per-lane partial sums of the open 1981-2010 (year, month) group
+    double* gacc = nullptr;    // [2][ncell][12] running sums over years of the group means
+    Scratch fixed, win, out;   // the arrays above; window dailies [2][ncell][15 + nwin + 15]; host-bound staging
+    void release() { fixed.release(); win.release(); out.release(); *this = TileState(); }
+};
+
 struct KedWork;                  // ked.cu: device scratch + launch configuration of the kriging stage
 struct KnnWork;                  // knn.cu: candidate lists of the gridded search
 void ked_work_free(KedWork*);
 void knn_work_free(KnnWork*);
-struct Ctx;
 int knn_mean_candidates(Ctx& c, double* out);
 
 struct Ctx {
@@ -150,7 +174,10 @@ struct Ctx {
     StnTable st{};
     ObsTable ob{};
     bool has_obs = false;
+    long long obs_gen = 0;         // number of twxi_ctx_set_obs calls
     std::vector<void*> obs_owned;
+    std::vector<int> h_day_of_pos; // host copies of ob.day_of_pos / grp_start / grp_len (window position ranges)
+    std::vector<int> h_grp_start, h_grp_len;
     double* climdivs = nullptr;
     int n_climdivs = -1;           // -1: no check
     Batch b;
@@ -158,6 +185,7 @@ struct Ctx {
     // device workspaces: owned by the context (one device, one stream), never shared between contexts
     Scratch scratch[5];
     AsyncOut async;
+    TileState tile;
     KedWork* ked = nullptr;
     KnnWork* knn = nullptr;
 };
@@ -171,6 +199,8 @@ int launch_krig(Ctx& c, Batch& b, int mth, const double* vario_override);
 int launch_vario_fit(Ctx& c, Batch& b, int mth);
 int launch_gwr(Ctx& c, Batch& b, int mth, const double* pt_norm_override, int write_daily,
                double* out_month, int kmax, int32_t* hat_k, int32_t* hat_idx, double* hat_z);
+// hat rows of all 12 months with the arithmetic of launch_gwr: [ncell][12] k and offset, [ncell][12][kh] indices and z
+int launch_gwr_hat_rows(Ctx& c, Batch& b, int kh, int32_t* hk, int32_t* hidx, double* hz, double* hoff);
 int launch_gwr_xval(Ctx& c, Batch& b, const int32_t* self, const int32_t* counts_host, int ncounts, double* out);
 int launch_station_points(Ctx& c, Batch& b, int npts, const int32_t* sidx);
 int launch_split3(cudaStream_t s, size_t n, const double* src, const int32_t* status, int per_point, double* a, double* b,
@@ -188,6 +218,17 @@ int launch_fixer(Ctx& cmin, Ctx& cmax, int ncells, int fix_invalid, int have_dai
                  int32_t* ninvalid);
 int launch_finalize_points(Ctx& c, Batch& b, double* daily, double* norms, double* se, double* var_out,
                            uint8_t* status);
+// record.cu: the day windows of an open tile (TileState)
+struct WindowSpan {
+    int w0, nwin, la;          // first day, window length, look-ahead days computed past the window (<= 15)
+    int p0[2][12], cnt[2][12]; // per variable and month: month-major obs positions of days w0 .. w0+nwin+la-1
+    int g0, g1;                // 1981-2010 groups overlapping the window
+};
+int launch_tile_init(cudaStream_t s, TileState& t, const Batch& bmin, const Batch& bmax);
+int launch_tile_window(cudaStream_t s, TileState& t, const Ctx& cmin, const Ctx& cmax, const WindowSpan& w,
+                       int16_t* qmin, int16_t* qmax, cudaEvent_t after_apply);
+int launch_tile_end(cudaStream_t s, TileState& t, const Ctx& cmin, float* fnmin, float* fnmax, float* fsemin,
+                    float* fsemax, int32_t* ninvalid, uint8_t* status);
 int launch_status_to_u8(cudaStream_t s, int n, const int32_t* in, uint8_t* out);
 int launch_gather_month(cudaStream_t s, int npts, int mth0, const int32_t* st, const double* src12, double* dst);
 int launch_gather_vario(cudaStream_t s, int npts, int mth0, const int32_t* st, const int32_t* nn, const double* src,

@@ -10,7 +10,7 @@ kernel; PredictorGrids / interp_to_lonlat read the rasters of a PredictorStore. 
 '''
 
 __all__ = ["GwrTairAnom", 'KrigTair', 'KrigTairAll', 'BuildKrigParams', 'InterpTair', 'StationDataWrkChk', 'PtInterpTair',
-           'PredictorGrids']
+           'RecordStream', 'PredictorGrids']
 
 import numpy as np
 
@@ -323,6 +323,46 @@ class PtInterpTair(object):
     def interp_chunk_wait(self):
         '''Completion of the chunks submitted with interp_chunk(..., wait=False).'''
         _context.interp_chunk_wait(self.ctx_tmin)
+
+    def interp_chunk_stream(self, wrk_chk):
+        '''
+        New: interp_chunk over a long record in day windows (twxi_tile_begin / _days / _end).  The kriging and the GWR hat
+        rows run once here; the returned RecordStream emits the record window by window, so the device holds one window of
+        dailies instead of the whole record.  The windows concatenate to exactly the bytes interp_chunk returns.  One
+        stream per context pair at a time: a new stream discards an open one.
+        '''
+        return RecordStream(self, wrk_chk)
+
+
+class RecordStream(object):
+    '''
+    The daily record of one work chunk in consecutive windows (PtInterpTair.interp_chunk_stream).  `day0` is the first day
+    the next window starts at; `days(n)` returns {tmin, tmax} int16 [n, ny, nx]; `years()` yields (day0, out) per calendar
+    year of the remaining days; `finish()` returns the normals, se, ninvalid and status of interp_chunk and closes the
+    stream.  Buffers live where wrk_chk lives (numpy on the host, torch tensors on its CUDA device).
+    '''
+
+    def __init__(self, pt_interp, wrk_chk):
+        self.ctx_tmin, self.ctx_tmax = pt_interp.ctx_tmin, pt_interp.ctx_tmax
+        self.days_meta = pt_interp.days
+        self.device = wrk_chk.device if _lib.is_device(wrk_chk) else None
+        self.shape = _context.tile_begin(self.ctx_tmin, self.ctx_tmax, wrk_chk)
+        self.day0 = 0
+
+    def days(self, n, out=None):
+        o = _context.tile_days(self.ctx_tmin, self.ctx_tmax, n, self.shape, out=out, device=self.device)
+        self.day0 += int(n)
+        return o
+
+    def years(self):
+        yrs = np.asarray(self.days_meta[YEAR])
+        while self.day0 < yrs.size:
+            d0 = self.day0
+            n = int(np.searchsorted(yrs, yrs[d0], side="right")) - d0
+            yield d0, self.days(n)
+
+    def finish(self, out=None):
+        return _context.tile_end(self.ctx_tmin, self.ctx_tmax, self.shape, out=out, device=self.device)
 
 
 class StationDataWrkChk(StationSerialDataDb):

@@ -396,6 +396,40 @@ class TileWriter():
         ds = self._open_dataset(tile_id, varname, days)
         self._write(ds, varname, slice(None), slice(None), daily_vals, mthly_normals, mthly_normals_se, ninvalid)
 
+    def open_tile_stream(self, tile_id, varname, days):
+        '''
+        New: a whole tile written window by window (PtInterpTair.interp_chunk_stream).  Returns a handle with
+        `write_days(day0, vals)` (int16 [n, tile_y, tile_x] for days day0 .. day0+n-1) and `close(normals, se, ninvalid)`.
+        One dataset stays open from the first window to close, so no window is read back or rewritten; the file equals what
+        write_tile writes from the whole-record result.  The scipy netCDF-3 backend holds a variable in host memory until
+        close (the whole record of the tile), netCDF4 writes each window through.
+        '''
+        fpath = self._fpath(tile_id, varname)
+        if os.path.exists(fpath):
+            os.remove(fpath)
+        return _TileStream(self._open_dataset(tile_id, varname, days), varname)
+
+
+class _TileStream(object):
+    '''Open dataset of TileWriter.open_tile_stream.'''
+
+    def __init__(self, ds, varname):
+        self.ds = ds
+        self.varname = varname
+        self.v = ds.variables[varname]
+        if hasattr(self.v, 'set_auto_maskandscale'):
+            self.v.set_auto_maskandscale(False)                # data is already scaled int16 (tiling.py:529)
+
+    def write_days(self, day0, vals):
+        self.v[day0:day0 + len(vals), :, :] = vals
+
+    def close(self, mthly_normals, mthly_normals_se, ninvalid):
+        ds = self.ds
+        ds.variables[self.varname + "_normal"][:, :, :] = mthly_normals
+        ds.variables[self.varname + "_se"][:, :, :] = mthly_normals_se
+        ds.variables['inconsist_tair'][:, :] = ninvalid
+        ds.close()
+
 
 class AsyncTileWriter(object):
     '''
