@@ -51,7 +51,8 @@ extern "C" {
 #define TWXI_ST_NO_VARIO 2      /* "Cannot determine variogram params!"                  interp_tair.py:843     */
 #define TWXI_ST_TOO_FEW_STNS 3  /* IndexError: nnghs >= #candidate stations               station_select.py:164  */
 #define TWXI_ST_SINGULAR 4      /* singular / non-finite kriging or GWR system (R error, FloatingPointError);   */
-                                /* two co-located stations among a point's kriging neighbours are reported here */
+                                /* two co-located stations among a point's kriging neighbours are reported here, */
+                                /* and so is a GWR neighbour count below 6 (intercept + five trend predictors)   */
 #define TWXI_ST_FIXER_EMPTY 5   /* 'No valid tmin/tmax in window'                          interp_tair.py:192     */
 #define TWXI_ST_CLIMDIV 6       /* KeyError: climate division unknown to the station DB    interp_tair.py:563     */
 #define TWXI_ST_KNN_TIES 7      /* more than 512 exact distance ties at the selection boundary (unsupported)     */
