@@ -53,6 +53,8 @@ extern "C" {
 #define TWXI_ST_SINGULAR 4      /* singular / non-finite kriging or GWR system (R error, FloatingPointError);   */
                                 /* two co-located stations among a point's kriging neighbours are reported here, */
                                 /* and so is a GWR neighbour count below 6 (intercept + five trend predictors)   */
+                                /* and a variogram fit with fewer than 7 neighbours (OLS residuals of 5 trend     */
+                                /* coefficients need at least 2 degrees of freedom to carry a variogram)          */
 #define TWXI_ST_FIXER_EMPTY 5   /* 'No valid tmin/tmax in window'                          interp_tair.py:192     */
 #define TWXI_ST_CLIMDIV 6       /* KeyError: climate division unknown to the station DB    interp_tair.py:563     */
 #define TWXI_ST_KNN_TIES 7      /* more than 512 exact distance ties at the selection boundary (unsupported)     */

@@ -559,7 +559,8 @@ def fit_exp_range(npairs, dist, gamma, nugget, sill):
     exponential model gamma(h) = nugget + psill (1 - exp(-h / range)) with nugget and psill = sill - nugget fixed, the
     range fitted by weighted least squares with weights N_j / h_j^2 (gstat fit.method 7), Gauss-Newton from
     range0 = 0.1 max(dist) (interp.R:311), steps halved while the error grows, stop when the relative change of the
-    weighted SSE is below 1e-6 or after 200 iterations - continued here to the minimiser itself (|step| <= 1e-10 range).
+    weighted SSE is below 1e-6 or after 200 iterations - continued here until the step is below 1e-10 range or no step
+    lowers the SSE, then polished by up to 4 Newton steps on the gradient to the root of dS/dr (vario.cu does the same).
     Returns (nugget, psill, range) or None where the R code falls
     back to a pure nugget (fit error, negative psill or range: interp.R:69-77, 391-401)."""
     psill = sill - nugget
@@ -603,6 +604,23 @@ def fit_exp_range(npairs, dist, gamma, nugget, sill):
         s_old = s_new
         if small_step or (it >= FIT_MAXIT and gstat_done):
             break
+    # near the minimum the SSE differences are rounding noise: Newton on g(r) = sum w J e (dS/dr = -2 g), each step taken
+    # only while S'' > 0 (g' < 0) and |step| <= 1e-3 r
+    for _it in range(4):
+        if not (np.isfinite(r) and r > 0):
+            break
+        ex = np.exp(-dist / r)
+        e = gamma - (nugget + psill * (1.0 - ex))
+        J = -psill * ex * dist / (r * r)
+        dJ = psill * ex * dist * (2.0 * r - dist) / (r * r * r * r)
+        g = float(np.sum(w * J * e))
+        gp = float(np.sum(w * (dJ * e - J * J)))
+        if not gp < 0:
+            break
+        step = -g / gp
+        if not abs(step) <= 1e-3 * r:
+            break
+        r = r + step
     if not (np.isfinite(r) and r > 0):
         return None
     if nugget == 0 and psill == 0:                         # interp.R:74-77
@@ -618,9 +636,16 @@ def _ols_resid(X, y):
 def get_vario_params(ngh_lon, ngh_lat, ngh_X, ngh_y, ngh_dist):
     """R ``get_vario_params`` (interp.R:54-113): exponential variogram (nugget, psill, range) of the regression-kriging
     residuals of one neighbourhood.  ``ngh_X`` n x 4 (lon, lat, elev, lst), ``ngh_dist`` the haversine distances of the
-    neighbours from the point (StationSelect.ngh_dists).  Pure nugget -> (sill, 0, 0)."""
+    neighbours from the point (StationSelect.ngh_dists).  Pure nugget -> (sill, 0, 0).
+    Raises OracleError(ST_SINGULAR) for fewer than 7 neighbours (at n <= 5 the five-coefficient OLS fits exactly, at
+    n = 6 one degree of freedom is left) and for two neighbours at the same location (gstat puts nugget + psill at h = 0,
+    so V has two equal rows), as vario.cu decides them."""
     n = ngh_lon.size
+    if n < 7:
+        raise OracleError(ST_SINGULAR, "fewer than 7 neighbours for the variogram")
     H = gcdist_sp(ngh_lon[:, None], ngh_lat[:, None], ngh_lon[None, :], ngh_lat[None, :])
+    if np.any(H[np.triu_indices(n, 1)] == 0.0):
+        raise OracleError(ST_SINGULAR, "co-located neighbours: singular covariance matrix")
     cutoff = float(np.max(ngh_dist)) * 1.4                                    # :63
     k0 = int(np.argmin(ngh_dist))                                             # centre on the nearest neighbour (exact)
     Xc = np.asarray(ngh_X, dtype=np.float64) - np.asarray(ngh_X, dtype=np.float64)[k0][None, :]

@@ -8,6 +8,9 @@
 //      fit.method 7 weights np / h^2 (Gauss-Newton from 0.1 max h); pure nugget where the fit fails (interp.R:69-77)
 //   4. GLS trend with that model (predict(BLUE=TRUE)): residuals at the stations, their sill
 //   5. steps 2-3 again on the GLS residuals -> (nugget, psill, range), or (sill, 0, 0) for a pure nugget.
+// Two rules of this library that R does not have, both reported as TWXI_ST_SINGULAR (the oracle raises the same):
+//   n < 7 neighbours: at n <= 5 the five-coefficient OLS fits exactly and the residuals are rounding noise, at n = 6 one
+//   degree of freedom is left;  two neighbours at the same location (H == 0): V of step 4 has two equal rows.
 // One CTA per (point, month): the pair distances come from the station-station table, pair lags are kept in shared memory
 // (both variograms share pairs, counts and mean distances), lag sums are accumulated in 64-bit fixed point so that the
 // result does not depend on the order of the atomics, the n x n covariance matrix of step 4 is factored in packed shared
@@ -127,11 +130,31 @@ __device__ double fit_range_warp(int K, const double* bn, const double* bd, cons
         const bool small_step = fabs(rn - r) <= 1e-10 * rn;
         r = rn;
         // gstat stops when the relative change of the weighted SSE is below 1e-6 (or after 200 iterations); the iteration is
-        // then continued to the minimiser itself (|step| <= 1e-10 range) so that the result does not depend on where
-        // inside its tolerance band an implementation happens to stop
+        // continued until the step is below 1e-10 range or no step lowers the SSE, and then polished below
         if (fabs(s_old - s_new) <= 1e-6 * fmax(s_new, 1e-300)) gstat_done = true;
         s_old = s_new;
         if (small_step || (it >= 200 && gstat_done)) break;
+    }
+    // Within about sqrt(eps) of the minimum the SSE differences above are rounding noise, so the loop stops wherever the
+    // noise stops it (1e-10 .. 2e-8 relative).  Newton on the gradient g(r) = sum w J e, whose own rounding is not
+    // squared, takes the range to the root of dS/dr: g'(r) = sum w (J' e - J^2) with J' = psill e^(-h/r) h (2r - h) / r^4,
+    // a step taken only while S'' > 0 (g' < 0) and |step| <= 1e-3 r, i.e. near a minimum the loop has already reached
+    // (where S is nearly flat in r the SSE-tested loop can stop 1e-5 short, so a tighter guard would leave it there).
+    for (int it = 0; it < 4 && isfinite(r) && r > 0.0; ++it) {
+        double g = 0.0, gp = 0.0;
+        for (int k = lane; k < K; k += 32) {
+            const double h = bd[k], ex = exp(-h / r), w = bn[k] / (h * h);
+            const double e = bg[k] - (nugget + psill * (1.0 - ex));
+            const double J = -psill * ex * h / (r * r);
+            const double dJ = psill * ex * h * (2.0 * r - h) / (r * r * r * r);
+            g += w * J * e;
+            gp += w * (dJ * e - J * J);
+        }
+        g = warp_sum(g); gp = warp_sum(gp);
+        if (!(gp < 0.0)) break;
+        const double step = -g / gp;
+        if (!(fabs(step) <= 1e-3 * r)) break;
+        r += step;
     }
     return (isfinite(r) && r > 0.0) ? r : 0.0;
 }
@@ -255,6 +278,7 @@ __global__ void __launch_bounds__(VF_THREADS) vario_fit_kernel(VarioArgs a, int 
                     V[(size_t)i * (i + 1) / 2 + j] = h;       // raw distance, turned into a covariance by the GLS step
                     b = h <= cutoff ? (int)floor(h / VF_WIDTH) : 0xffff;
                     lag[base + j] = (unsigned short)b;
+                    if (h == 0.0) s_fail = 1;                 // two neighbours at one location: see the check below
                     if (b != 0xffff) {
                         atomicAdd(&cnt[b], 1);
                         atomicAdd(&sh[b], (unsigned long long)(h * VF_HSCALE + 0.5));
@@ -306,6 +330,13 @@ __global__ void __launch_bounds__(VF_THREADS) vario_fit_kernel(VarioArgs a, int 
     }
     residuals();
     variogram(true);
+    // two neighbours at the same location make the covariance matrix of step 4 singular (gstat puts nugget + psill at
+    // h = 0, so their rows are equal; R stops with an error): decided exactly, as the kriging kernel decides it, instead of
+    // by the sign of a rounded pivot, and for a pure nugget too
+    if (s_fail) {
+        if (tid == 0) atomicCAS(a.status + q, TWXI_ST_OK, TWXI_ST_SINGULAR);
+        return;
+    }
     fit();
 
     // ---- 4. GLS trend with the fitted model: beta = (X'V^-1X)^-1 X'V^-1 y -------------------------------------------
