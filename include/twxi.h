@@ -102,6 +102,8 @@ int twxi_ctx_create(twxi_ctx** ctx, int device, int n_stns,
  * year[ndays] (StationSerialDataDb.days, station_data.py:571-580).  Replaces StationDataWrkChk.set_obs /
  * load_obs (interp_tair.py:1027-1097): the whole table is resident in HBM, so there is no per-chunk cache.
  * Years 1981-2010 define the normals that are recomputed after a Tmin>=Tmax fix (interp_tair.py:466-479).
+ * The runs of consecutive days with one (year, month) over the whole record are the months of twxi_tile_days_mth; a
+ * record in which a (year, month) falls in two runs is accepted, it only has no monthly means.
  */
 int twxi_ctx_set_obs(twxi_ctx* ctx, const float* obs, int ndays, const int32_t* month, const int32_t* year);
 
@@ -280,7 +282,7 @@ int twxi_interp_chunk_wait(twxi_ctx* ctx_tmin, int host_sync);
  * daily record on the device, 12.4 GB per variable for a 250 x 250 tile over 1948-2015).
  *   twxi_tile_begin  everything of twxi_interp_chunk that does not depend on the day: unpack, kNN, neighbour counts,
  *                    kriging of the 12 normals and the 12 GWR hat rows of both variables.  Opens a "tile" on the pair
- *                    (state owned by ctx_tmin: 288 kh + 1 624 bytes per cell, kh = the largest neighbour count;
+ *                    (state owned by ctx_tmin: 288 kh + 1 632 bytes per cell, kh = the largest neighbour count;
  *                    2.75 GB for a 250 x 250 tile at kh = 147; kept for the next tile until the context is destroyed); a new begin discards an open tile.  `mem` is the memory space of
  *                    wrk_chk.
  *   twxi_tile_days   the next `ndays` days of the record (windows are consecutive, any length >= 1, chronological):
@@ -299,6 +301,32 @@ int twxi_tile_begin(twxi_ctx* ctx_tmin, twxi_ctx* ctx_tmax, const double* wrk_ch
 int twxi_tile_days(twxi_ctx* ctx_tmin, twxi_ctx* ctx_tmax, int ndays, int16_t* tmin, int16_t* tmax, int mem);
 int twxi_tile_end(twxi_ctx* ctx_tmin, twxi_ctx* ctx_tmax, float* tmin_norm, float* tmax_norm, float* tmin_se,
                   float* tmax_se, int32_t* ninvalid, uint8_t* status, int mem);
+
+/*
+ * Monthly means of the daily product, the third part of TopoWx next to the dailies and the normals (the reference writes
+ * them in a post-processing pass over the daily tile files, write_ds_mthly / _TairAggregate, tiling.py:1080-1219).
+ *   A month run is a maximal run of consecutive record days with one (year, month) as given to twxi_ctx_set_obs
+ *   (ctx_tmin's record).  The monthly value of a cell, variable and run is
+ *       float32( ((double)S / (double)n) * (double)0.01f )      (IEEE division and product, no contraction)
+ *   with S the exact int32 sum of the run's int16 counts as twxi_tile_days emits them (after the Tmin >= Tmax fixer) and
+ *   n the run's days in the record: a month the record covers in part averages the days it has.  The sum is exact, so no
+ *   order and no window boundary changes it.  A cell whose status is not TWXI_ST_OK (masked, failed at begin, or failed
+ *   by the fixer in the first window) gets TWXI_FILL_F4 in every month; fill counts never enter a sum.
+ *   The means are of the stored int16 values, not of the f64 dailies, on purpose: the reference averages what it reads
+ *   back from the daily files.  Parity with _TairAggregate is unpinned (it is not in this tree).
+ * twxi_tile_days_mth = twxi_tile_days (the same daily bytes) plus the monthly means of every month run whose last day
+ * falls in this window, chronological: tmin_mth, tmax_mth float32 [*nmth][ny][nx]; *nmth (host int32) = runs completed
+ * (0 allowed).  A month kernel after the window's fixer adds the counts into an int32 carry [2][ny][nx] of the tile, so
+ * nothing grows with the record.  Every argument is checked before any work is enqueued, and an error leaves the tile as
+ * it was: the errors of twxi_tile_days; max_mth < 0, nmth NULL, month buffers NULL with max_mth > 0, more than max_mth
+ * runs completed by the window, or a record in which a (year, month) falls in two runs or has more than 31 days ->
+ * TWXI_ERR_ARG (twxi_ctx_set_obs and the daily calls accept such a record); a twxi_tile_days window earlier in the same
+ * tile -> TWXI_ERR_STATE (the carry is valid only when every window since twxi_tile_begin went through this call).  The
+ * month kernel is not a stage: stage timing reports the slots of twxi_tile_days.  Measured on a B200 at a 1 000 W power
+ * limit: 0.065 ms per year window of a 250 x 250 tile, 2 % of the 1948-2015 stream (DESIGN.md section 5).
+ */
+int twxi_tile_days_mth(twxi_ctx* ctx_tmin, twxi_ctx* ctx_tmax, int ndays, int16_t* tmin, int16_t* tmax, int max_mth,
+                       float* tmin_mth, float* tmax_mth, int32_t* nmth, int mem);
 
 /*
  * Instrumentation for bench.py: number of kernels this library launched on the calling thread's contexts

@@ -3,7 +3,7 @@
 Gridded interpolation driver: the Python-3 / GPU counterpart of scripts/step25_mpi_interp_tair.py.
 
     python scripts/step25_interp_tair.py --out /tmp/twx_out [--rows 500 --cols 750] [--format nc|raw]
-                                         [--year0 1948 --years 68 --window year]
+                                         [--year0 1948 --years 68 --window year] [--months]
     torchrun --nproc-per-node N scripts/step25_interp_tair.py ...     (one process per GPU)
 
 The reference runs an MPI task farm: rank 0 reads every 50x50 work chunk's 27 predictor windows from netCDF and hands it
@@ -18,6 +18,10 @@ The synthetic station record covers --years calendar years from --year0.  --wind
 whole record in one call; --window year goes through PtInterpTair.interp_chunk_stream instead: kriging and GWR hat rows
 once per tile, then one calendar year at a time, so a multi-decade record never sits whole on the device or in pinned
 memory.  Each year is written as it comes (TileWriter.open_tile_stream; --format raw: one .npy per year window).
+--months also writes the monthly means of the dailies beside the daily tiles (<tile>_<var>_mthly.nc through
+TileWriter.open_tile_stream_mthly; --format raw: one <tile>_<var>_mthly_<day0>.npy per window and variable).  It always
+goes through interp_chunk_stream(months=True); with --window record the stream has one window covering the whole record,
+which gives the bytes of the whole-record call.
 '''
 import argparse
 import os
@@ -49,6 +53,7 @@ def main():
     ap.add_argument("--years", type=int, default=1, help="calendar years of the synthetic station record")
     ap.add_argument("--window", default="record", choices=["record", "year"],
                     help="whole record per tile in one call, or one calendar year at a time")
+    ap.add_argument("--months", action="store_true", help="also write the monthly means of the dailies")
     args = ap.parse_args()
     import torch
     rank = int(os.environ.get("RANK", "0"))
@@ -75,8 +80,8 @@ def main():
 
     mine = partition_chunks(tiler.tile_chks, tiler.mask, P_TILESIZE, P_TILESIZE, world, rank)
     nd = days.size
-    if args.window == "year":
-        return by_year(args, pt_interp, TileFeed(tiler, chunks=mine, depth=4), TileWriter(info, args.out), days, rank, world,
+    if args.window == "year" or args.months:
+        return streamed(args, pt_interp, TileFeed(tiler, chunks=mine, depth=4), TileWriter(info, args.out), days, rank, world,
                        len(mine))
     pin = lambda shape, dt: torch.empty(shape, dtype=dt).pin_memory()
     outs = [dict(tmin=pin((nd, P_TILESIZE, P_TILESIZE), torch.int16), tmax=pin((nd, P_TILESIZE, P_TILESIZE), torch.int16),
@@ -113,35 +118,50 @@ def main():
                                        nbytes / 1e6))
 
 
-def by_year(args, pt_interp, feed, tw, days, rank, world, ntiles):
+def streamed(args, pt_interp, feed, tw, days, rank, world, ntiles):
     t0 = time.time()
     ncells, nbytes = 0, 0
     for k, tid, wrk in feed:
-        s = pt_interp.interp_chunk_stream(wrk)
+        s = pt_interp.interp_chunk_stream(wrk, months=args.months)
         d = os.path.join(args.out, tid)
         os.makedirs(d, exist_ok=True)
-        hs = {v: tw.open_tile_stream(tid, v, days) for v in ("tmin", "tmax")} if args.format == "nc" else None
-        for d0, o in s.years():
+        nc = args.format == "nc"
+        hs = {v: tw.open_tile_stream(tid, v, days) for v in ("tmin", "tmax")} if nc else None
+        hm = {v: tw.open_tile_stream_mthly(tid, v, days) for v in ("tmin", "tmax")} if nc and args.months else None
+        windows = s.years() if args.window == "year" else iter([(0, s.days(days.size))])
+        m0 = 0
+        for d0, o in windows:
             for v in ("tmin", "tmax"):
                 if hs:
                     hs[v].write_days(d0, o[v])
                 else:
                     np.save(os.path.join(d, "%s_%s_%05d.npy" % (tid, v, d0)), o[v])
                     nbytes += o[v].nbytes
+                if hm:
+                    hm[v].write_months(m0, o[v + "_mth"])
+                elif args.months:
+                    np.save(os.path.join(d, "%s_%s_mthly_%05d.npy" % (tid, v, d0)), o[v + "_mth"])
+                    nbytes += o[v + "_mth"].nbytes
+            if args.months:
+                m0 += len(o["mth_groups"])
         fin = s.finish()
         for v in ("tmin", "tmax"):
             if hs:
                 hs[v].close(fin[v + "_norm"], fin[v + "_se"], fin["ninvalid"])
                 nbytes += os.path.getsize(tw._fpath(tid, v))
+            if hm:
+                hm[v].close()
+                nbytes += os.path.getsize(tw._fpath_mthly(tid, v))
         if not hs:
             for key, a in fin.items():
                 np.save(os.path.join(d, "%s_%s.npy" % (tid, key)), a)
                 nbytes += a.nbytes
         ncells += int((fin["status"] == 0).sum())
     dt = time.time() - t0
-    print("rank %d/%d: %d tiles, %d cells x %d days in %.2f s = %.3g cell-days/s in year windows to %s tiles on disk "
-          "(%.1f MB)" % (rank, world, ntiles, ncells, days.size, dt, ncells * days.size / max(dt, 1e-9),
-                         tw.format if args.format == "nc" else "raw .npy", nbytes / 1e6))
+    print("rank %d/%d: %d tiles, %d cells x %d days in %.2f s = %.3g cell-days/s in %s windows%s to %s tiles on disk "
+          "(%.1f MB)" % (rank, world, ntiles, ncells, days.size, dt, ncells * days.size / max(dt, 1e-9), args.window,
+                         " with monthly means" if args.months else "", tw.format if args.format == "nc" else "raw .npy",
+                         nbytes / 1e6))
 
 
 if __name__ == "__main__":

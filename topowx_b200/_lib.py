@@ -75,6 +75,7 @@ def _load():
         "twxi_interp_chunk_wait": (i32, [vp, i32]),
         "twxi_tile_begin": (i32, [vp, vp, vp, i32, i32, i32]),
         "twxi_tile_days": (i32, [vp, vp, i32, vp, vp, i32]),
+        "twxi_tile_days_mth": (i32, [vp, vp, i32, vp, vp, i32, vp, vp, vp, i32]),
         "twxi_tile_end": (i32, [vp, vp] + [vp] * 6 + [i32]),
         "twxi_measure_fp64_peak": (i32, [i32, vp, vp]),
     }

@@ -348,6 +348,42 @@ def tile_days(ctx_tmin, ctx_tmax, ndays, shape, out=None, device=None):
     return out
 
 
+class MonthGroups(object):
+    """The month runs of the record's days table (db.month_runs) and `day0`, the first day of the next window of the open
+    tile: tile_days_mth reads the runs a window completes from it and advances it.  Make one after each tile_begin."""
+
+    def __init__(self, days):
+        self.start, self.ndays, self.year, self.month = db.month_runs(days)
+        self.day0 = 0
+
+    def completed(self, n):
+        """Indices [g0, g1) of the runs whose last day falls in the days day0 .. day0 + n - 1."""
+        ends = self.start + self.ndays
+        return int(np.searchsorted(ends, self.day0, side="right")), int(np.searchsorted(ends, self.day0 + n, side="right"))
+
+
+def tile_days_mth(ctx_tmin, ctx_tmax, ndays, shape, groups, out=None, device=None):
+    """twxi_tile_days_mth: tile_days plus the monthly means of every month run that ends in the window ->
+    {tmin, tmax} int16 [ndays, ny, nx], {tmin_mth, tmax_mth} float32 [nmth, ny, nx] and mth_groups, the (year, month,
+    ndays) of each month, chronological.  ``groups`` is the MonthGroups of the tile (advanced by ndays); the month count
+    is exact, so ``out``'s month buffers must be [nmth, ny, nx]."""
+    ny, nx = shape
+    g0, g1 = groups.completed(int(ndays))
+    nm = g1 - g0
+    want = dict(tmin=("int16", (int(ndays), ny, nx)), tmax=("int16", (int(ndays), ny, nx)),
+                tmin_mth=("float32", (nm, ny, nx)), tmax_mth=("float32", (nm, ny, nx)))
+    out, dev = _result_buffers(want, out, device)
+    n = C.c_int32(-1)
+    check(lib.twxi_tile_days_mth(ctx_tmin.handle, ctx_tmax.handle, int(ndays), ptr(out["tmin"]), ptr(out["tmax"]), nm,
+                                 ptr(out["tmin_mth"]) if nm else None, ptr(out["tmax_mth"]) if nm else None, C.byref(n),
+                                 MEM_DEVICE if dev else MEM_HOST))
+    if n.value != nm:
+        raise RuntimeError("twxi_tile_days_mth completed %d months, the days table %d" % (n.value, nm))
+    groups.day0 += int(ndays)
+    out["mth_groups"] = [(int(groups.year[g]), int(groups.month[g]), int(groups.ndays[g])) for g in range(g0, g1)]
+    return out
+
+
 def tile_end(ctx_tmin, ctx_tmax, shape, out=None, device=None):
     """twxi_tile_end after the last day: {tmin_norm, tmax_norm, tmin_se, tmax_se, ninvalid, status} of interp_chunk
     (normals recomputed from the fixed 1981-2010 dailies when a day was fixed); closes the tile."""

@@ -207,9 +207,9 @@ static int copy_out_on(cudaStream_t s, T* dst, const T* src, size_t count) {
 static int tile_alloc(TileState& t) {
     const size_t nc = (size_t)t.ncell, nh = (size_t)2 * nc * 12 * t.kh;
     const size_t sizes[] = {2 * nc * 12 * 4, nh * 4, nh * 8, 2 * nc * 12 * 8, 2 * nc * 12 * 8, 2 * nc * 12 * 8, nc * 4,
-                            nc * 4, 2 * nc * 15 * 8, 2 * nc * 32 * 8, 2 * nc * 12 * 8};
-    size_t off[11], tot = 0;
-    for (int i = 0; i < 11; ++i) { off[i] = tot; tot += (sizes[i] + 255) & ~(size_t)255; }
+                            nc * 4, 2 * nc * 15 * 8, 2 * nc * 32 * 8, 2 * nc * 12 * 8, 2 * nc * 4};
+    size_t off[12], tot = 0;
+    for (int i = 0; i < 12; ++i) { off[i] = tot; tot += (sizes[i] + 255) & ~(size_t)255; }
     char* p;
     TWXI_TRY(t.fixed.get((void**)&p, tot));
     t.hk = reinterpret_cast<int32_t*>(p + off[0]); t.hidx = reinterpret_cast<int32_t*>(p + off[1]);
@@ -217,7 +217,7 @@ static int tile_alloc(TileState& t) {
     t.mean = reinterpret_cast<double*>(p + off[4]); t.var = reinterpret_cast<double*>(p + off[5]);
     t.status = reinterpret_cast<int32_t*>(p + off[6]); t.ninv = reinterpret_cast<int32_t*>(p + off[7]);
     t.carry = reinterpret_cast<double*>(p + off[8]); t.gpart = reinterpret_cast<double*>(p + off[9]);
-    t.gacc = reinterpret_cast<double*>(p + off[10]);
+    t.gacc = reinterpret_cast<double*>(p + off[10]); t.mcarry = reinterpret_cast<int32_t*>(p + off[11]);
     return TWXI_OK;
 }
 
@@ -456,16 +456,41 @@ int twxi_ctx_set_obs(twxi_ctx* c, const float* obs, int ndays, const int32_t* mo
         glen[g]++;
     }
     ob.ngroups = nyr * 12;
-    const float* d_obsT; const int *d_dop, *d_gs, *d_gl;
+    // month runs of the whole record (twxi_tile_days_mth): maximal runs of consecutive days with one (year, month); a
+    // (year, month) met in two runs leaves the record without monthly means, it is not an error of the record
+    std::vector<int> rstart, rlen;
+    std::vector<long long> rkey;
+    for (int d = 0; d < ndays; ++d) {
+        const long long key = (long long)year[d] * 16 + month[d];
+        if (d == 0 || key != rkey.back()) {
+            rstart.push_back(d);
+            rlen.push_back(0);
+            rkey.push_back(key);
+        }
+        rlen.back()++;
+    }
+    std::string mth_error;
+    std::sort(rkey.begin(), rkey.end());
+    if (std::adjacent_find(rkey.begin(), rkey.end()) != rkey.end())
+        mth_error = "the days of a (year, month) of the record are not consecutive: monthly means need a chronological record";
+    else if (*std::max_element(rlen.begin(), rlen.end()) > 31)       // keeps the int32 sums of int16 counts exact
+        mth_error = "a (year, month) of the record has more than 31 days";
+    const float* d_obsT; const int *d_dop, *d_gs, *d_gl, *d_rs, *d_rl;
     TWXI_TRY(dev_upload(*c, c->obs_owned, &d_obsT, obsT.data(), obsT.size()));
     TWXI_TRY(dev_upload(*c, c->obs_owned, &d_dop, day_of_pos.data(), day_of_pos.size()));
     TWXI_TRY(dev_upload(*c, c->obs_owned, &d_gs, gstart.data(), gstart.size()));
     TWXI_TRY(dev_upload(*c, c->obs_owned, &d_gl, glen.data(), glen.size()));
+    TWXI_TRY(dev_upload(*c, c->obs_owned, &d_rs, rstart.data(), rstart.size()));
+    TWXI_TRY(dev_upload(*c, c->obs_owned, &d_rl, rlen.data(), rlen.size()));
     TWXI_CUDA(cudaStreamSynchronize(c->stream));
     ob.obsT = d_obsT; ob.day_of_pos = d_dop; ob.grp_start = d_gs; ob.grp_len = d_gl;
+    c->mrun_start = d_rs; c->mrun_len = d_rl;
     c->h_day_of_pos = std::move(day_of_pos);
     c->h_grp_start = std::move(gstart);
     c->h_grp_len = std::move(glen);
+    c->h_mrun_start = std::move(rstart);
+    c->h_mrun_len = std::move(rlen);
+    c->mth_error = std::move(mth_error);
     c->has_obs = true;
     return TWXI_OK;
 }
@@ -1021,6 +1046,7 @@ static int tile_begin_impl(twxi_ctx* cmin, twxi_ctx* cmax, const double* wrk_chk
     t.gen_min = cmin->obs_gen; t.gen_max = cmax->obs_gen;
     t.ndays = cmin->ob.ndays;
     t.next_day = 0;
+    t.plain_days = false;
     TWXI_TRY(finish(*cmin, mem));
     t.open = true;
     return TWXI_OK;
@@ -1049,7 +1075,20 @@ static void month_positions(const Ctx& c, int m, int d0, int d1, int* p0, int* c
     *cnt = (int)(hi - lo);
 }
 
-static int tile_days_impl(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, int16_t* tmin, int16_t* tmax, int mem) {
+// Month runs of the days [w0, w1) (ascending run starts: the runs overlapping the window are the last one that starts at
+// or before w0 up to the last one that starts before w1, and all but that last one end inside the window).
+static MonthSpan month_span(const Ctx& c, int w0, int w1) {
+    const std::vector<int>& st = c.h_mrun_start;
+    MonthSpan m;
+    m.g0 = (int)(std::upper_bound(st.begin(), st.end(), w0) - st.begin()) - 1;
+    m.g1 = (int)(std::lower_bound(st.begin(), st.end(), w1) - st.begin());
+    m.nmth = m.g1 - m.g0 - (st[m.g1 - 1] + c.h_mrun_len[m.g1 - 1] > w1 ? 1 : 0);
+    return m;
+}
+
+// One window of the open tile; with `mth`, also the monthly means of the runs that end in it (twxi_tile_days_mth).
+static int tile_days_impl(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, int16_t* tmin, int16_t* tmax, int mem,
+                          const MonthSpan* mth = nullptr, float* tmin_mth = nullptr, float* tmax_mth = nullptr) {
     TileState& t = cmin->tile;
     WindowSpan w;
     w.w0 = t.next_day; w.nwin = ndays;
@@ -1065,11 +1104,14 @@ static int tile_days_impl(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, int16_t* tm
         if (w.g0 == w.g1) w.g0 = g;
         w.g1 = g + 1;
     }
-    const size_t nq = (size_t)ndays * t.ncell;
+    const size_t nq = (size_t)ndays * t.ncell, nf = mth ? (size_t)mth->nmth * t.ncell : 0;
     int16_t *d_qmin = tmin, *d_qmax = tmax;
+    float *d_fmin = tmin_mth, *d_fmax = tmax_mth;
     if (mem != TWXI_MEM_DEVICE) {
-        TWXI_TRY(t.out.get((void**)&d_qmin, 2 * nq * 2));
+        TWXI_TRY(t.out.get((void**)&d_qmin, 2 * nq * 2 + 2 * nf * 4));
         d_qmax = d_qmin + nq;
+        d_fmin = reinterpret_cast<float*>(d_qmax + nq);
+        d_fmax = d_fmin + nf;
     }
     cudaEvent_t ev[3];
     const bool timing = stage_timing_on();
@@ -1086,9 +1128,12 @@ static int tile_days_impl(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, int16_t* tm
         cudaEventElapsedTime(&g_stage_ms[4], ev[1], ev[2]);
         for (auto& e : ev) cudaEventDestroy(e);
     }
+    if (mth) TWXI_TRY(launch_tile_month(cmin->stream, t, *cmin, w, *mth, d_qmin, d_qmax, d_fmin, d_fmax));
     if (mem != TWXI_MEM_DEVICE) {
         TWXI_TRY(copy_out(*cmin, tmin, d_qmin, nq));
         TWXI_TRY(copy_out(*cmin, tmax, d_qmax, nq));
+        TWXI_TRY(copy_out(*cmin, tmin_mth, d_fmin, nf));
+        TWXI_TRY(copy_out(*cmin, tmax_mth, d_fmax, nf));
     }
     t.next_day = w1;
     return finish(*cmin, mem);
@@ -1139,7 +1184,33 @@ int twxi_tile_days(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, int16_t* tmin, int
     TWXI_ARG(tmin && tmax, "null argument");
     TWXI_ARG(ndays >= 1 && ndays <= cmin->tile.ndays - cmin->tile.next_day, "ndays must be 1 .. the days that remain");
     TWXI_CUDA(cudaSetDevice(cmin->device));
+    cmin->tile.plain_days = true;
     return tile_days_impl(cmin, cmax, ndays, tmin, tmax, mem);
+}
+
+int twxi_tile_days_mth(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, int16_t* tmin, int16_t* tmax, int max_mth,
+                       float* tmin_mth, float* tmax_mth, int32_t* nmth, int mem) {
+    TWXI_TRY(tile_check(cmin, cmax));
+    TWXI_ARG(tmin && tmax && nmth, "null argument");
+    TWXI_ARG(ndays >= 1 && ndays <= cmin->tile.ndays - cmin->tile.next_day, "ndays must be 1 .. the days that remain");
+    TWXI_ARG(max_mth >= 0, "max_mth must be >= 0");
+    TWXI_ARG(max_mth == 0 || (tmin_mth && tmax_mth), "null month buffer");
+    TWXI_ARG(cmin->mth_error.empty(), cmin->mth_error);
+    const TileState& t = cmin->tile;
+    if (t.plain_days) {
+        set_error("twxi_tile_days_mth after twxi_tile_days in the same tile: the month sums miss that window");
+        return TWXI_ERR_STATE;
+    }
+    const MonthSpan m = month_span(*cmin, t.next_day, t.next_day + ndays);
+    if (m.nmth > max_mth) {
+        set_error("the window completes " + std::to_string(m.nmth) + " months, more than max_mth = " +
+                  std::to_string(max_mth));
+        return TWXI_ERR_ARG;
+    }
+    TWXI_CUDA(cudaSetDevice(cmin->device));
+    TWXI_TRY(tile_days_impl(cmin, cmax, ndays, tmin, tmax, mem, &m, tmin_mth, tmax_mth));
+    *nmth = m.nmth;
+    return TWXI_OK;
 }
 
 int twxi_tile_end(twxi_ctx* cmin, twxi_ctx* cmax, float* tmin_norm, float* tmax_norm, float* tmin_se, float* tmax_se,

@@ -11,6 +11,10 @@
 //             group, warp_sum, accumulated year by year), with the lane partials of an unfinished group carried over.
 // A fixed day is valid (tavg -/+ half, half > 0), so only the fix of day 0 can find no valid day in its window; that
 // decision falls in the first window, which always computes days 1..15 as look-ahead.
+//
+// twxi_tile_days_mth adds the monthly means of the emitted int16 counts (tile_month_kernel, after tile_fix_kernel):
+// exact int32 sums per (cell, month run), so no order or window boundary can change them, with the sum of the run that
+// the window leaves open carried to the next window.
 #include "twxi_internal.cuh"
 
 namespace twxi {
@@ -260,6 +264,60 @@ int launch_tile_window(cudaStream_t s, TileState& t, const Ctx& cmin, const Ctx&
     f.grp_start = cmin.ob.grp_start; f.grp_len = cmin.ob.grp_len; f.g0 = w.g0; f.g1 = w.g1;
     f.qmin = qmin; f.qmax = qmax;
     tile_fix_kernel<<<(t.ncell + 3) / 4, 128, 0, s>>>(f);
+    TWXI_LAUNCH_CHECK();
+    return TWXI_OK;
+}
+
+struct MonthArgs {
+    int ncell, w0, w1, g0, g1;
+    const int* run_start;      // month runs of the record (Ctx::mrun_*)
+    const int* run_len;
+    const int32_t* status;
+    int32_t* carry;            // [2][ncell]
+    const int16_t* qmin;       // [w1 - w0][ncell] the window's quantised tmin / tmax
+    const int16_t* qmax;
+    float* fmin;               // [nmth][ncell] monthly means of tmin / tmax
+    float* fmax;
+};
+
+// One thread per (cell, variable), days in order: every day is one coalesced [d][ncell] row.  S / n * 0.01f in double,
+// rounded once to float (no contraction).  Cells that are not ok (masked, failed at begin or by the fixer of the first
+// window, which ran before this kernel) have fill counts and get fill in every month.
+__global__ void tile_month_kernel(MonthArgs a) {
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= a.ncell) return;
+    const int v = blockIdx.y;
+    const size_t P = (size_t)a.ncell;
+    const int16_t* in = (v ? a.qmax : a.qmin) + q;
+    float* out = (v ? a.fmax : a.fmin) + q;
+    const bool good = a.status[q] == TWXI_ST_OK;
+    int s = a.w0 == 0 ? 0 : a.carry[v * P + q];               // the first window starts every sum at zero
+    int d = a.w0;
+    for (int g = a.g0; g < a.g1; ++g) {
+        const int gend = a.run_start[g] + a.run_len[g];
+        const int end = min(gend, a.w1);
+        if (good) {
+#pragma unroll 8
+            for (; d < end; ++d) s += in[(size_t)(d - a.w0) * P];
+        }
+        d = end;
+        if (gend <= a.w1) {
+            const double mean = __dmul_rn(__ddiv_rn((double)s, (double)a.run_len[g]), (double)0.01f);
+            out[(size_t)(g - a.g0) * P] = good ? (float)mean : TWXI_FILL_F4;
+            s = 0;
+        }
+    }
+    a.carry[v * P + q] = s;
+}
+
+int launch_tile_month(cudaStream_t s, TileState& t, const Ctx& cmin, const WindowSpan& w, const MonthSpan& m,
+                      const int16_t* qmin, const int16_t* qmax, float* fmin, float* fmax) {
+    MonthArgs a;
+    a.ncell = t.ncell; a.w0 = w.w0; a.w1 = w.w0 + w.nwin; a.g0 = m.g0; a.g1 = m.g1;
+    a.run_start = cmin.mrun_start; a.run_len = cmin.mrun_len;
+    a.status = t.status; a.carry = t.mcarry;
+    a.qmin = qmin; a.qmax = qmax; a.fmin = fmin; a.fmax = fmax;
+    tile_month_kernel<<<dim3((t.ncell + 255) / 256, 2), 256, 0, s>>>(a);
     TWXI_LAUNCH_CHECK();
     return TWXI_OK;
 }

@@ -156,6 +156,8 @@ struct TileState {
     double* carry = nullptr;   // [2][ncell][15] the last 15 fixed dailies before the next window
     double* gpart = nullptr;   // [2][ncell][32] per-lane partial sums of the open 1981-2010 (year, month) group
     double* gacc = nullptr;    // [2][ncell][12] running sums over years of the group means
+    int32_t* mcarry = nullptr; // [2][ncell] int16 counts summed so far of the month run the next window continues
+    bool plain_days = false;   // a twxi_tile_days window since begin: mcarry misses its days
     Scratch fixed, win, out;   // the arrays above; window dailies [2][ncell][15 + nwin + 15]; host-bound staging
     void release() { fixed.release(); win.release(); out.release(); *this = TileState(); }
 };
@@ -178,6 +180,12 @@ struct Ctx {
     std::vector<void*> obs_owned;
     std::vector<int> h_day_of_pos; // host copies of ob.day_of_pos / grp_start / grp_len (window position ranges)
     std::vector<int> h_grp_start, h_grp_len;
+    // month runs of the whole record (twxi_tile_days_mth): maximal runs of consecutive days with one (year, month), first
+    // day (ascending) and length, on the device and the host (kept out of ObsTable, which the stage kernels take by value)
+    const int* mrun_start = nullptr;
+    const int* mrun_len = nullptr;
+    std::vector<int> h_mrun_start, h_mrun_len;
+    std::string mth_error;         // why the record has no monthly means (a (year, month) in two runs); empty: it has
     double* climdivs = nullptr;
     int n_climdivs = -1;           // -1: no check
     Batch b;
@@ -227,6 +235,12 @@ struct WindowSpan {
 int launch_tile_init(cudaStream_t s, TileState& t, const Batch& bmin, const Batch& bmax);
 int launch_tile_window(cudaStream_t s, TileState& t, const Ctx& cmin, const Ctx& cmax, const WindowSpan& w,
                        int16_t* qmin, int16_t* qmax, cudaEvent_t after_apply);
+// Month runs of the window [w0, w1) of twxi_tile_days_mth: runs g0 .. g1-1 overlap it, the first nmth of them end in it.
+struct MonthSpan {
+    int g0, g1, nmth;
+};
+int launch_tile_month(cudaStream_t s, TileState& t, const Ctx& cmin, const WindowSpan& w, const MonthSpan& m,
+                      const int16_t* qmin, const int16_t* qmax, float* fmin, float* fmax);
 int launch_tile_end(cudaStream_t s, TileState& t, const Ctx& cmin, float* fnmin, float* fnmax, float* fsemin,
                     float* fsemax, int32_t* ninvalid, uint8_t* status);
 int launch_status_to_u8(cudaStream_t s, int n, const int32_t* in, uint8_t* out);

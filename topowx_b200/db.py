@@ -60,6 +60,15 @@ def get_days_metadata_dates(dates):
     return days
 
 
+def month_runs(days):
+    """Month groups of a days table (new): maximal runs of consecutive days with one (YEAR, MONTH), as
+    twxi_tile_days_mth averages them.  Returns int64 arrays start, ndays, year, month (one entry per run, chronological)."""
+    y, m = np.asarray(days[YEAR]), np.asarray(days[MONTH])
+    start = np.concatenate([[0], np.flatnonzero((y[1:] != y[:-1]) | (m[1:] != m[:-1])) + 1]).astype(np.int64)
+    ndays = np.diff(np.append(start, y.size))
+    return start, ndays, y[start].astype(np.int64), m[start].astype(np.int64)
+
+
 def station_dtype(id_len=16):
     """dtype of the structured station array the hot path reads (numeric fields float64,
     ``station_data.py:159-164``)."""

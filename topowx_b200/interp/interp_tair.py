@@ -324,14 +324,15 @@ class PtInterpTair(object):
         '''Completion of the chunks submitted with interp_chunk(..., wait=False).'''
         _context.interp_chunk_wait(self.ctx_tmin)
 
-    def interp_chunk_stream(self, wrk_chk):
+    def interp_chunk_stream(self, wrk_chk, months=False):
         '''
         New: interp_chunk over a long record in day windows (twxi_tile_begin / _days / _end).  The kriging and the GWR hat
         rows run once here; the returned RecordStream emits the record window by window, so the device holds one window of
         dailies instead of the whole record.  The windows concatenate to exactly the bytes interp_chunk returns.  One
-        stream per context pair at a time: a new stream discards an open one.
+        stream per context pair at a time: a new stream discards an open one.  months=True: every window also returns the
+        monthly means of the months it completes (twxi_tile_days_mth), so one pass emits dailies, normals and monthly grids.
         '''
-        return RecordStream(self, wrk_chk)
+        return RecordStream(self, wrk_chk, months)
 
 
 class RecordStream(object):
@@ -339,18 +340,25 @@ class RecordStream(object):
     The daily record of one work chunk in consecutive windows (PtInterpTair.interp_chunk_stream).  `day0` is the first day
     the next window starts at; `days(n)` returns {tmin, tmax} int16 [n, ny, nx]; `years()` yields (day0, out) per calendar
     year of the remaining days; `finish()` returns the normals, se, ninvalid and status of interp_chunk and closes the
-    stream.  Buffers live where wrk_chk lives (numpy on the host, torch tensors on its CUDA device).
+    stream.  Buffers live where wrk_chk lives (numpy on the host, torch tensors on its CUDA device).  With months=True
+    each window's dict also holds tmin_mth, tmax_mth float32 [nmth, ny, nx] and mth_groups [(year, month, ndays)] of the
+    months that end in it (context.tile_days_mth).
     '''
 
-    def __init__(self, pt_interp, wrk_chk):
+    def __init__(self, pt_interp, wrk_chk, months=False):
         self.ctx_tmin, self.ctx_tmax = pt_interp.ctx_tmin, pt_interp.ctx_tmax
         self.days_meta = pt_interp.days
         self.device = wrk_chk.device if _lib.is_device(wrk_chk) else None
         self.shape = _context.tile_begin(self.ctx_tmin, self.ctx_tmax, wrk_chk)
+        self.groups = _context.MonthGroups(self.days_meta) if months else None
         self.day0 = 0
 
     def days(self, n, out=None):
-        o = _context.tile_days(self.ctx_tmin, self.ctx_tmax, n, self.shape, out=out, device=self.device)
+        if self.groups is None:
+            o = _context.tile_days(self.ctx_tmin, self.ctx_tmax, n, self.shape, out=out, device=self.device)
+        else:
+            o = _context.tile_days_mth(self.ctx_tmin, self.ctx_tmax, n, self.shape, self.groups, out=out,
+                                       device=self.device)
         self.day0 += int(n)
         return o
 

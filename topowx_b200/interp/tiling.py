@@ -13,6 +13,8 @@ from datetime import datetime
 
 import numpy as np
 
+from ..db import month_runs
+
 
 class Tiler():
     '''
@@ -261,25 +263,26 @@ class TileWriter():
         os.makedirs(os.path.join(self.path_out, tile_id), exist_ok=True)
         return self._create_ncdf(fpath, tile_id, varname, days)
 
-    def _create_ncdf(self, fpath, tile_id, varname, days):
+    def _new_tile_dataset(self, fpath, tile_id, days, ntime, title, comment, extra_dims=()):
+        """A new tile file with the global attributes, the dimensions time (ntime), lat, lon, nv and extra_dims, and the
+        time coordinate (values left to the caller) in days since the record's first day.  Returns (ds, d0, units)."""
         from .. import __version__ as twx_version
         nc = self._nc
         ds = nc.open(fpath, 'w')
-        ds.title = "".join(["Daily Interpolated Meteorological Data ", str(days['YMD'][0]), "-", str(days['YMD'][-1])])
+        ds.title = "".join([title, str(days['YMD'][0]), "-", str(days['YMD'][-1])])
         ds.institution = "University of Montana"
         ds.source = "TopoWx %s (topowx_b200 GPU path)" % twx_version
         ds.history = "".join(["Created on: ", datetime.strftime(datetime.today(), "%Y-%m-%d")])
         ds.references = "http://www.ntsg.umt.edu/project/TopoWx"
-        ds.comment = "30-arcsec spatial resolution, daily timestep"
+        ds.comment = comment
         ds.Conventions = "CF-1.6"
+        ds.createDimension('time', ntime)
         str_row, str_col = self.tile_rc[tile_id]
-        lons = self.lons[str_col:str_col + self.tile_size_x]
-        lats = self.lats[str_row:str_row + self.tile_size_y]
-        ds.createDimension('time', days.size)
-        ds.createDimension('lat', lats.size)
-        ds.createDimension('lon', lons.size)
+        ds.createDimension('lat', self.lats[str_row:str_row + self.tile_size_y].size)
+        ds.createDimension('lon', self.lons[str_col:str_col + self.tile_size_x].size)
         ds.createDimension('nv', 2)
-        ds.createDimension('time_normals', 12)
+        for name, size in extra_dims:
+            ds.createDimension(name, size)
         min_date = days['DATE'][0]
         d0 = datetime(min_date.year, min_date.month, min_date.day)
         units = "".join(["days since ", str(min_date.year), "-", str(min_date.month), "-", str(min_date.day), " 0:0:0"])
@@ -289,10 +292,36 @@ class TileWriter():
         times.standard_name = "time"
         times.calendar = "standard"
         times.bounds = 'time_bnds'
-        time_bnds = nc.create_variable(ds, 'time_bnds', 'f8', ('time', 'nv'))
+        nc.create_variable(ds, 'time_bnds', 'f8', ('time', 'nv'))
+        return ds, d0, units
+
+    def _add_grid(self, ds, tile_id):
+        """lat, lon and the crs grid mapping of the tile."""
+        nc = self._nc
+        str_row, str_col = self.tile_rc[tile_id]
+        latitudes = nc.create_variable(ds, 'lat', 'f8', ('lat',))
+        latitudes.long_name = "latitude"
+        latitudes.units = "degrees_north"
+        latitudes.standard_name = "latitude"
+        latitudes[:] = self.lats[str_row:str_row + self.tile_size_y]
+        longitudes = nc.create_variable(ds, 'lon', 'f8', ('lon',))
+        longitudes.long_name = "longitude"
+        longitudes.units = "degrees_east"
+        longitudes.standard_name = "longitude"
+        longitudes[:] = self.lons[str_col:str_col + self.tile_size_x]
+        crs = nc.create_variable(ds, 'crs', 'i2', ())
+        crs.grid_mapping_name = "latitude_longitude"
+        crs.longitude_of_prime_meridian = 0.0
+        crs.semi_major_axis = 6378137.0
+        crs.inverse_flattening = 298.257223563
+
+    def _create_ncdf(self, fpath, tile_id, varname, days):
+        nc = self._nc
+        ds, d0, units = self._new_tile_dataset(fpath, tile_id, days, days.size, "Daily Interpolated Meteorological Data ",
+                                               "30-arcsec spatial resolution, daily timestep", [('time_normals', 12)])
         time_nums = _date2num(days['DATE'], d0) + 0.5
-        times[:] = time_nums
-        time_bnds[:] = np.stack([time_nums - 0.5, time_nums + 0.5], axis=1)
+        ds.variables['time'][:] = time_nums
+        ds.variables['time_bnds'][:] = np.stack([time_nums - 0.5, time_nums + 0.5], axis=1)
         time_means = nc.create_variable(ds, 'time_normals', 'f8', ('time_normals',))
         time_means.long_name = "time"
         time_means.units = units
@@ -310,21 +339,7 @@ class TileWriter():
             cb[mth - 1] = _date2num([datetime(1981, mth, 1), datetime(2010 if mth != 12 else 2011, mth_next, 1)], d0)
         time_means[:] = tm
         clim_bnds[:] = cb
-        latitudes = nc.create_variable(ds, 'lat', 'f8', ('lat',))
-        latitudes.long_name = "latitude"
-        latitudes.units = "degrees_north"
-        latitudes.standard_name = "latitude"
-        latitudes[:] = lats
-        longitudes = nc.create_variable(ds, 'lon', 'f8', ('lon',))
-        longitudes.long_name = "longitude"
-        longitudes.units = "degrees_east"
-        longitudes.standard_name = "longitude"
-        longitudes[:] = lons
-        crs = nc.create_variable(ds, 'crs', 'i2', ())
-        crs.grid_mapping_name = "latitude_longitude"
-        crs.longitude_of_prime_meridian = 0.0
-        crs.semi_major_axis = 6378137.0
-        crs.inverse_flattening = 298.257223563
+        self._add_grid(ds, tile_id)
         self._add_dim_vars(ds, varname, days)
         return ds
 
@@ -409,6 +424,43 @@ class TileWriter():
             os.remove(fpath)
         return _TileStream(self._open_dataset(tile_id, varname, days), varname)
 
+    def _fpath_mthly(self, tile_id, varname):
+        return os.path.join(self.path_out, tile_id, "%s_%s_mthly.nc" % (tile_id, varname))
+
+    def open_tile_stream_mthly(self, tile_id, varname, days):
+        '''
+        New: the monthly means of a tile (PtInterpTair.interp_chunk_stream(months=True)) written as the windows complete
+        them, to <tile_id>_<varname>_mthly.nc beside the daily file.  One time step per month run of `days`
+        (db.month_runs): `time` is its middle, `time_bnds` its first day and its last day + 1 in the record, so a month the
+        record covers in part is bounded by the days it has.  Returns a handle with `write_months(m0, vals)` (float32
+        [n, tile_y, tile_x] for months m0 .. m0+n-1) and `close()`.
+        '''
+        nc = self._nc
+        fpath = self._fpath_mthly(tile_id, varname)
+        if os.path.exists(fpath):
+            os.remove(fpath)
+        os.makedirs(os.path.join(self.path_out, tile_id), exist_ok=True)
+        start, ndays, _, _ = month_runs(days)
+        ds, d0, _ = self._new_tile_dataset(fpath, tile_id, days, start.size, "Monthly Interpolated Meteorological Data ",
+                                           "30-arcsec spatial resolution, monthly timestep")
+        first = _date2num(days['DATE'][start], d0)
+        last1 = _date2num(days['DATE'][start + ndays - 1], d0) + 1.0
+        ds.variables['time'][:] = (first + last1) / 2.0
+        ds.variables['time_bnds'][:] = np.stack([first, last1], axis=1)
+        self._add_grid(ds, tile_id)
+        long_name, units, standard_name, _, cell_method = VAR_ATTRS[varname]
+        v = nc.create_variable(ds, varname, 'f4', ('time', 'lat', 'lon'), fill_value=FILL_F4,
+                               chunksizes=(1, self.chk_size_y, self.chk_size_x))
+        v.long_name = "monthly mean " + long_name
+        v.units = units
+        v.standard_name = standard_name
+        v.cell_methods = "area: mean time: %s within days time: mean over days" % cell_method
+        v.comment = ("Mean of the month's daily values as stored in the daily tile (int16, scale_factor 0.01); a month the "
+                     "record covers in part is the mean of the days it has")
+        v.coordinates = "lat lon"
+        v.grid_mapping = "crs"
+        return _MonthStream(ds, varname)
+
 
 class _TileStream(object):
     '''Open dataset of TileWriter.open_tile_stream.'''
@@ -429,6 +481,21 @@ class _TileStream(object):
         ds.variables[self.varname + "_se"][:, :, :] = mthly_normals_se
         ds.variables['inconsist_tair'][:, :] = ninvalid
         ds.close()
+
+
+class _MonthStream(object):
+    '''Open dataset of TileWriter.open_tile_stream_mthly.'''
+
+    def __init__(self, ds, varname):
+        self.ds = ds
+        self.v = ds.variables[varname]
+
+    def write_months(self, m0, vals):
+        if len(vals):
+            self.v[m0:m0 + len(vals), :, :] = vals
+
+    def close(self):
+        self.ds.close()
 
 
 class AsyncTileWriter(object):
