@@ -242,45 +242,18 @@ def interp_chunk(ctx_tmin, ctx_tmax, wrk_chk, out=None, daily=True, wait=True):
     submits the chunk with twxi_interp_chunk_async: its buffers belong to the library until ``interp_chunk_wait`` returns or
     until two further chunks have been submitted on the same context pair (the second submission blocks the host until this
     chunk's results are in the host buffers); the copies overlap the neighbouring chunks' kernels."""
-    dev = _lib.is_device(wrk_chk)
-    if len(wrk_chk.shape) != 3 or wrk_chk.shape[0] != 32:
-        raise ValueError("wrk_chk must be [32, ny, nx] (planes of tiling.py:205-213 / step25:273-279), got %r"
-                         % (tuple(wrk_chk.shape),))
-    if _dtype_name(wrk_chk) != "float64":
-        raise ValueError("wrk_chk must be float64, got %s" % _dtype_name(wrk_chk))
-    _, ny, nx = wrk_chk.shape
+    ny, nx = _check_wrk_chk(wrk_chk)
     if daily and ctx_tmin.ndays != ctx_tmax.ndays:
         raise ValueError("tmin and tmax contexts hold observation records of different length")
     nd = ctx_tmin.ndays
-    if out is None:
-        if dev:
-            import torch
-            mk = lambda shape, dt: torch.empty(shape, dtype=dt, device=wrk_chk.device)
-            out = dict(tmin=mk((nd, ny, nx), torch.int16) if daily else None,
-                       tmax=mk((nd, ny, nx), torch.int16) if daily else None,
-                       tmin_norm=mk((12, ny, nx), torch.float32), tmax_norm=mk((12, ny, nx), torch.float32),
-                       tmin_se=mk((12, ny, nx), torch.float32), tmax_se=mk((12, ny, nx), torch.float32),
-                       ninvalid=mk((ny, nx), torch.int32), status=mk((ny, nx), torch.uint8))
-        else:
-            out = dict(tmin=np.empty((nd, ny, nx), np.int16) if daily else None,
-                       tmax=np.empty((nd, ny, nx), np.int16) if daily else None,
-                       tmin_norm=np.empty((12, ny, nx), np.float32), tmax_norm=np.empty((12, ny, nx), np.float32),
-                       tmin_se=np.empty((12, ny, nx), np.float32), tmax_se=np.empty((12, ny, nx), np.float32),
-                       ninvalid=np.empty((ny, nx), np.int32), status=np.empty((ny, nx), np.uint8))
-    else:
-        want = dict(tmin=("int16", (nd, ny, nx)), tmax=("int16", (nd, ny, nx)), tmin_norm=("float32", (12, ny, nx)),
-                    tmax_norm=("float32", (12, ny, nx)), tmin_se=("float32", (12, ny, nx)), tmax_se=("float32", (12, ny, nx)),
-                    ninvalid=("int32", (ny, nx)), status=("uint8", (ny, nx)))
-        for k, (dt, shp) in want.items():
-            b = out.get(k)
-            if b is None:
-                if k in ("tmin", "tmax") and not daily:
-                    continue
-                raise ValueError("out[%r] is missing" % k)
-            if _dtype_name(b) != dt or tuple(b.shape) != shp:
-                raise ValueError("out[%r] must be %s %r, got %s %r" % (k, dt, shp, _dtype_name(b), tuple(b.shape)))
-            if _lib.is_device(b) != dev:
-                raise ValueError("out[%r] must live in the same memory space as wrk_chk" % k)
+    dev = _lib.is_device(wrk_chk)
+    want = dict(tmin=("int16", (nd, ny, nx)), tmax=("int16", (nd, ny, nx)), tmin_norm=("float32", (12, ny, nx)),
+                tmax_norm=("float32", (12, ny, nx)), tmin_se=("float32", (12, ny, nx)), tmax_se=("float32", (12, ny, nx)),
+                ninvalid=("int32", (ny, nx)), status=("uint8", (ny, nx)))
+    if not daily:                                             # normals only: tmin / tmax may be absent
+        want = {k: v for k, v in want.items() if k not in ("tmin", "tmax") or (out or {}).get(k) is not None}
+    bufs, _ = _result_buffers(want, out, wrk_chk.device if dev else None, wrk_dev=dev)
+    out = dict(tmin=None, tmax=None, **bufs) if out is None and not daily else bufs
     fn = lib.twxi_interp_chunk if wait else lib.twxi_interp_chunk_async
     check(fn(ctx_tmin.handle, ctx_tmax.handle, ptr(wrk_chk), int(ny), int(nx),
              ptr(out["tmin"]), ptr(out["tmax"]), ptr(out["tmin_norm"]), ptr(out["tmax_norm"]),
@@ -303,15 +276,16 @@ def _check_wrk_chk(wrk_chk):
     return int(wrk_chk.shape[1]), int(wrk_chk.shape[2])
 
 
-def _result_buffers(want, out, device):
+def _result_buffers(want, out, device, wrk_dev=None):
     """Result buffers {name: (dtype, shape)}: allocated when ``out`` is None (numpy on the host, or torch tensors on the CUDA
-    ``device``), otherwise checked like interp_chunk's (dtype, shape, one memory space).  Returns (buffers, on_device)."""
+    ``device``), otherwise checked (dtype, shape, one memory space: that of wrk_chk when ``wrk_dev`` gives it).  Returns
+    (buffers, on_device)."""
     if out is None:
         if device is None:
             return {k: np.empty(shp, dtype=dt) for k, (dt, shp) in want.items()}, False
         import torch
         return {k: torch.empty(shp, dtype=getattr(torch, dt), device=device) for k, (dt, shp) in want.items()}, True
-    dev = None
+    dev = wrk_dev
     for k, (dt, shp) in want.items():
         b = out.get(k)
         if b is None:
@@ -321,7 +295,8 @@ def _result_buffers(want, out, device):
         if dev is None:
             dev = _lib.is_device(b)
         elif _lib.is_device(b) != dev:
-            raise ValueError("out[%r] must live in the same memory space as the other result buffers" % k)
+            raise ValueError("out[%r] must live in the same memory space as %s"
+                             % (k, "the other result buffers" if wrk_dev is None else "wrk_chk"))
     return out, dev
 
 

@@ -123,16 +123,20 @@ static int run_knn(Ctx& c) {
                       nullptr, b.status, b.gy, b.gx);
 }
 
+// Device time of the five stages (knn, nngh_params, krig, gwr, fixer): event i is recorded where stage i starts, event 5
+// after the last.  A call whose work starts at stage `first` reports 0 for the stages before it.
 struct StageTimer {
     cudaEvent_t ev[6];
     bool on = false;
+    int first = 0;
     cudaStream_t s = 0;
-    void begin(cudaStream_t stream) {
+    void begin(cudaStream_t stream, int first_stage = 0) {
         on = g_timing != 0;
         s = stream;
+        first = first_stage;
         if (!on) return;
-        for (auto& e : ev) cudaEventCreate(&e);
-        cudaEventRecord(ev[0], s);
+        for (int i = first; i < 6; ++i) cudaEventCreate(&ev[i]);
+        cudaEventRecord(ev[first], s);
     }
     void mark(int i) { if (on) cudaEventRecord(ev[i], s); }
     void end(bool accumulate) {
@@ -140,35 +144,101 @@ struct StageTimer {
         cudaEventSynchronize(ev[5]);
         for (int i = 0; i < 5; ++i) {
             float ms = 0;
-            cudaEventElapsedTime(&ms, ev[i], ev[i + 1]);
+            if (i >= first) cudaEventElapsedTime(&ms, ev[i], ev[i + 1]);
             g_stage_ms[i] = accumulate ? g_stage_ms[i] + ms : ms;
         }
-        for (auto& e : ev) cudaEventDestroy(e);
+        for (int i = first; i < 6; ++i) cudaEventDestroy(ev[i]);
     }
 };
 
-// knn -> nngh_params -> krig -> gwr for the points already loaded in c.b
-static int run_variable(Ctx& c, bool daily, StageTimer* t) {
+// knn -> nngh_params -> krig -> gwr for the points already loaded in c.b.  The GWR step is the daily apply into c.b.daily
+// with `daily`, none without it, or with `hat` the hat rows of variable v (0 tmin, 1 tmax) into that tile.
+static int run_variable(Ctx& c, bool daily, StageTimer& t, TileState* hat = nullptr, int v = 0) {
     TWXI_TRY(run_knn(c));
-    if (t) t->mark(1);
+    t.mark(1);
     TWXI_TRY(launch_nngh_params(c, c.b, nullptr, nullptr, 0, 1, daily ? 1 : 0, 1));
-    if (t) t->mark(2);
+    t.mark(2);
     TWXI_TRY(launch_krig(c, c.b, 0, nullptr));
-    if (t) t->mark(3);
-    if (daily) TWXI_TRY(launch_gwr(c, c.b, 0, nullptr, 1, nullptr, 0, nullptr, nullptr, nullptr));
-    if (t) t->mark(4);
+    t.mark(3);
+    if (hat) {
+        const size_t n12 = (size_t)v * hat->ncell * 12;
+        TWXI_TRY(launch_gwr_hat_rows(c, c.b, hat->kh, hat->hk + n12, hat->hidx + n12 * hat->kh, hat->hz + n12 * hat->kh,
+                                     hat->hoff + n12));
+    } else if (daily) {
+        TWXI_TRY(launch_gwr(c, c.b, 0, nullptr, 1, nullptr, 0, nullptr, nullptr, nullptr));
+    }
+    t.mark(4);
     return TWXI_OK;
 }
 
 template <typename T>
-static int copy_out(Ctx& c, T* dst, const T* src, size_t count) {
-    if (dst && count) TWXI_CUDA(cudaMemcpyAsync(dst, src, count * sizeof(T), cudaMemcpyDefault, c.stream));
+static int copy_out(cudaStream_t s, T* dst, const T* src, size_t count) {
+    if (dst && count) TWXI_CUDA(cudaMemcpyAsync(dst, src, count * sizeof(T), cudaMemcpyDefault, s));
     return TWXI_OK;
 }
+
+// Calls f(field of a, the same field of b, element count) for each field of a pair's chunk outputs, in one fixed order.
+template <typename A, typename B, typename F>
+static int each_field(A& a, B& b, F f) {
+    const size_t nc = a.ncell;
+    for (int v = 0; v < 2; ++v) TWXI_TRY(f(a.q[v], b.q[v], a.ndays * nc));
+    for (int v = 0; v < 2; ++v) TWXI_TRY(f(a.norm[v], b.norm[v], 12 * nc));
+    for (int v = 0; v < 2; ++v) TWXI_TRY(f(a.se[v], b.se[v], 12 * nc));
+    TWXI_TRY(f(a.ninv, b.ninv, nc));
+    TWXI_TRY(f(a.st, b.st, nc));
+    for (int v = 0; v < 2; ++v) TWXI_TRY(f(a.mth[v], b.mth[v], a.nmth * nc));
+    return TWXI_OK;
+}
+
+static size_t piece_bytes(size_t bytes) { return (bytes + 255) & ~(size_t)255; }
+
+// Device twin *d of the caller's outputs o in s: one 256-byte aligned piece for each field that o gives, null otherwise.
+static int stage_out(Scratch& s, const ChunkOut& o, ChunkOut* d) {
+    *d = o;
+    size_t tot = 0;
+    each_field(o, *d, [&](auto* src, auto*&, size_t n) {
+        if (src) tot += piece_bytes(n * sizeof(*src));
+        return TWXI_OK;
+    });
+    char* p;
+    TWXI_TRY(s.get((void**)&p, tot));
+    return each_field(o, *d, [&](auto* src, auto*& dst, size_t n) {
+        if (src) {
+            dst = reinterpret_cast<decltype(src)>(p);
+            p += piece_bytes(n * sizeof(*src));
+        }
+        return TWXI_OK;
+    });
+}
+
+// Enqueues on s the copies of the device twin d to the caller's outputs o (null and empty fields are skipped).
+static int copy_out(cudaStream_t s, const ChunkOut& o, const ChunkOut& d) {
+    return each_field(d, o, [&](auto* src, auto* dst, size_t n) { return copy_out(s, dst, src, n); });
+}
+
+// A pair call enqueues the work of both variables on ctx_tmin's stream: ctx_tmax's stream points there for the scope of
+// the call, whichever way it returns.
+struct PairStream {
+    Ctx& cmax;
+    cudaStream_t saved;
+    PairStream(Ctx& cmin, Ctx& cmax_) : cmax(cmax_), saved(cmax_.stream) { cmax.stream = cmin.stream; }
+    ~PairStream() { cmax.stream = saved; }
+};
 
 static int finish(Ctx& c, int mem) {
     if (mem == TWXI_MEM_HOST) TWXI_CUDA(cudaStreamSynchronize(c.stream));
     return TWXI_OK;
+}
+
+// End of a point entry point: the points' status converted to uint8, the outputs that `outputs` enqueues, then the status.
+template <typename F>
+static int status_tail(Ctx& c, int npts, uint8_t* status, int mem, F outputs) {
+    uint8_t* st8;
+    TWXI_TRY(c.scratch[1].get((void**)&st8, npts));
+    TWXI_TRY(launch_status_to_u8(c.stream, npts, c.b.status, st8));
+    TWXI_TRY(outputs());
+    TWXI_TRY(copy_out(c.stream, status, st8, (size_t)npts));
+    return finish(c, mem);
 }
 
 int AsyncOut::init() {
@@ -195,12 +265,6 @@ void AsyncOut::destroy() {
     if (copy) cudaStreamDestroy(copy);
     if (h2d) cudaStreamDestroy(h2d);
     *this = AsyncOut();
-}
-
-template <typename T>
-static int copy_out_on(cudaStream_t s, T* dst, const T* src, size_t count) {
-    if (dst && count) TWXI_CUDA(cudaMemcpyAsync(dst, src, count * sizeof(T), cudaMemcpyDefault, s));
-    return TWXI_OK;
 }
 
 // Lay out the per-tile arrays of TileState in one allocation (256-byte aligned pieces).
@@ -507,14 +571,11 @@ int twxi_knn(twxi_ctx* c, int npts, const double* lat, const double* lon, const 
     if (out_wgt) TWXI_TRY(c->scratch[0].get((void**)&wgt, (size_t)npts * k1 * 8));
     TWXI_TRY(launch_knn(*c, npts, b.lat, b.lon, b.n_rm ? b.rm_idx : nullptr, b.n_rm, b.rm_zero, k1, b.idx, b.dist,
                         wgt, b.status));
-    uint8_t* st8;
-    TWXI_TRY(c->scratch[1].get((void**)&st8, npts));
-    TWXI_TRY(launch_status_to_u8(c->stream, npts, b.status, st8));
-    TWXI_TRY(copy_out(*c, out_idx, b.idx, (size_t)npts * k1));
-    TWXI_TRY(copy_out(*c, out_dist, b.dist, (size_t)npts * k1));
-    TWXI_TRY(copy_out(*c, out_wgt, wgt, (size_t)npts * k1));
-    TWXI_TRY(copy_out(*c, status, st8, (size_t)npts));
-    return finish(*c, mem);
+    return status_tail(*c, npts, status, mem, [&] {
+        TWXI_TRY(copy_out(c->stream, out_idx, b.idx, (size_t)npts * k1));
+        TWXI_TRY(copy_out(c->stream, out_dist, b.dist, (size_t)npts * k1));
+        return copy_out(c->stream, out_wgt, wgt, (size_t)npts * k1);
+    });
 }
 
 // k1 needed when the caller overrides neighbour counts (host arrays are scanned; device arrays use the maximum)
@@ -552,14 +613,11 @@ int twxi_nngh_params(twxi_ctx* c, const twxi_points* pts, int32_t* nnghs_norm, i
     Batch& b = c->b;
     TWXI_TRY(run_knn(*c));
     TWXI_TRY(launch_nngh_params(*c, b, nullptr, nullptr, 0, 1, 1, 1));
-    uint8_t* st8;
-    TWXI_TRY(c->scratch[1].get((void**)&st8, npts));
-    TWXI_TRY(launch_status_to_u8(c->stream, npts, b.status, st8));
-    if (nnghs_norm) TWXI_CUDA(cudaMemcpy2DAsync(nnghs_norm, 48, b.nn, 96, 48, npts, cudaMemcpyDefault, c->stream));
-    if (nnghs_anom) TWXI_CUDA(cudaMemcpy2DAsync(nnghs_anom, 48, b.nn + 12, 96, 48, npts, cudaMemcpyDefault, c->stream));
-    TWXI_TRY(copy_out(*c, vario, b.vario, (size_t)npts * 36));
-    TWXI_TRY(copy_out(*c, status, st8, (size_t)npts));
-    return finish(*c, mem);
+    return status_tail(*c, npts, status, mem, [&] {
+        if (nnghs_norm) TWXI_CUDA(cudaMemcpy2DAsync(nnghs_norm, 48, b.nn, 96, 48, npts, cudaMemcpyDefault, c->stream));
+        if (nnghs_anom) TWXI_CUDA(cudaMemcpy2DAsync(nnghs_anom, 48, b.nn + 12, 96, 48, npts, cudaMemcpyDefault, c->stream));
+        return copy_out(c->stream, vario, b.vario, (size_t)npts * 36);
+    });
 }
 
 int twxi_krig(twxi_ctx* c, const twxi_points* pts, int mth, const int32_t* nnghs_override,
@@ -569,9 +627,7 @@ int twxi_krig(twxi_ctx* c, const twxi_points* pts, int mth, const int32_t* nnghs
     TWXI_ARG(pts->elev && pts->lst, "elev and lst are required for kriging");
     TWXI_CUDA(cudaSetDevice(c->device));
     const int npts = pts->npts;
-    const bool need_smooth = nnghs_override == nullptr || vario_override == nullptr;
     TWXI_TRY(load_points(*c, pts, k1_for_override(*c, nnghs_override, npts, mem, nnghs_override == nullptr), false));
-    (void)need_smooth;
     if (npts == 0) return TWXI_OK;
     Batch& b = c->b;
     const int32_t* d_ovr;
@@ -584,18 +640,15 @@ int twxi_krig(twxi_ctx* c, const twxi_points* pts, int mth, const int32_t* nnghs
     TWXI_TRY(run_knn(*c));
     TWXI_TRY(launch_nngh_params(*c, b, d_ovr, nullptr, mth, 1, 0, vario_override ? 0 : 1));
     TWXI_TRY(launch_krig(*c, b, mth, d_vo));
-    uint8_t* st8;
-    double* tmp;
-    const size_t cnt = (size_t)npts * (mth ? 1 : 12);
-    TWXI_TRY(c->scratch[1].get((void**)&st8, npts));
-    TWXI_TRY(c->scratch[0].get((void**)&tmp, cnt * 16));
-    TWXI_TRY(launch_status_to_u8(c->stream, npts, b.status, st8));
-    TWXI_TRY(launch_gather_month(c->stream, npts, mth - 1, b.status, b.mean, tmp));
-    TWXI_TRY(launch_gather_month(c->stream, npts, mth - 1, b.status, b.var, tmp + cnt));
-    TWXI_TRY(copy_out(*c, mean, tmp, cnt));
-    TWXI_TRY(copy_out(*c, var, tmp + cnt, cnt));
-    TWXI_TRY(copy_out(*c, status, st8, (size_t)npts));
-    return finish(*c, mem);
+    return status_tail(*c, npts, status, mem, [&] {
+        double* tmp;
+        const size_t cnt = (size_t)npts * (mth ? 1 : 12);
+        TWXI_TRY(c->scratch[0].get((void**)&tmp, cnt * 16));
+        TWXI_TRY(launch_gather_month(c->stream, npts, mth - 1, b.status, b.mean, tmp));
+        TWXI_TRY(launch_gather_month(c->stream, npts, mth - 1, b.status, b.var, tmp + cnt));
+        TWXI_TRY(copy_out(c->stream, mean, tmp, cnt));
+        return copy_out(c->stream, var, tmp + cnt, cnt);
+    });
 }
 
 // vario [npts][12][3] -> caller's [npts][12|1][3] with NaN for failed points (and for months that were not requested)
@@ -604,7 +657,7 @@ static int copy_vario(Ctx& c, int npts, int mth, double* out) {
     double* tmp;
     TWXI_TRY(c.scratch[0].get((void**)&tmp, (size_t)npts * nm * 3 * 8));
     TWXI_TRY(launch_gather_vario(c.stream, npts, mth - 1, c.b.status, c.b.nn, c.b.vario, tmp));
-    return copy_out(c, out, tmp, (size_t)npts * nm * 3);
+    return copy_out(c.stream, out, tmp, (size_t)npts * nm * 3);
 }
 
 int twxi_fit_vario(twxi_ctx* c, const twxi_points* pts, int mth, const int32_t* nnghs_override, double* vario,
@@ -621,12 +674,7 @@ int twxi_fit_vario(twxi_ctx* c, const twxi_points* pts, int mth, const int32_t* 
     TWXI_TRY(run_knn(*c));
     TWXI_TRY(launch_nngh_params(*c, b, d_ovr, nullptr, mth, 1, 0, 0));
     TWXI_TRY(launch_vario_fit(*c, b, mth));
-    uint8_t* st8;
-    TWXI_TRY(c->scratch[1].get((void**)&st8, npts));
-    TWXI_TRY(launch_status_to_u8(c->stream, npts, b.status, st8));
-    TWXI_TRY(copy_vario(*c, npts, mth, vario));
-    TWXI_TRY(copy_out(*c, status, st8, (size_t)npts));
-    return finish(*c, mem);
+    return status_tail(*c, npts, status, mem, [&] { return copy_vario(*c, npts, mth, vario); });
 }
 
 int twxi_krig_all(twxi_ctx* c, const twxi_points* pts, const int32_t* nnghs, double* mean, double* var, double* vario,
@@ -644,19 +692,16 @@ int twxi_krig_all(twxi_ctx* c, const twxi_points* pts, const int32_t* nnghs, dou
     TWXI_TRY(launch_nngh_params(*c, b, d_ovr, nullptr, 0, 1, 0, 0));
     TWXI_TRY(launch_vario_fit(*c, b, 0));
     TWXI_TRY(launch_krig(*c, b, 0, nullptr));
-    uint8_t* st8;
-    double* tmp;
-    const size_t cnt = (size_t)npts * 12;
-    TWXI_TRY(c->scratch[1].get((void**)&st8, npts));
-    TWXI_TRY(c->scratch[3].get((void**)&tmp, cnt * 16));
-    TWXI_TRY(launch_status_to_u8(c->stream, npts, b.status, st8));
-    TWXI_TRY(launch_gather_month(c->stream, npts, -1, b.status, b.mean, tmp));
-    TWXI_TRY(launch_gather_month(c->stream, npts, -1, b.status, b.var, tmp + cnt));
-    TWXI_TRY(copy_out(*c, mean, tmp, cnt));
-    TWXI_TRY(copy_out(*c, var, tmp + cnt, cnt));
-    if (vario) TWXI_TRY(copy_vario(*c, npts, 0, vario));
-    TWXI_TRY(copy_out(*c, status, st8, (size_t)npts));
-    return finish(*c, mem);
+    return status_tail(*c, npts, status, mem, [&] {
+        double* tmp;
+        const size_t cnt = (size_t)npts * 12;
+        TWXI_TRY(c->scratch[3].get((void**)&tmp, cnt * 16));
+        TWXI_TRY(launch_gather_month(c->stream, npts, -1, b.status, b.mean, tmp));
+        TWXI_TRY(launch_gather_month(c->stream, npts, -1, b.status, b.var, tmp + cnt));
+        TWXI_TRY(copy_out(c->stream, mean, tmp, cnt));
+        TWXI_TRY(copy_out(c->stream, var, tmp + cnt, cnt));
+        return vario ? copy_vario(*c, npts, 0, vario) : TWXI_OK;
+    });
 }
 
 int twxi_gwr_hat(twxi_ctx* c, const twxi_points* pts, int mth, const int32_t* nnghs_override, int kmax, int32_t* k,
@@ -684,14 +729,11 @@ int twxi_gwr_hat(twxi_ctx* c, const twxi_points* pts, int mth, const int32_t* nn
     int32_t* d_k = reinterpret_cast<int32_t*>(tmp + nz * 12);
     TWXI_CUDA(cudaMemsetAsync(tmp, 0, nz * 12 + (size_t)npts * 4, c->stream));
     TWXI_TRY(launch_gwr(*c, b, mth, nullptr, 0, nullptr, kmax, d_k, d_idx, d_z));
-    uint8_t* st8;
-    TWXI_TRY(c->scratch[1].get((void**)&st8, npts));
-    TWXI_TRY(launch_status_to_u8(c->stream, npts, b.status, st8));
-    TWXI_TRY(copy_out(*c, z, d_z, nz));
-    TWXI_TRY(copy_out(*c, idx, d_idx, nz));
-    TWXI_TRY(copy_out(*c, k, d_k, (size_t)npts));
-    TWXI_TRY(copy_out(*c, status, st8, (size_t)npts));
-    return finish(*c, mem);
+    return status_tail(*c, npts, status, mem, [&] {
+        TWXI_TRY(copy_out(c->stream, z, d_z, nz));
+        TWXI_TRY(copy_out(c->stream, idx, d_idx, nz));
+        return copy_out(c->stream, k, d_k, (size_t)npts);
+    });
 }
 
 int twxi_gwr_mth(twxi_ctx* c, const twxi_points* pts, int mth, const int32_t* nnghs_override, const double* pt_norm,
@@ -717,12 +759,7 @@ int twxi_gwr_mth(twxi_ctx* c, const twxi_points* pts, int mth, const int32_t* nn
     TWXI_TRY(run_knn(*c));
     TWXI_TRY(launch_nngh_params(*c, b, nullptr, d_ovr, mth, 0, 1, 0));
     TWXI_TRY(launch_gwr(*c, b, mth, d_ptn, 0, d_out, 0, nullptr, nullptr, nullptr));
-    uint8_t* st8;
-    TWXI_TRY(c->scratch[1].get((void**)&st8, npts));
-    TWXI_TRY(launch_status_to_u8(c->stream, npts, b.status, st8));
-    TWXI_TRY(copy_out(*c, out, d_out, (size_t)npts * D));
-    TWXI_TRY(copy_out(*c, status, st8, (size_t)npts));
-    return finish(*c, mem);
+    return status_tail(*c, npts, status, mem, [&] { return copy_out(c->stream, out, d_out, (size_t)npts * D); });
 }
 
 int twxi_xval_anom(twxi_ctx* c, int npts, const int32_t* stn_idx, int n_counts, const int32_t* nnghs, double* bias,
@@ -752,14 +789,11 @@ int twxi_xval_anom(twxi_ctx* c, int npts, const int32_t* stn_idx, int n_counts, 
     TWXI_TRY(launch_gwr_xval(*c, b, d_idx, nnghs, n_counts, d_out));
     double* d_split = d_out + cnt * 3;
     TWXI_TRY(launch_split3(c->stream, cnt, d_out, b.status, n_counts * 12, d_split, d_split + cnt, d_split + 2 * cnt));
-    uint8_t* st8;
-    TWXI_TRY(c->scratch[1].get((void**)&st8, npts));
-    TWXI_TRY(launch_status_to_u8(c->stream, npts, b.status, st8));
-    TWXI_TRY(copy_out(*c, bias, d_split, cnt));
-    TWXI_TRY(copy_out(*c, mae, d_split + cnt, cnt));
-    TWXI_TRY(copy_out(*c, r2, d_split + 2 * cnt, cnt));
-    TWXI_TRY(copy_out(*c, status, st8, (size_t)npts));
-    return finish(*c, mem);
+    return status_tail(*c, npts, status, mem, [&] {
+        TWXI_TRY(copy_out(c->stream, bias, d_split, cnt));
+        TWXI_TRY(copy_out(c->stream, mae, d_split + cnt, cnt));
+        return copy_out(c->stream, r2, d_split + 2 * cnt, cnt);
+    });
 }
 
 int twxi_interp_points(twxi_ctx* c, const twxi_points* pts, double* daily, double* norms, double* se, double* var,
@@ -774,7 +808,7 @@ int twxi_interp_points(twxi_ctx* c, const twxi_points* pts, double* daily, doubl
     Batch& b = c->b;
     StageTimer t;
     t.begin(c->stream);
-    TWXI_TRY(run_variable(*c, daily != nullptr, &t));
+    TWXI_TRY(run_variable(*c, daily != nullptr, t));
     char* tmp;
     TWXI_TRY(c->scratch[0].get((void**)&tmp, (size_t)npts * (12 * 8 * 3 + 1)));
     double* d_norms = reinterpret_cast<double*>(tmp);
@@ -783,11 +817,11 @@ int twxi_interp_points(twxi_ctx* c, const twxi_points* pts, double* daily, doubl
     uint8_t* st8 = reinterpret_cast<uint8_t*>(d_var + (size_t)npts * 12);
     TWXI_TRY(launch_finalize_points(*c, b, daily ? b.daily : nullptr, d_norms, d_se, d_var, st8));
     t.mark(5);
-    TWXI_TRY(copy_out(*c, norms, d_norms, (size_t)npts * 12));
-    TWXI_TRY(copy_out(*c, se, d_se, (size_t)npts * 12));
-    TWXI_TRY(copy_out(*c, var, d_var, (size_t)npts * 12));
-    TWXI_TRY(copy_out(*c, status, st8, (size_t)npts));
-    if (daily) TWXI_TRY(copy_out(*c, daily, b.daily, (size_t)npts * c->ob.ndays));
+    TWXI_TRY(copy_out(c->stream, norms, d_norms, (size_t)npts * 12));
+    TWXI_TRY(copy_out(c->stream, se, d_se, (size_t)npts * 12));
+    TWXI_TRY(copy_out(c->stream, var, d_var, (size_t)npts * 12));
+    TWXI_TRY(copy_out(c->stream, status, st8, (size_t)npts));
+    if (daily) TWXI_TRY(copy_out(c->stream, daily, b.daily, (size_t)npts * c->ob.ndays));
     t.end(false);
     return finish(*c, mem);
 }
@@ -802,6 +836,16 @@ static int check_pair(twxi_ctx* a, twxi_ctx* b, bool daily) {
     return TWXI_OK;
 }
 
+// Workspaces of both variables for the ny x nx cells of a work chunk (unpack_chunk_kernel fills them).
+static int chunk_batches(Ctx& cmin, Ctx& cmax, int ny, int nx, bool need_daily) {
+    for (Ctx* c : {&cmin, &cmax}) {
+        TWXI_TRY(ensure_batch(*c, ny * nx, default_k1(*c), need_daily));
+        c->b.n_rm = 0; c->b.rm_zero = 0;
+        c->b.gy = ny; c->b.gx = nx;
+    }
+    return TWXI_OK;
+}
+
 int twxi_interp_cells(twxi_ctx* cmin, twxi_ctx* cmax, int ncells, const double* lat, const double* lon,
                       const double* elev, const double* tdi, const double* climdiv, const double* lst_tmin,
                       const double* lst_tmax, const int32_t* rm_idx_tmin, const int32_t* rm_idx_tmax, int n_rm,
@@ -811,57 +855,47 @@ int twxi_interp_cells(twxi_ctx* cmin, twxi_ctx* cmax, int ncells, const double* 
     TWXI_ARG(tmin && tmax && tmin_norms && tmax_norms && tmin_se && tmax_se && ninvalid && status, "null output");
     TWXI_TRY(check_pair(cmin, cmax, true));
     TWXI_CUDA(cudaSetDevice(cmin->device));
-    cudaStream_t saved = cmax->stream;
-    cmax->stream = cmin->stream;
-    int rc = TWXI_OK;
-    do {
-        // leave-out indices are context-local: the tmin and tmax station tables are different subsets of the DB
-        twxi_points pa{ncells, lat, lon, elev, tdi, lst_tmin, rm_idx_tmin, n_rm, rm_zero_dist};
-        twxi_points pb{ncells, lat, lon, elev, tdi, lst_tmax, rm_idx_tmax, n_rm, rm_zero_dist};
-        if ((rc = load_points(*cmin, &pa, default_k1(*cmin), true)) != TWXI_OK) break;
-        if ((rc = load_points(*cmax, &pb, default_k1(*cmax), true)) != TWXI_OK) break;
-        if (ncells == 0) break;
-        const int nd = cmin->ob.ndays;
-        if (climdiv) {
-            double* d_cd;
-            if ((rc = cmin->scratch[2].get((void**)&d_cd, (size_t)ncells * 8)) != TWXI_OK) break;
-            if (cudaMemcpyAsync(d_cd, climdiv, (size_t)ncells * 8, cudaMemcpyDefault, cmin->stream) != cudaSuccess) {
-                set_error("climdiv copy failed"); rc = TWXI_ERR_CUDA; break;
-            }
-            if ((rc = launch_cells_status(cmin->stream, ncells, d_cd, cmin->climdivs, cmin->n_climdivs, cmax->climdivs,
-                                          cmax->n_climdivs, cmin->b.status, cmax->b.status)) != TWXI_OK) break;
-        }
-        StageTimer ta, tb;
-        ta.begin(cmin->stream);
-        if ((rc = run_variable(*cmin, true, &ta)) != TWXI_OK) break;
-        ta.mark(5);
-        tb.begin(cmin->stream);
-        if ((rc = run_variable(*cmax, true, &tb)) != TWXI_OK) break;
-        char* tmp;
-        if ((rc = cmin->scratch[0].get((void**)&tmp, (size_t)ncells * (12 * 8 * 4 + 4 + 1))) != TWXI_OK) break;
-        double* d_nmin = reinterpret_cast<double*>(tmp);
-        double* d_nmax = d_nmin + (size_t)ncells * 12;
-        double* d_semin = d_nmax + (size_t)ncells * 12;
-        double* d_semax = d_semin + (size_t)ncells * 12;
-        int32_t* d_ninv = reinterpret_cast<int32_t*>(d_semax + (size_t)ncells * 12);
-        uint8_t* d_st = reinterpret_cast<uint8_t*>(d_ninv + ncells);
-        if ((rc = launch_fixer(*cmin, *cmax, ncells, fix_invalid, 1, d_st, d_nmin, d_nmax, d_semin, d_semax, nullptr,
-                               nullptr, nullptr, nullptr, nullptr, nullptr, d_ninv)) != TWXI_OK) break;
-        tb.mark(5);
-        if ((rc = copy_out(*cmin, tmin, cmin->b.daily, (size_t)ncells * nd)) != TWXI_OK) break;
-        if ((rc = copy_out(*cmin, tmax, cmax->b.daily, (size_t)ncells * nd)) != TWXI_OK) break;
-        if ((rc = copy_out(*cmin, tmin_norms, d_nmin, (size_t)ncells * 12)) != TWXI_OK) break;
-        if ((rc = copy_out(*cmin, tmax_norms, d_nmax, (size_t)ncells * 12)) != TWXI_OK) break;
-        if ((rc = copy_out(*cmin, tmin_se, d_semin, (size_t)ncells * 12)) != TWXI_OK) break;
-        if ((rc = copy_out(*cmin, tmax_se, d_semax, (size_t)ncells * 12)) != TWXI_OK) break;
-        if ((rc = copy_out(*cmin, ninvalid, d_ninv, (size_t)ncells)) != TWXI_OK) break;
-        if ((rc = copy_out(*cmin, status, d_st, (size_t)ncells)) != TWXI_OK) break;
-        ta.end(false);
-        tb.end(true);
-        rc = finish(*cmin, mem);
-    } while (0);
-    cmax->stream = saved;
-    return rc;
+    PairStream pair(*cmin, *cmax);
+    // leave-out indices are context-local: the tmin and tmax station tables are different subsets of the DB
+    twxi_points pa{ncells, lat, lon, elev, tdi, lst_tmin, rm_idx_tmin, n_rm, rm_zero_dist};
+    twxi_points pb{ncells, lat, lon, elev, tdi, lst_tmax, rm_idx_tmax, n_rm, rm_zero_dist};
+    TWXI_TRY(load_points(*cmin, &pa, default_k1(*cmin), true));
+    TWXI_TRY(load_points(*cmax, &pb, default_k1(*cmax), true));
+    if (ncells == 0) return TWXI_OK;
+    const int nd = cmin->ob.ndays;
+    if (climdiv) {
+        double* d_cd;
+        TWXI_TRY(cmin->scratch[2].get((void**)&d_cd, (size_t)ncells * 8));
+        TWXI_CUDA(cudaMemcpyAsync(d_cd, climdiv, (size_t)ncells * 8, cudaMemcpyDefault, cmin->stream));
+        TWXI_TRY(launch_cells_status(cmin->stream, ncells, d_cd, cmin->climdivs, cmin->n_climdivs, cmax->climdivs,
+                                     cmax->n_climdivs, cmin->b.status, cmax->b.status));
+    }
+    StageTimer ta, tb;
+    ta.begin(cmin->stream);
+    TWXI_TRY(run_variable(*cmin, true, ta));
+    ta.mark(5);
+    tb.begin(cmin->stream);
+    TWXI_TRY(run_variable(*cmax, true, tb));
+    const size_t n12 = (size_t)ncells * 12;
+    char* tmp;
+    TWXI_TRY(cmin->scratch[0].get((void**)&tmp, (size_t)ncells * (12 * 8 * 4 + 4 + 1)));
+    double* d_f8 = reinterpret_cast<double*>(tmp);          // normals of tmin, tmax, then se of tmin, tmax
+    ChunkOut d;
+    d.ninv = reinterpret_cast<int32_t*>(d_f8 + 4 * n12);
+    d.st = reinterpret_cast<uint8_t*>(d.ninv + ncells);
+    TWXI_TRY(launch_fixer(*cmin, *cmax, ncells, fix_invalid, 1, d, d_f8));
+    tb.mark(5);
+    TWXI_TRY(copy_out(cmin->stream, tmin, cmin->b.daily, (size_t)ncells * nd));
+    TWXI_TRY(copy_out(cmin->stream, tmax, cmax->b.daily, (size_t)ncells * nd));
+    TWXI_TRY(copy_out(cmin->stream, tmin_norms, d_f8, n12));
+    TWXI_TRY(copy_out(cmin->stream, tmax_norms, d_f8 + n12, n12));
+    TWXI_TRY(copy_out(cmin->stream, tmin_se, d_f8 + 2 * n12, n12));
+    TWXI_TRY(copy_out(cmin->stream, tmax_se, d_f8 + 3 * n12, n12));
+    TWXI_TRY(copy_out(cmin->stream, ninvalid, d.ninv, (size_t)ncells));
+    TWXI_TRY(copy_out(cmin->stream, status, d.st, (size_t)ncells));
+    ta.end(false);
+    tb.end(true);
+    return finish(*cmin, mem);
 }
 
 static int interp_chunk_impl(twxi_ctx* cmin, twxi_ctx* cmax, const double* wrk_chk, int ny, int nx, int16_t* tmin,
@@ -873,117 +907,72 @@ static int interp_chunk_impl(twxi_ctx* cmin, twxi_ctx* cmax, const double* wrk_c
     const bool daily = tmin != nullptr;
     TWXI_TRY(check_pair(cmin, cmax, daily));
     TWXI_CUDA(cudaSetDevice(cmin->device));
-    cudaStream_t saved = cmax->stream;
-    cmax->stream = cmin->stream;
+    PairStream pair(*cmin, *cmax);
     const int ncell = ny * nx;
-    int rc = TWXI_OK;
-    do {
-        if ((rc = ensure_batch(*cmin, ncell, default_k1(*cmin), daily)) != TWXI_OK) break;
-        if ((rc = ensure_batch(*cmax, ncell, default_k1(*cmax), daily)) != TWXI_OK) break;
-        cmin->b.n_rm = cmax->b.n_rm = 0;
-        cmin->b.rm_zero = cmax->b.rm_zero = 0;
-        cmin->b.gy = cmax->b.gy = ny;
-        cmin->b.gx = cmax->b.gx = nx;
-        const int nd = daily ? cmin->ob.ndays : 0;
-        const bool host = !(mem == TWXI_MEM_DEVICE);
-        // device staging of the chunk and of the results when the caller's buffers are on the host
-        const size_t wrk_bytes = (size_t)32 * ncell * 8;
-        const double* d_wrk = wrk_chk;
-        const bool acopy = async && host;                    // chunk and results travel on the copy streams
-        AsyncOut& ao = cmin->async;
-        if (acopy && (rc = ao.init()) != TWXI_OK) break;
-        if (acopy) {
-            double* w;
-            const int sl = ao.slot;
-            // The chunk submitted two calls ago used this slot.  Block the HOST until its work chunk has been read and its
-            // results are in the caller's buffers: this is what makes "valid after two further submissions" true
-            // (include/twxi.h).  The device still has the previous chunk queued, so no overlap is lost.
-            if (ao.inflight_in[sl] && cudaEventSynchronize(ao.loaded[sl]) != cudaSuccess) { set_error("event wait failed"); rc = TWXI_ERR_CUDA; break; }
-            ao.inflight_in[sl] = false;
-            if (ao.pending[sl] && cudaEventSynchronize(ao.copied[sl]) != cudaSuccess) { set_error("event wait failed"); rc = TWXI_ERR_CUDA; break; }
-            ao.pending[sl] = false;
-            if ((rc = ao.win[sl].get((void**)&w, wrk_bytes)) != TWXI_OK) break;
-            bool ok = true;
-            if (ao.consumed[sl]) ok = cudaStreamWaitEvent(ao.h2d, ao.unpacked[sl], 0) == cudaSuccess;    // slot free again
-            ok = ok && cudaMemcpyAsync(w, wrk_chk, wrk_bytes, cudaMemcpyHostToDevice, ao.h2d) == cudaSuccess;
-            ok = ok && cudaEventRecord(ao.loaded[sl], ao.h2d) == cudaSuccess;
-            ao.inflight_in[sl] = ok;
-            ok = ok && cudaStreamWaitEvent(cmin->stream, ao.loaded[sl], 0) == cudaSuccess;
-            if (!ok) { set_error("wrk_chk copy failed"); rc = TWXI_ERR_CUDA; break; }
-            d_wrk = w;
-        } else if (host) {
-            double* w;
-            if ((rc = cmin->scratch[2].get((void**)&w, wrk_bytes)) != TWXI_OK) break;
-            if (cudaMemcpyAsync(w, wrk_chk, wrk_bytes, cudaMemcpyHostToDevice, cmin->stream) != cudaSuccess) {
-                set_error("wrk_chk copy failed"); rc = TWXI_ERR_CUDA; break;
-            }
-            d_wrk = w;
-        }
-        const size_t q_bytes = (size_t)nd * ncell * 2, f_bytes = (size_t)12 * ncell * 4;
-        int16_t *d_qmin = tmin, *d_qmax = tmax;
-        float *d_fnmin = tmin_norm, *d_fnmax = tmax_norm, *d_fsemin = tmin_se, *d_fsemax = tmax_se;
-        int32_t* d_ninv = ninvalid;
-        uint8_t* d_st = status;
-        if (host) {
-            char* o;
-            Scratch& so = acopy ? ao.stage[ao.slot] : cmin->scratch[0];
-            if ((rc = so.get((void**)&o, 2 * q_bytes + 4 * f_bytes + (size_t)ncell * 5 + 64)) != TWXI_OK) break;
-            d_fnmin = reinterpret_cast<float*>(o); d_fnmax = d_fnmin + (size_t)12 * ncell;
-            d_fsemin = d_fnmax + (size_t)12 * ncell; d_fsemax = d_fsemin + (size_t)12 * ncell;
-            d_ninv = reinterpret_cast<int32_t*>(d_fsemax + (size_t)12 * ncell);
-            d_qmin = reinterpret_cast<int16_t*>(d_ninv + ncell);
-            d_qmax = d_qmin + (size_t)nd * ncell;
-            d_st = reinterpret_cast<uint8_t*>(d_qmax + (size_t)nd * ncell);
-        }
-        StageTimer ta, tb;
-        ta.begin(cmin->stream);
-        if ((rc = launch_unpack_chunk(cmin->stream, d_wrk, ny, nx, cmin->climdivs, cmin->n_climdivs, cmax->climdivs,
-                                      cmax->n_climdivs, cmin->b, cmax->b)) != TWXI_OK) break;
-        if (acopy) {
-            if (cudaEventRecord(ao.unpacked[ao.slot], cmin->stream) != cudaSuccess) { set_error("event record failed"); rc = TWXI_ERR_CUDA; break; }
-            ao.consumed[ao.slot] = true;
-        }
-        if ((rc = run_variable(*cmin, daily, &ta)) != TWXI_OK) break;
-        ta.mark(5);
-        tb.begin(cmin->stream);
-        if ((rc = run_variable(*cmax, daily, &tb)) != TWXI_OK) break;
-        if ((rc = launch_fixer(*cmin, *cmax, ncell, 1, daily ? 1 : 0, d_st, nullptr, nullptr, nullptr, nullptr, d_qmin,
-                               d_qmax, d_fnmin, d_fnmax, d_fsemin, d_fsemax, d_ninv)) != TWXI_OK) break;
-        tb.mark(5);
-        if (acopy) {
-            cudaStream_t cs = ao.copy;
-            if (cudaEventRecord(ao.done, cmin->stream) != cudaSuccess || cudaStreamWaitEvent(cs, ao.done, 0) != cudaSuccess) {
-                set_error("event record failed"); rc = TWXI_ERR_CUDA; break;
-            }
-            if ((rc = copy_out_on(cs, tmin, d_qmin, (size_t)nd * ncell)) != TWXI_OK) break;
-            if ((rc = copy_out_on(cs, tmax, d_qmax, (size_t)nd * ncell)) != TWXI_OK) break;
-            if ((rc = copy_out_on(cs, tmin_norm, d_fnmin, (size_t)12 * ncell)) != TWXI_OK) break;
-            if ((rc = copy_out_on(cs, tmax_norm, d_fnmax, (size_t)12 * ncell)) != TWXI_OK) break;
-            if ((rc = copy_out_on(cs, tmin_se, d_fsemin, (size_t)12 * ncell)) != TWXI_OK) break;
-            if ((rc = copy_out_on(cs, tmax_se, d_fsemax, (size_t)12 * ncell)) != TWXI_OK) break;
-            if ((rc = copy_out_on(cs, ninvalid, d_ninv, (size_t)ncell)) != TWXI_OK) break;
-            if ((rc = copy_out_on(cs, status, d_st, (size_t)ncell)) != TWXI_OK) break;
-            if (cudaEventRecord(ao.copied[ao.slot], cs) != cudaSuccess) { set_error("event record failed"); rc = TWXI_ERR_CUDA; break; }
-            ao.pending[ao.slot] = true;
-            ao.last = ao.slot;
-            ao.slot ^= 1;
-            ++ao.submitted;
-        } else if (host) {
-            if ((rc = copy_out(*cmin, tmin, d_qmin, (size_t)nd * ncell)) != TWXI_OK) break;
-            if ((rc = copy_out(*cmin, tmax, d_qmax, (size_t)nd * ncell)) != TWXI_OK) break;
-            if ((rc = copy_out(*cmin, tmin_norm, d_fnmin, (size_t)12 * ncell)) != TWXI_OK) break;
-            if ((rc = copy_out(*cmin, tmax_norm, d_fnmax, (size_t)12 * ncell)) != TWXI_OK) break;
-            if ((rc = copy_out(*cmin, tmin_se, d_fsemin, (size_t)12 * ncell)) != TWXI_OK) break;
-            if ((rc = copy_out(*cmin, tmax_se, d_fsemax, (size_t)12 * ncell)) != TWXI_OK) break;
-            if ((rc = copy_out(*cmin, ninvalid, d_ninv, (size_t)ncell)) != TWXI_OK) break;
-            if ((rc = copy_out(*cmin, status, d_st, (size_t)ncell)) != TWXI_OK) break;
-        }
-        ta.end(false);
-        tb.end(true);
-        if (!async) rc = finish(*cmin, mem);
-    } while (0);
-    cmax->stream = saved;
-    return rc;
+    TWXI_TRY(chunk_batches(*cmin, *cmax, ny, nx, daily));
+    const bool host = mem != TWXI_MEM_DEVICE;
+    // device staging of the chunk and of the results when the caller's buffers are on the host
+    const size_t wrk_bytes = (size_t)32 * ncell * 8;
+    const double* d_wrk = wrk_chk;
+    const bool acopy = async && host;                    // chunk and results travel on the copy streams
+    AsyncOut& ao = cmin->async;
+    if (acopy) {
+        TWXI_TRY(ao.init());
+        const int sl = ao.slot;
+        // The chunk submitted two calls ago used this slot.  Block the HOST until its work chunk has been read and its
+        // results are in the caller's buffers: this is what makes "valid after two further submissions" true
+        // (include/twxi.h).  The device still has the previous chunk queued, so no overlap is lost.
+        if (ao.inflight_in[sl]) TWXI_CUDA(cudaEventSynchronize(ao.loaded[sl]));
+        ao.inflight_in[sl] = false;
+        if (ao.pending[sl]) TWXI_CUDA(cudaEventSynchronize(ao.copied[sl]));
+        ao.pending[sl] = false;
+        double* w;
+        TWXI_TRY(ao.win[sl].get((void**)&w, wrk_bytes));
+        if (ao.consumed[sl]) TWXI_CUDA(cudaStreamWaitEvent(ao.h2d, ao.unpacked[sl], 0));    // slot free again
+        TWXI_CUDA(cudaMemcpyAsync(w, wrk_chk, wrk_bytes, cudaMemcpyHostToDevice, ao.h2d));
+        TWXI_CUDA(cudaEventRecord(ao.loaded[sl], ao.h2d));
+        ao.inflight_in[sl] = true;
+        TWXI_CUDA(cudaStreamWaitEvent(cmin->stream, ao.loaded[sl], 0));
+        d_wrk = w;
+    } else if (host) {
+        double* w;
+        TWXI_TRY(cmin->scratch[2].get((void**)&w, wrk_bytes));
+        TWXI_CUDA(cudaMemcpyAsync(w, wrk_chk, wrk_bytes, cudaMemcpyHostToDevice, cmin->stream));
+        d_wrk = w;
+    }
+    const ChunkOut o{{tmin, tmax}, {tmin_norm, tmax_norm}, {tmin_se, tmax_se}, ninvalid, status, {nullptr, nullptr},
+                     (size_t)ncell, daily ? (size_t)cmin->ob.ndays : 0};
+    ChunkOut d = o;
+    if (host) TWXI_TRY(stage_out(acopy ? ao.stage[ao.slot] : cmin->scratch[0], o, &d));
+    StageTimer ta, tb;
+    ta.begin(cmin->stream);
+    TWXI_TRY(launch_unpack_chunk(cmin->stream, d_wrk, ny, nx, cmin->climdivs, cmin->n_climdivs, cmax->climdivs,
+                                 cmax->n_climdivs, cmin->b, cmax->b));
+    if (acopy) {
+        TWXI_CUDA(cudaEventRecord(ao.unpacked[ao.slot], cmin->stream));
+        ao.consumed[ao.slot] = true;
+    }
+    TWXI_TRY(run_variable(*cmin, daily, ta));
+    ta.mark(5);
+    tb.begin(cmin->stream);
+    TWXI_TRY(run_variable(*cmax, daily, tb));
+    TWXI_TRY(launch_fixer(*cmin, *cmax, ncell, 1, daily ? 1 : 0, d));
+    tb.mark(5);
+    if (acopy) {
+        TWXI_CUDA(cudaEventRecord(ao.done, cmin->stream));
+        TWXI_CUDA(cudaStreamWaitEvent(ao.copy, ao.done, 0));
+        TWXI_TRY(copy_out(ao.copy, o, d));
+        TWXI_CUDA(cudaEventRecord(ao.copied[ao.slot], ao.copy));
+        ao.pending[ao.slot] = true;
+        ao.last = ao.slot;
+        ao.slot ^= 1;
+        ++ao.submitted;
+    } else if (host) {
+        TWXI_TRY(copy_out(cmin->stream, o, d));
+    }
+    ta.end(false);
+    tb.end(true);
+    return async ? TWXI_OK : finish(*cmin, mem);
 }
 
 int twxi_interp_chunk(twxi_ctx* cmin, twxi_ctx* cmax, const double* wrk_chk, int ny, int nx, int16_t* tmin,
@@ -1000,15 +989,15 @@ int twxi_interp_chunk_async(twxi_ctx* cmin, twxi_ctx* cmax, const double* wrk_ch
                              status, mem, true);
 }
 
-static int tile_begin_impl(twxi_ctx* cmin, twxi_ctx* cmax, const double* wrk_chk, int ny, int nx, int mem) {
+int twxi_tile_begin(twxi_ctx* cmin, twxi_ctx* cmax, const double* wrk_chk, int ny, int nx, int mem) {
+    TWXI_ARG(wrk_chk, "null argument");
+    TWXI_ARG(ny >= 1 && nx >= 1 && (long long)ny * nx <= (1 << 24), "bad chunk size");
+    TWXI_TRY(check_pair(cmin, cmax, true));
+    TWXI_CUDA(cudaSetDevice(cmin->device));
+    cmin->tile.open = false;                                  // a new begin discards an open tile
+    PairStream pair(*cmin, *cmax);
     const int ncell = ny * nx;
-    TWXI_TRY(ensure_batch(*cmin, ncell, default_k1(*cmin), false));
-    TWXI_TRY(ensure_batch(*cmax, ncell, default_k1(*cmax), false));
-    Ctx* cs[2] = {cmin, cmax};
-    for (Ctx* c : cs) {
-        c->b.n_rm = 0; c->b.rm_zero = 0;
-        c->b.gy = ny; c->b.gx = nx;
-    }
+    TWXI_TRY(chunk_batches(*cmin, *cmax, ny, nx, false));
     const double* d_wrk = wrk_chk;
     if (mem != TWXI_MEM_DEVICE) {
         double* w;
@@ -1021,27 +1010,18 @@ static int tile_begin_impl(twxi_ctx* cmin, twxi_ctx* cmax, const double* wrk_chk
     t.ny = ny; t.nx = nx; t.ncell = ncell;
     t.kh = std::max(cmin->b.k1, cmax->b.k1) - 1;              // k_anom < k1 of its context
     TWXI_TRY(tile_alloc(t));
-    StageTimer tm[2];
-    tm[0].begin(cmin->stream);
+    StageTimer ta, tb;
+    ta.begin(cmin->stream);
     TWXI_TRY(launch_unpack_chunk(cmin->stream, d_wrk, ny, nx, cmin->climdivs, cmin->n_climdivs, cmax->climdivs,
                                  cmax->n_climdivs, cmin->b, cmax->b));
-    for (int v = 0; v < 2; ++v) {                             // run_variable with hat rows instead of the daily apply
-        Ctx& c = *cs[v];
-        if (v) tm[1].begin(cmin->stream);
-        TWXI_TRY(run_knn(c));
-        tm[v].mark(1);
-        TWXI_TRY(launch_nngh_params(c, c.b, nullptr, nullptr, 0, 1, 1, 1));
-        tm[v].mark(2);
-        TWXI_TRY(launch_krig(c, c.b, 0, nullptr));
-        tm[v].mark(3);
-        const size_t n12 = (size_t)v * ncell * 12;
-        TWXI_TRY(launch_gwr_hat_rows(c, c.b, t.kh, t.hk + n12, t.hidx + n12 * t.kh, t.hz + n12 * t.kh, t.hoff + n12));
-        tm[v].mark(4);
-        if (v) TWXI_TRY(launch_tile_init(cmin->stream, t, cmin->b, cmax->b));
-        tm[v].mark(5);
-    }
-    tm[0].end(false);
-    tm[1].end(true);
+    TWXI_TRY(run_variable(*cmin, true, ta, &t, 0));
+    ta.mark(5);
+    tb.begin(cmin->stream);
+    TWXI_TRY(run_variable(*cmax, true, tb, &t, 1));
+    TWXI_TRY(launch_tile_init(cmin->stream, t, cmin->b, cmax->b));
+    tb.mark(5);
+    ta.end(false);
+    tb.end(true);
     t.cmax = cmax;
     t.gen_min = cmin->obs_gen; t.gen_max = cmax->obs_gen;
     t.ndays = cmin->ob.ndays;
@@ -1052,7 +1032,6 @@ static int tile_begin_impl(twxi_ctx* cmin, twxi_ctx* cmax, const double* wrk_chk
     return TWXI_OK;
 }
 
-// The calls after begin: an open tile of this pair whose observation records have not been replaced since.
 static int tile_check(twxi_ctx* cmin, twxi_ctx* cmax) {
     TWXI_ARG(cmin && cmax, "null ctx");
     const TileState& t = cmin->tile;
@@ -1086,9 +1065,10 @@ static MonthSpan month_span(const Ctx& c, int w0, int w1) {
     return m;
 }
 
-// One window of the open tile; with `mth`, also the monthly means of the runs that end in it (twxi_tile_days_mth).
-static int tile_days_impl(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, int16_t* tmin, int16_t* tmax, int mem,
-                          const MonthSpan* mth = nullptr, float* tmin_mth = nullptr, float* tmax_mth = nullptr) {
+// One window of the open tile into o.q; with `mth`, also the monthly means of the runs that end in it into o.mth
+// (twxi_tile_days_mth).
+static int tile_days_impl(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, ChunkOut o, int mem,
+                          const MonthSpan* mth = nullptr) {
     TileState& t = cmin->tile;
     WindowSpan w;
     w.w0 = t.next_day; w.nwin = ndays;
@@ -1104,79 +1084,20 @@ static int tile_days_impl(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, int16_t* tm
         if (w.g0 == w.g1) w.g0 = g;
         w.g1 = g + 1;
     }
-    const size_t nq = (size_t)ndays * t.ncell, nf = mth ? (size_t)mth->nmth * t.ncell : 0;
-    int16_t *d_qmin = tmin, *d_qmax = tmax;
-    float *d_fmin = tmin_mth, *d_fmax = tmax_mth;
-    if (mem != TWXI_MEM_DEVICE) {
-        TWXI_TRY(t.out.get((void**)&d_qmin, 2 * nq * 2 + 2 * nf * 4));
-        d_qmax = d_qmin + nq;
-        d_fmin = reinterpret_cast<float*>(d_qmax + nq);
-        d_fmax = d_fmin + nf;
-    }
-    cudaEvent_t ev[3];
-    const bool timing = stage_timing_on();
-    if (timing) {
-        for (auto& e : ev) cudaEventCreate(&e);
-        cudaEventRecord(ev[0], cmin->stream);
-    }
-    TWXI_TRY(launch_tile_window(cmin->stream, t, *cmin, *cmax, w, d_qmin, d_qmax, timing ? ev[1] : nullptr));
-    if (timing) {                                             // stage slots 3 (GWR daily apply) and 4 (fixer / quantise)
-        cudaEventRecord(ev[2], cmin->stream);
-        cudaEventSynchronize(ev[2]);
-        g_stage_ms[0] = g_stage_ms[1] = g_stage_ms[2] = 0.0f;
-        cudaEventElapsedTime(&g_stage_ms[3], ev[0], ev[1]);
-        cudaEventElapsedTime(&g_stage_ms[4], ev[1], ev[2]);
-        for (auto& e : ev) cudaEventDestroy(e);
-    }
-    if (mth) TWXI_TRY(launch_tile_month(cmin->stream, t, *cmin, w, *mth, d_qmin, d_qmax, d_fmin, d_fmax));
-    if (mem != TWXI_MEM_DEVICE) {
-        TWXI_TRY(copy_out(*cmin, tmin, d_qmin, nq));
-        TWXI_TRY(copy_out(*cmin, tmax, d_qmax, nq));
-        TWXI_TRY(copy_out(*cmin, tmin_mth, d_fmin, nf));
-        TWXI_TRY(copy_out(*cmin, tmax_mth, d_fmax, nf));
-    }
+    o.ncell = t.ncell; o.ndays = ndays; o.nmth = mth ? mth->nmth : 0;
+    ChunkOut d = o;
+    if (mem != TWXI_MEM_DEVICE) TWXI_TRY(stage_out(t.out, o, &d));
+    StageTimer tm;
+    tm.begin(cmin->stream, 3);                                // stage slots 3 (GWR daily apply) and 4 (fixer / quantise)
+    TWXI_TRY(launch_tile_apply(cmin->stream, t, *cmin, *cmax, w));
+    tm.mark(4);
+    TWXI_TRY(launch_tile_fix(cmin->stream, t, *cmin, w, d.q[0], d.q[1]));
+    tm.mark(5);
+    tm.end(false);
+    if (mth) TWXI_TRY(launch_tile_month(cmin->stream, t, *cmin, w, *mth, d.q[0], d.q[1], d.mth[0], d.mth[1]));
+    if (mem != TWXI_MEM_DEVICE) TWXI_TRY(copy_out(cmin->stream, o, d));
     t.next_day = w1;
     return finish(*cmin, mem);
-}
-
-static int tile_end_impl(twxi_ctx* cmin, float* tmin_norm, float* tmax_norm, float* tmin_se, float* tmax_se,
-                         int32_t* ninvalid, uint8_t* status, int mem) {
-    TileState& t = cmin->tile;
-    const size_t nc = (size_t)t.ncell, f = 12 * nc;
-    float *d_fnmin = tmin_norm, *d_fnmax = tmax_norm, *d_fsemin = tmin_se, *d_fsemax = tmax_se;
-    int32_t* d_ninv = ninvalid;
-    uint8_t* d_st = status;
-    if (mem != TWXI_MEM_DEVICE) {
-        char* o;
-        TWXI_TRY(t.out.get((void**)&o, 4 * f * 4 + nc * 5));
-        d_fnmin = reinterpret_cast<float*>(o); d_fnmax = d_fnmin + f; d_fsemin = d_fnmax + f; d_fsemax = d_fsemin + f;
-        d_ninv = reinterpret_cast<int32_t*>(d_fsemax + f);
-        d_st = reinterpret_cast<uint8_t*>(d_ninv + nc);
-    }
-    TWXI_TRY(launch_tile_end(cmin->stream, t, *cmin, d_fnmin, d_fnmax, d_fsemin, d_fsemax, d_ninv, d_st));
-    if (mem != TWXI_MEM_DEVICE) {
-        TWXI_TRY(copy_out(*cmin, tmin_norm, d_fnmin, f));
-        TWXI_TRY(copy_out(*cmin, tmax_norm, d_fnmax, f));
-        TWXI_TRY(copy_out(*cmin, tmin_se, d_fsemin, f));
-        TWXI_TRY(copy_out(*cmin, tmax_se, d_fsemax, f));
-        TWXI_TRY(copy_out(*cmin, ninvalid, d_ninv, nc));
-        TWXI_TRY(copy_out(*cmin, status, d_st, nc));
-    }
-    t.open = false;
-    return finish(*cmin, mem);
-}
-
-int twxi_tile_begin(twxi_ctx* cmin, twxi_ctx* cmax, const double* wrk_chk, int ny, int nx, int mem) {
-    TWXI_ARG(wrk_chk, "null argument");
-    TWXI_ARG(ny >= 1 && nx >= 1 && (long long)ny * nx <= (1 << 24), "bad chunk size");
-    TWXI_TRY(check_pair(cmin, cmax, true));
-    TWXI_CUDA(cudaSetDevice(cmin->device));
-    cmin->tile.open = false;                                  // a new begin discards an open tile
-    cudaStream_t saved = cmax->stream;
-    cmax->stream = cmin->stream;
-    const int rc = tile_begin_impl(cmin, cmax, wrk_chk, ny, nx, mem);
-    cmax->stream = saved;
-    return rc;
 }
 
 int twxi_tile_days(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, int16_t* tmin, int16_t* tmax, int mem) {
@@ -1185,7 +1106,7 @@ int twxi_tile_days(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, int16_t* tmin, int
     TWXI_ARG(ndays >= 1 && ndays <= cmin->tile.ndays - cmin->tile.next_day, "ndays must be 1 .. the days that remain");
     TWXI_CUDA(cudaSetDevice(cmin->device));
     cmin->tile.plain_days = true;
-    return tile_days_impl(cmin, cmax, ndays, tmin, tmax, mem);
+    return tile_days_impl(cmin, cmax, ndays, ChunkOut{{tmin, tmax}}, mem);
 }
 
 int twxi_tile_days_mth(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, int16_t* tmin, int16_t* tmax, int max_mth,
@@ -1208,7 +1129,9 @@ int twxi_tile_days_mth(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, int16_t* tmin,
         return TWXI_ERR_ARG;
     }
     TWXI_CUDA(cudaSetDevice(cmin->device));
-    TWXI_TRY(tile_days_impl(cmin, cmax, ndays, tmin, tmax, mem, &m, tmin_mth, tmax_mth));
+    ChunkOut o{{tmin, tmax}};
+    o.mth[0] = tmin_mth; o.mth[1] = tmax_mth;
+    TWXI_TRY(tile_days_impl(cmin, cmax, ndays, o, mem, &m));
     *nmth = m.nmth;
     return TWXI_OK;
 }
@@ -1217,12 +1140,20 @@ int twxi_tile_end(twxi_ctx* cmin, twxi_ctx* cmax, float* tmin_norm, float* tmax_
                   int32_t* ninvalid, uint8_t* status, int mem) {
     TWXI_TRY(tile_check(cmin, cmax));
     TWXI_ARG(tmin_norm && tmax_norm && tmin_se && tmax_se && ninvalid && status, "null argument");
-    if (cmin->tile.next_day != cmin->tile.ndays) {
+    TileState& t = cmin->tile;
+    if (t.next_day != t.ndays) {
         set_error("twxi_tile_end before every day of the record was emitted");
         return TWXI_ERR_STATE;
     }
     TWXI_CUDA(cudaSetDevice(cmin->device));
-    return tile_end_impl(cmin, tmin_norm, tmax_norm, tmin_se, tmax_se, ninvalid, status, mem);
+    const ChunkOut o{{nullptr, nullptr}, {tmin_norm, tmax_norm}, {tmin_se, tmax_se}, ninvalid, status, {nullptr, nullptr},
+                     (size_t)t.ncell};
+    ChunkOut d = o;
+    if (mem != TWXI_MEM_DEVICE) TWXI_TRY(stage_out(t.out, o, &d));
+    TWXI_TRY(launch_tile_end(cmin->stream, t, *cmin, d));
+    if (mem != TWXI_MEM_DEVICE) TWXI_TRY(copy_out(cmin->stream, o, d));
+    t.open = false;
+    return finish(*cmin, mem);
 }
 
 int twxi_interp_chunk_wait(twxi_ctx* cmin, int host_sync) {

@@ -86,13 +86,6 @@ struct FixerArgs {
     int32_t* ninvalid;
 };
 
-__device__ __forceinline__ int16_t quantize(double x) {
-    // step25:163-164  np.round(x, 2) / np.float32(0.01) stored into int16 (C truncation)
-    const double r = rint(x * 100.0) / 100.0;
-    const double v = r / (double)0.01f;
-    return (int16_t)(int)v;
-}
-
 __global__ void __launch_bounds__(128) fixer_kernel(FixerArgs a) {
     const int q = blockIdx.x * 4 + (threadIdx.x >> 5);
     const int lane = threadIdx.x & 31;
@@ -205,20 +198,19 @@ __global__ void __launch_bounds__(128) fixer_kernel(FixerArgs a) {
     }
 }
 
-int launch_fixer(Ctx& cmin, Ctx& cmax, int ncells, int fix_invalid, int have_daily, uint8_t* status,
-                 double* nmin, double* nmax, double* semin, double* semax,
-                 int16_t* qmin, int16_t* qmax, float* fnmin, float* fnmax, float* fsemin, float* fsemax,
-                 int32_t* ninvalid) {
+int launch_fixer(Ctx& cmin, Ctx& cmax, int ncells, int fix_invalid, int have_daily, const ChunkOut& out, double* f8) {
     if (ncells <= 0) return TWXI_OK;
+    const size_t n12 = (size_t)ncells * 12;
     FixerArgs a;
     a.ncell = ncells; a.ndays = cmin.ob.ndays; a.fix_invalid = fix_invalid; a.ob = cmin.ob;
     a.dmin = have_daily ? cmin.b.daily : nullptr;
     a.dmax = have_daily ? cmax.b.daily : nullptr;
     a.mean_min = cmin.b.mean; a.var_min = cmin.b.var; a.mean_max = cmax.b.mean; a.var_max = cmax.b.var;
     a.st_min = cmin.b.status; a.st_max = cmax.b.status;
-    a.status = status; a.nmin = nmin; a.nmax = nmax; a.semin = semin; a.semax = semax;
-    a.qmin = have_daily ? qmin : nullptr; a.qmax = have_daily ? qmax : nullptr;
-    a.fnmin = fnmin; a.fnmax = fnmax; a.fsemin = fsemin; a.fsemax = fsemax; a.ninvalid = ninvalid;
+    a.status = out.st;
+    a.nmin = f8; a.nmax = f8 ? f8 + n12 : nullptr; a.semin = f8 ? f8 + 2 * n12 : nullptr; a.semax = f8 ? f8 + 3 * n12 : nullptr;
+    a.qmin = have_daily ? out.q[0] : nullptr; a.qmax = have_daily ? out.q[1] : nullptr;
+    a.fnmin = out.norm[0]; a.fnmax = out.norm[1]; a.fsemin = out.se[0]; a.fsemax = out.se[1]; a.ninvalid = out.ninv;
     fixer_kernel<<<(ncells + 3) / 4, 128, 0, cmin.stream>>>(a);
     TWXI_LAUNCH_CHECK();
     return TWXI_OK;

@@ -292,15 +292,11 @@ int launch_gwr(Ctx& c, Batch& b, int mth, const double* pt_norm_override, int wr
     if (b.npts <= 0) return TWXI_OK;
     GwrArgs a;
     gwr_fill(a, c, b, mth);
-    a.st = c.st; a.ob = c.ob; a.npts = b.npts; a.k1 = b.k1; a.single_mth = mth >= 1 ? mth - 1 : -1;
-    a.idx = b.idx; a.dist = b.dist; a.nn = b.nn;
-    a.qlon = b.lon; a.qlat = b.lat; a.qelev = b.elev; a.qtdi = b.tdi; a.qlst = b.lst;
     a.pt_norm = pt_norm_override ? pt_norm_override : b.mean;
     a.pt_norm_single = pt_norm_override != nullptr;
     a.daily = write_daily ? b.daily : nullptr;
     a.out_month = out_month;
     a.kmax = kmax; a.hat_k = hat_k; a.hat_idx = hat_idx; a.hat_z = hat_z;
-    a.status = b.status;
     const long long items = (long long)b.npts * (mth >= 1 ? 1 : 12);
     const unsigned grid = (unsigned)((items + GWR_WARPS - 1) / GWR_WARPS);
     if (a.st.n > TWXI_GWR_PACKED_MIN_N) gwr_kernel<false, true><<<grid, GWR_THREADS, 0, c.stream>>>(a);

@@ -24,13 +24,6 @@ constexpr int REC_THREADS = 256;
 constexpr int REC_WARPS = REC_THREADS / 32;
 constexpr int REC_MAXK = 256;
 
-__device__ __forceinline__ int16_t quantize_rec(double x) {
-    // step25:163-164, as fixer.cu quantize()
-    const double r = rint(x * 100.0) / 100.0;
-    const double v = r / (double)0.01f;
-    return (int16_t)(int)v;
-}
-
 __global__ void tile_init_kernel(int ncell, const int32_t* st_min, const int32_t* st_max, int32_t* status,
                                  int32_t* ninv, double* carry, double* gpart, double* gacc) {
     const int q = blockIdx.x * blockDim.x + threadIdx.x;
@@ -231,13 +224,12 @@ __global__ void __launch_bounds__(128) tile_fix_kernel(FixArgs a) {
         a.ninv[q] += ninv;
     }
     for (int d = lane; d < a.nwin; d += 32) {
-        a.qmin[(size_t)d * P + q] = good ? quantize_rec(tmin[TAIL + d]) : TWXI_FILL_I2;
-        a.qmax[(size_t)d * P + q] = good ? quantize_rec(tmax[TAIL + d]) : TWXI_FILL_I2;
+        a.qmin[(size_t)d * P + q] = good ? quantize(tmin[TAIL + d]) : TWXI_FILL_I2;
+        a.qmax[(size_t)d * P + q] = good ? quantize(tmax[TAIL + d]) : TWXI_FILL_I2;
     }
 }
 
-int launch_tile_window(cudaStream_t s, TileState& t, const Ctx& cmin, const Ctx& cmax, const WindowSpan& w,
-                       int16_t* qmin, int16_t* qmax, cudaEvent_t after_apply) {
+int launch_tile_apply(cudaStream_t s, TileState& t, const Ctx& cmin, const Ctx& cmax, const WindowSpan& w) {
     const int wst = w.nwin + 2 * TAIL;
     void* p;
     const int rc = t.win.get(&p, (size_t)2 * t.ncell * wst * 8);
@@ -256,7 +248,12 @@ int launch_tile_window(cudaStream_t s, TileState& t, const Ctx& cmin, const Ctx&
         tile_apply_kernel<<<(unsigned)((items + REC_WARPS - 1) / REC_WARPS), REC_THREADS, 0, s>>>(a);
         TWXI_LAUNCH_CHECK();
     }
-    if (after_apply) TWXI_CUDA(cudaEventRecord(after_apply, s));
+    return TWXI_OK;
+}
+
+int launch_tile_fix(cudaStream_t s, TileState& t, const Ctx& cmin, const WindowSpan& w, int16_t* qmin, int16_t* qmax) {
+    const int wst = w.nwin + 2 * TAIL;
+    double* buf = static_cast<double*>(t.win.p);              // the window dailies of launch_tile_apply
     FixArgs f;
     f.ncell = t.ncell; f.nd = t.ndays; f.w0 = w.w0; f.nwin = w.nwin; f.la = w.la; f.wst = wst;
     f.dmin = buf; f.dmax = buf + (size_t)t.ncell * wst;
@@ -355,11 +352,11 @@ __global__ void tile_end_kernel(int ncell, int ngroups, const int* grp_len, cons
     }
 }
 
-int launch_tile_end(cudaStream_t s, TileState& t, const Ctx& cmin, float* fnmin, float* fnmax, float* fsemin,
-                    float* fsemax, int32_t* ninvalid, uint8_t* status) {
+int launch_tile_end(cudaStream_t s, TileState& t, const Ctx& cmin, const ChunkOut& out) {
     const int n = t.ncell * 12;
     tile_end_kernel<<<(n + 255) / 256, 256, 0, s>>>(t.ncell, cmin.ob.ngroups, cmin.ob.grp_len, t.status, t.ninv, t.mean,
-                                                    t.var, t.gacc, fnmin, fnmax, fsemin, fsemax, ninvalid, status);
+                                                    t.var, t.gacc, out.norm[0], out.norm[1], out.se[0], out.se[1],
+                                                    out.ninv, out.st);
     TWXI_LAUNCH_CHECK();
     return TWXI_OK;
 }

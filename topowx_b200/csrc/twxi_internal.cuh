@@ -220,10 +220,19 @@ int launch_unpack_chunk(cudaStream_t s, const double* wrk, int ny, int nx, const
                         const double* cd_b, int n_b, Batch& bmin, Batch& bmax);
 int launch_cells_status(cudaStream_t s, int ncell, const double* climdiv, const double* cd_a, int n_a,
                         const double* cd_b, int n_b, int32_t* sa, int32_t* sb);
-int launch_fixer(Ctx& cmin, Ctx& cmax, int ncells, int fix_invalid, int have_daily, uint8_t* status,
-                 double* nmin, double* nmax, double* semin, double* semax,
-                 int16_t* qmin, int16_t* qmax, float* fnmin, float* fnmax, float* fsemin, float* fsemax,
-                 int32_t* ninvalid);
+// Outputs of a Tmin/Tmax pair call on the ncell cells of a chunk, [v] = tmin, tmax.  A null field is not produced.
+struct ChunkOut {
+    int16_t* q[2] = {nullptr, nullptr};       // [ndays][ncell] quantised dailies
+    float* norm[2] = {nullptr, nullptr};      // [12][ncell] normals
+    float* se[2] = {nullptr, nullptr};        // [12][ncell] standard errors of the normals
+    int32_t* ninv = nullptr;                  // [ncell] Tmin >= Tmax days
+    uint8_t* st = nullptr;                    // [ncell] status of the pair
+    float* mth[2] = {nullptr, nullptr};       // [nmth][ncell] monthly means
+    size_t ncell = 0, ndays = 0, nmth = 0;
+};
+// f8 (twxi_interp_cells): f64 [4][ncells][12] normals of tmin, tmax, then se of tmin, tmax; may be null.
+int launch_fixer(Ctx& cmin, Ctx& cmax, int ncells, int fix_invalid, int have_daily, const ChunkOut& out,
+                 double* f8 = nullptr);
 int launch_finalize_points(Ctx& c, Batch& b, double* daily, double* norms, double* se, double* var_out,
                            uint8_t* status);
 // record.cu: the day windows of an open tile (TileState)
@@ -233,16 +242,16 @@ struct WindowSpan {
     int g0, g1;                // 1981-2010 groups overlapping the window
 };
 int launch_tile_init(cudaStream_t s, TileState& t, const Batch& bmin, const Batch& bmax);
-int launch_tile_window(cudaStream_t s, TileState& t, const Ctx& cmin, const Ctx& cmax, const WindowSpan& w,
-                       int16_t* qmin, int16_t* qmax, cudaEvent_t after_apply);
+// A window is the GWR apply of both variables into t.win, then the fixer / quantisation from t.win.
+int launch_tile_apply(cudaStream_t s, TileState& t, const Ctx& cmin, const Ctx& cmax, const WindowSpan& w);
+int launch_tile_fix(cudaStream_t s, TileState& t, const Ctx& cmin, const WindowSpan& w, int16_t* qmin, int16_t* qmax);
 // Month runs of the window [w0, w1) of twxi_tile_days_mth: runs g0 .. g1-1 overlap it, the first nmth of them end in it.
 struct MonthSpan {
     int g0, g1, nmth;
 };
 int launch_tile_month(cudaStream_t s, TileState& t, const Ctx& cmin, const WindowSpan& w, const MonthSpan& m,
                       const int16_t* qmin, const int16_t* qmax, float* fmin, float* fmax);
-int launch_tile_end(cudaStream_t s, TileState& t, const Ctx& cmin, float* fnmin, float* fnmax, float* fsemin,
-                    float* fsemax, int32_t* ninvalid, uint8_t* status);
+int launch_tile_end(cudaStream_t s, TileState& t, const Ctx& cmin, const ChunkOut& out);
 int launch_status_to_u8(cudaStream_t s, int n, const int32_t* in, uint8_t* out);
 int launch_gather_month(cudaStream_t s, int npts, int mth0, const int32_t* st, const double* src12, double* dst);
 int launch_gather_vario(cudaStream_t s, int npts, int mth0, const int32_t* st, const int32_t* nn, const double* src,
@@ -258,6 +267,14 @@ __device__ __forceinline__ int warp_max_i(int v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v = max(v, __shfl_xor_sync(0xffffffffu, v, o));
     return v;
+}
+
+// Output quantisation of step25:163-164, np.round(x, 2) / np.float32(0.01) stored into int16 (C truncation).  The
+// whole-record fixer and the day windows share it: their int16 dailies are byte-identical.
+__device__ __forceinline__ int16_t quantize(double x) {
+    const double r = rint(x * 100.0) / 100.0;
+    const double v = r / (double)0.01f;
+    return (int16_t)(int)v;
 }
 
 // Haversine "a" term with the reference's operation order and no FMA contraction
