@@ -52,7 +52,9 @@ extern "C" {
 #define TWXI_ST_TOO_FEW_STNS 3  /* IndexError: nnghs >= #candidate stations               station_select.py:164  */
 #define TWXI_ST_SINGULAR 4      /* singular / non-finite kriging or GWR system (R error, FloatingPointError);   */
                                 /* two co-located stations among a point's kriging neighbours are reported here, */
-                                /* and so is a GWR neighbour count below 6 (intercept + five trend predictors)   */
+                                /* and so is a kriging neighbour count below 5 (intercept + four drift columns:   */
+                                /* the trend matrix X'V^-1X is singular), a GWR neighbour count below 6           */
+                                /* (intercept + five trend predictors)                                            */
                                 /* and a variogram fit with fewer than 7 neighbours (OLS residuals of 5 trend     */
                                 /* coefficients need at least 2 degrees of freedom to carry a variogram)          */
 #define TWXI_ST_FIXER_EMPTY 5   /* 'No valid tmin/tmax in window'                          interp_tair.py:192     */
@@ -165,6 +167,8 @@ int twxi_nngh_params(twxi_ctx* ctx, const twxi_points* pts, int32_t* nnghs_norm,
  *   mth            1..12 = that month only (outputs [npts][1]); 0 = all months (outputs [npts][12])
  *   nnghs_override int32 [npts] or NULL (krig(nnghs=...)); vario_override float64 [npts][3] or NULL
  * Outputs float64: mean, var (kriging prediction variance), plus status uint8 [npts].
+ * A point whose neighbour count (override or smoothed, in any requested month) is below 5 gets TWXI_ST_SINGULAR: the
+ * trend has an intercept and four drift columns, so X'V^-1X is singular in exact arithmetic and there is no predictor.
  */
 int twxi_krig(twxi_ctx* ctx, const twxi_points* pts, int mth,
               const int32_t* nnghs_override, const double* vario_override,

@@ -26,6 +26,7 @@ STN_ID, MASK, BAD, CLIMDIV = "station_id", "mask", "bad", "climdiv"
 YEAR, MONTH = "YEAR", "MONTH"
 KRIG_TREND_VARS = (LON, LAT, ELEV, LST)            # interp_tair.py:46
 GWR_TREND_VARS = (LON, LAT, ELEV, TDI, LST)        # interp_tair.py:47
+KED_MIN_NNGHS = 1 + len(KRIG_TREND_VARS)           # fewer neighbours: the kriging trend matrix is singular
 DFLT_INIT_NNGHS = 100                              # interp_tair.py:51
 RADIAN_CONVERSION_FACTOR = 0.017453292519943295    # util_geo.py:21
 AVG_EARTH_RADIUS_KM = 6371.009                     # util_geo.py:22
@@ -201,8 +202,12 @@ def ked_gstat(ngh_lon, ngh_lat, ngh_X, ngh_y, pt_lon, pt_lat, pt_x, nug, psill, 
     The drift columns are centred on the prediction point and scaled before factorising; with an
     intercept in X this is an exact reparametrisation of the same predictor (tests compare it with
     the uncentred augmented system solved in extended precision).
-    Raises OracleError(ST_SINGULAR) where R would stop with a singular covariance matrix."""
+    Raises OracleError(ST_SINGULAR) where R would stop with a singular covariance matrix, and for fewer than 5
+    neighbours: X'V^-1X of the intercept and four drift columns is then singular in exact arithmetic, whatever the
+    rounded Cholesky factorisation of it says."""
     n = ngh_lon.size
+    if n < KED_MIN_NNGHS:
+        raise OracleError(ST_SINGULAR, "fewer than 5 neighbours: singular trend matrix")
     H = gcdist_sp(ngh_lon[:, None], ngh_lat[:, None], ngh_lon[None, :], ngh_lat[None, :])
     V = covariance_gstat(H, nug, psill, rng)
     V[np.diag_indices(n)] = nug + psill

@@ -10,6 +10,9 @@ namespace twxi {
 constexpr int SETUP_THREADS = 128;
 // the GWR fits an intercept and the five GWR_TREND_VARS (interp_tair.py:47): with fewer neighbours X'WX is singular
 constexpr int GWR_MIN_NNGHS = 1 + 5;
+// the kriging trend is an intercept and four drift columns (lon, lat, elev, lst; interp.R:256): with fewer neighbours
+// G = X'V^-1X is singular in exact arithmetic, and a rounded pivot must not decide it
+constexpr int KED_MIN_NNGHS = 1 + 4;
 
 struct SetupArgs {
     StnTable st;
@@ -97,7 +100,10 @@ __global__ void __launch_bounds__(SETUP_THREADS) nngh_params_kernel(SetupArgs a)
             if (!need_m) continue;
             if ((a.need_norm && knorm[m] < 0) || (a.need_anom && kanom[m] < 0)) { st = TWXI_ST_NO_NNGHS; break; }
             if (knorm[m] >= k1 || kanom[m] >= k1) { st = TWXI_ST_TOO_FEW_STNS; break; }
-            if ((a.need_norm && knorm[m] < 1) || (a.need_anom && kanom[m] < GWR_MIN_NNGHS)) { st = TWXI_ST_SINGULAR; break; }
+            if ((a.need_norm && knorm[m] < KED_MIN_NNGHS) || (a.need_anom && kanom[m] < GWR_MIN_NNGHS)) {
+                st = TWXI_ST_SINGULAR;
+                break;
+            }
             kmax = max(kmax, knorm[m]);
         }
     }
