@@ -59,7 +59,7 @@ extern "C" {
                                 /* coefficients need at least 2 degrees of freedom to carry a variogram)          */
 #define TWXI_ST_FIXER_EMPTY 5   /* 'No valid tmin/tmax in window'                          interp_tair.py:192     */
 #define TWXI_ST_CLIMDIV 6       /* KeyError: climate division unknown to the station DB    interp_tair.py:563     */
-#define TWXI_ST_KNN_TIES 7      /* more than 512 exact distance ties at the selection boundary (unsupported)     */
+#define TWXI_ST_KNN_TIES 7      /* more than 512 stations at a distance <= the (k+1)-th (boundary ties; twxi_knn) */
 #define TWXI_ST_LIMIT 8         /* neighbour count of the point exceeds TWXI_MAX_KRIG_NNGHS (kriging kernel limit) */
 #define TWXI_ST_MASKED 255      /* chunk cell with mask == 0: not a failure, nothing computed (step25:132)      */
 
@@ -126,7 +126,10 @@ int twxi_ctx_n_days(const twxi_ctx* ctx);
  *   rm_idx         [npts][n_rm] station indices to leave out (stns_rm), -1 = none; NULL if n_rm == 0
  *   rm_zero_dist   rm_zero_dist_stns flag (station_select.py:97-99)
  *   k1             candidates kept = nnghs + 1 (the (k+1)-th distance is the bandwidth, :164)
- * Outputs, in ascending (distance, station index) order – the caller re-sorts by station id (:179-182):
+ * Outputs: the first k1 stations of the order (distance in km, station index) ascending, i.e. argsort(kind='stable') of
+ * the distance vector with the distances this function returns; the caller re-sorts by station id (:179-182).  Stations
+ * at one km are ordered by index even where their haversine terms differ, so the result for k1 is the first k1 entries of
+ * the result for any larger k1.  TWXI_ST_KNN_TIES: more than 512 candidate stations lie at a distance <= the k1-th.
  *   out_idx  int32 [npts][k1], out_dist float64 [npts][k1] haversine km,
  *   out_wgt  float64 [npts][k1] bisquare weights (1-(d/d[k1-1])^2)^2 (:169), last entry 0; may be NULL
  *   status   uint8 [npts]

@@ -3,14 +3,19 @@
 //
 // One CTA per query point.  The whole station table (lat/lon in radians, cos(lat)) is streamed from L2, the
 // haversine "a" term of every station is written to a shared-memory key table (8 B per station), the
-// (k+1)-th smallest key is found with an 8-pass byte-wise radix select over that table, the keys <= that
-// threshold are compacted and sorted with a bitonic network, and only then the k+1 survivors get the
-// asin/sqrt that turns "a" into kilometres.  Ordering is (distance, station index) ascending: the
-// north_star tie-break, i.e. numpy argsort(kind='stable') of the reference's distance vector.
+// (k+1)-th smallest key is found with an 8-pass byte-wise radix select over that table, the threshold is widened
+// to the last key with the same distance in km, and only the keys <= that threshold get the asin/sqrt that turns
+// "a" into kilometres; they are compacted and sorted on (km, station index).
+//
+// Contract: the k+1 stations returned are the first k+1 of the order (km, station index) ascending, the north_star
+// tie-break, i.e. numpy argsort(kind='stable') of the distance vector, with km as this kernel computes it.  Distinct
+// keys often round to the same km (sqrt halves the relative spacing), so the selection boundary is decided in km, not
+// in "a": knn(k) is then a prefix of knn(k+1).  TWXI_ST_KNN_TIES: more than KNN_SEL = 512 candidate stations lie at a
+// distance <= the (k+1)-th distance.
 //
 // Bit-exactness: the "a" term uses the reference's operation order with explicit _rn intrinsics (no FMA
-// contraction).  a -> km is monotone (sqrt is correctly rounded, asin monotone up to its 1-ulp error); the
-// selected set is re-checked in km and re-sorted on (km, index) if asin ever breaks monotonicity.
+// contraction).  a -> km is monotone (sqrt is correctly rounded, asin monotone up to its 1-ulp error); the widening
+// takes every following key whose km is <= the threshold's, and the fast path's result is re-sorted on (km, index).
 #include <algorithm>
 #include <cstdlib>
 #include "twxi_internal.cuh"
@@ -77,7 +82,8 @@ __device__ void knn_query(const KnnArgs& a, const int q, unsigned long long* sme
     int* selidx = reinterpret_cast<int*>(selkey + KNN_SEL);    // [KNN_SEL]
     unsigned* hist = reinterpret_cast<unsigned*>(selidx + KNN_SEL);   // [256]
     __shared__ unsigned long long s_prefix;
-    __shared__ unsigned s_remaining, s_bincount, s_cnt;
+    __shared__ unsigned long long s_bkm[2];                    // fast path: km bits of ranks k1 - 1 and k1
+    __shared__ unsigned s_remaining, s_cnt;
 
     const int tid = threadIdx.x;
     const int k1 = a.k1;
@@ -113,13 +119,14 @@ __device__ void knn_query(const KnnArgs& a, const int q, unsigned long long* sme
         if (removed || !(av >= 0.0)) key = ~0ull;
         keys[t] = key;
     }
-    if (tid == 0) { s_prefix = 0ull; s_remaining = (unsigned)k1; s_cnt = 0u; }
+    if (tid == 0) { s_prefix = 0ull; s_remaining = (unsigned)k1; s_cnt = 0u; s_bkm[0] = 0ull; s_bkm[1] = ~0ull; }
     __syncthreads();
 
     // ---- fast path (pruned candidate lists): at most one candidate per thread.  Every key is ranked directly by counting
     // the strictly smaller keys (one 64-bit compare per pair, broadcast reads); no select passes, no compaction, two
     // barriers.  Equal keys get equal ranks: a collision among the first k1 ranks (an exact distance tie, decided by the
-    // station index) sends the query to the general path below, which sorts on (key, index).
+    // station index) sends the query to the general path below, which sorts on (km, index).  So does a best excluded key
+    // (rank k1) whose km equals that of the last selected one: the station index decides that boundary, not the key.
     bool fast_done = false;
     if (n <= KNN_THREADS) {
         const unsigned long long mk = tid < n ? keys[tid] : ~0ull;
@@ -138,9 +145,11 @@ __device__ void knn_query(const KnnArgs& a, const int q, unsigned long long* sme
         const int mi = cand ? (tid < n ? cand[tid] : 0) : tid;
         const bool mine = mk != ~0ull && rank < k1;
         if (mine) { selkey[rank] = mk; selidx[rank] = mi; }
+        if (mk != ~0ull && (rank == k1 - 1 || rank == k1))    // several writers only with equal keys: the same value
+            s_bkm[rank - (k1 - 1)] = (unsigned long long)__double_as_longlong(hav_km(__longlong_as_double((long long)mk)));
         __syncthreads();
         const int collide = __syncthreads_or(mine && selidx[rank] != mi);
-        fast_done = !collide;
+        fast_done = !collide && s_bkm[0] != s_bkm[1];
     }
     if (!fast_done) {
     // ---- phase 2: radix select of the k1-th smallest key -----------------------------------------
@@ -175,7 +184,6 @@ __device__ void knn_query(const KnnArgs& a, const int q, unsigned long long* sme
                     if (r <= c[i]) {
                         s_prefix = prefix | ((unsigned long long)(tid * 8 + i) << shift);
                         s_remaining = r;
-                        s_bincount = c[i];
                         break;
                     }
                     r -= c[i];
@@ -184,33 +192,39 @@ __device__ void knn_query(const KnnArgs& a, const int q, unsigned long long* sme
         }
         __syncthreads();
     }
-    const unsigned long long T = s_prefix;
+    unsigned long long T = s_prefix;
     if (T == ~0ull) {   // fewer than k1 candidate stations: IndexError at station_select.py:164
         if (tid == 0) a.status[q] = TWXI_ST_TOO_FEW_STNS;
         return;
     }
-    const unsigned count_le = (unsigned)k1 - s_remaining + s_bincount;
-    if (count_le > (unsigned)KNN_SEL) {
-        if (tid == 0) a.status[q] = TWXI_ST_KNN_TIES;
-        return;
-    }
+    // keys that differ can round to the km of the k1-th smallest key: take them all, so that (km, index) decides the
+    // boundary (a few nextafter steps; every thread computes the same T)
+    const double Tkm = hav_km(__longlong_as_double((long long)T));
+    while (hav_km(__longlong_as_double((long long)(T + 1))) <= Tkm) ++T;
 
-    // ---- phase 3: compact keys <= T, sort by (key, index) -----------------------------------------
-    int P = 32;
-    while (P < (int)count_le) P <<= 1;
-    for (int t = tid; t < P; t += KNN_THREADS) { selkey[t] = ~0ull; selidx[t] = 0x7fffffff; }
+    // ---- phase 3: compact keys <= T as (km, index), sort -------------------------------------------
+    for (int t = tid; t < KNN_SEL; t += KNN_THREADS) { selkey[t] = ~0ull; selidx[t] = 0x7fffffff; }
     __syncthreads();
     for (int s = tid; s < n; s += KNN_THREADS) {
         unsigned long long k = keys[s];
         if (k <= T) {
             unsigned p = atomicAdd(&s_cnt, 1u);
-            selkey[p] = k;
-            selidx[p] = cand ? cand[s] : s;
+            if (p < (unsigned)KNN_SEL) {
+                selkey[p] = (unsigned long long)__double_as_longlong(hav_km(__longlong_as_double((long long)k)));
+                selidx[p] = cand ? cand[s] : s;
+            }
         }
     }
     __syncthreads();
+    const unsigned count_le = s_cnt;
+    if (count_le > (unsigned)KNN_SEL) {
+        if (tid == 0) a.status[q] = TWXI_ST_KNN_TIES;
+        return;
+    }
+    int P = 32;
+    while (P < (int)count_le) P <<= 1;
     if (count_le <= (unsigned)KNN_THREADS) {
-        // rank by counting: every survivor counts the survivors that precede it in (key, index) order — no barriers,
+        // rank by counting: every survivor counts the survivors that precede it in (km, index) order — no barriers,
         // broadcast shared-memory reads; pairs are distinct, so the ranks are a permutation
         unsigned long long mk = 0ull;
         int mi = 0, rank = 0;
@@ -227,9 +241,9 @@ __device__ void knn_query(const KnnArgs& a, const int q, unsigned long long* sme
     }
     }   // general path
 
-    // ---- phase 4: kilometres for the k1 survivors; verify (km, index) order ---------------------------
+    // ---- phase 4: kilometres for the fast path's k1 survivors; verify (km, index) order -------------
     int bad = 0;
-    if (tid < k1) {
+    if (fast_done && tid < k1) {
         double d = hav_km(__longlong_as_double((long long)selkey[tid]));
         selkey[tid] = (unsigned long long)__double_as_longlong(d);
     }
