@@ -1,11 +1,12 @@
 """Every GWR kernel instance against an extended-precision solve of the reference's formula.
 
-gwr_kernel is compiled for the daily values (gwr_mth), the leave-one-out statistics (xval_anom) and the hat rows of the
-record path (tile_begin), each with the separate-array gather and with the packed 64-byte station rows used above
-TWXI_GWR_PACKED_MIN_N stations; tile_apply_kernel repeats the day loop.  The referee here is not the float64 oracle
-(which inverts the uncentred X'WX, condition up to ~1e15 on these neighbourhoods, and is itself off by up to 2e-6 C) but
-``gwr_exact``: the same formula in 40-digit arithmetic, rounded once.  Each tolerance comes from the problem's own
-conditioning, so a kernel that drops precision anywhere (a float accumulator, a wrong constant, a lost neighbour) fails.
+gwr_kernel is compiled for the daily values (gwr_mth), the leave-one-out statistics (xval_anom) and the hat rows
+(gwr_hat and the record path, tile_begin), each with the separate-array gather and with the packed 64-byte station rows
+used above TWXI_GWR_PACKED_MIN_N stations; tile_apply_kernel sums the day loop with the same hat_dot.  The referee here
+is not the float64 oracle (which inverts the uncentred X'WX, condition up to ~1e15 on these neighbourhoods, and is itself
+off by up to 2e-6 C) but ``gwr_exact``: the same formula in 40-digit arithmetic, rounded once.  Each tolerance comes from
+the problem's own conditioning, so a kernel that drops precision anywhere (a float accumulator, a wrong constant, a lost
+neighbour) fails.
 
 Neighbour counts cover k mod 8 and k mod 16 (the 8-, 4- and 1-wide passes of the day loop, the padded DMMA staging),
 the extremes 6 and TWXI_MAX_NNGHS = 255, and k = 1..5 (fewer stations than the six coefficients: TWXI_ST_SINGULAR).

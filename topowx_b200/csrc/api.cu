@@ -162,10 +162,10 @@ static int run_variable(Ctx& c, bool daily, StageTimer& t, TileState* hat = null
     t.mark(3);
     if (hat) {
         const size_t n12 = (size_t)v * hat->ncell * 12;
-        TWXI_TRY(launch_gwr_hat_rows(c, c.b, hat->kh, hat->hk + n12, hat->hidx + n12 * hat->kh, hat->hz + n12 * hat->kh,
-                                     hat->hoff + n12));
+        TWXI_TRY(launch_gwr_hat_rows(c, c.b, 0, hat->kh, hat->hk + n12, hat->hidx + n12 * hat->kh,
+                                     hat->hz + n12 * hat->kh, hat->hoff + n12));
     } else if (daily) {
-        TWXI_TRY(launch_gwr(c, c.b, 0, nullptr, 1, nullptr, 0, nullptr, nullptr, nullptr));
+        TWXI_TRY(launch_gwr(c, c.b, 0, nullptr, 1, nullptr));
     }
     t.mark(4);
     return TWXI_OK;
@@ -728,7 +728,7 @@ int twxi_gwr_hat(twxi_ctx* c, const twxi_points* pts, int mth, const int32_t* nn
     int32_t* d_idx = reinterpret_cast<int32_t*>(tmp + nz * 8);
     int32_t* d_k = reinterpret_cast<int32_t*>(tmp + nz * 12);
     TWXI_CUDA(cudaMemsetAsync(tmp, 0, nz * 12 + (size_t)npts * 4, c->stream));
-    TWXI_TRY(launch_gwr(*c, b, mth, nullptr, 0, nullptr, kmax, d_k, d_idx, d_z));
+    TWXI_TRY(launch_gwr_hat_rows(*c, b, mth, kmax, d_k, d_idx, d_z, nullptr));
     return status_tail(*c, npts, status, mem, [&] {
         TWXI_TRY(copy_out(c->stream, z, d_z, nz));
         TWXI_TRY(copy_out(c->stream, idx, d_idx, nz));
@@ -758,7 +758,7 @@ int twxi_gwr_mth(twxi_ctx* c, const twxi_points* pts, int mth, const int32_t* nn
     TWXI_CUDA(cudaMemsetAsync(d_out, 0xff, (size_t)npts * D * 8, c->stream));   // NaN for failed points
     TWXI_TRY(run_knn(*c));
     TWXI_TRY(launch_nngh_params(*c, b, nullptr, d_ovr, mth, 0, 1, 0));
-    TWXI_TRY(launch_gwr(*c, b, mth, d_ptn, 0, d_out, 0, nullptr, nullptr, nullptr));
+    TWXI_TRY(launch_gwr(*c, b, mth, d_ptn, 0, d_out));
     return status_tail(*c, npts, status, mem, [&] { return copy_out(c->stream, out, d_out, (size_t)npts * D); });
 }
 

@@ -102,33 +102,7 @@ __global__ void __launch_bounds__(128) fixer_kernel(FixerArgs a) {
 
     if (st == TWXI_ST_OK && tmin && a.fix_invalid) {
         // invalid_days = nonzero(tmin >= tmax) on the unfixed series (interp_tair.py:171)
-        for (int d0 = 0; d0 < nd && st == TWXI_ST_OK; d0 += 32) {
-            const int d = d0 + lane;
-            const bool inv = d < nd && tmin[d] >= tmax[d];
-            unsigned mask = __ballot_sync(0xffffffffu, inv);
-            ninv += __popc(mask);
-            while (mask) {
-                const int x = d0 + __ffs(mask) - 1;
-                mask &= mask - 1;
-                const int dd = x - 15 + lane;                 // window x-15 .. x+15 (tail=15, :177-183)
-                double diff = 0.0;
-                int ok = 0;
-                if (lane < 31 && dd >= 0 && dd < nd) {
-                    const double lo = tmin[dd], hi = tmax[dd];
-                    if (lo < hi) { diff = hi - lo; ok = 1; }
-                }
-                const double sum = warp_sum(diff);
-                const int cnt = __popc(__ballot_sync(0xffffffffu, ok));
-                if (cnt == 0) { st = TWXI_ST_FIXER_EMPTY; break; }     // 'No valid tmin/tmax in window' :192
-                if (lane == 0) {
-                    const double tavg = (tmin[x] + tmax[x]) / 2.0;
-                    const double half = (sum / cnt) / 2.0;
-                    tmin[x] = tavg - half;
-                    tmax[x] = tavg + half;
-                }
-                __syncwarp();
-            }
-        }
+        ninv = fix_inverted(tmin, tmax, 0, 0, nd, nd, lane, st);
         recompute = st == TWXI_ST_OK && ninv > 0;
     }
 
@@ -147,7 +121,7 @@ __global__ void __launch_bounds__(128) fixer_kernel(FixerArgs a) {
                     const int g = y * 12 + m;
                     const int s0 = a.ob.grp_start[g], len = a.ob.grp_len[g];
                     double smin = 0.0, smax = 0.0;
-                    for (int d = lane; d < len; d += 32) { smin += tmin[s0 + d]; smax += tmax[s0 + d]; }
+                    group_lane_days(0, len, lane, [&](int o) { smin += tmin[s0 + o]; smax += tmax[s0 + o]; });
                     smin = warp_sum(smin); smax = warp_sum(smax);
                     accmin += smin / len;                     // len == 0 -> NaN, like np.mean of an empty slice
                     accmax += smax / len;

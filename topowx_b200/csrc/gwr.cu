@@ -11,7 +11,7 @@
 // the kriging kernel (chol8_inverse_t), and the hat row is kept in shared memory while the warp streams the month's
 // days: lanes = days, neighbours gathered from the station-major,
 // month-major observation table (coalesced 128 B per neighbour, L2 resident).
-// One warp per (point, month); no intermediate hat rows go to HBM unless the caller asks for them.
+// One warp per (point, month); hat rows go to HBM only from the HAT instance (twxi_tile_begin, twxi_gwr_hat).
 #include "twxi_internal.cuh"
 
 #ifndef TWXI_GWR_PACKED_MIN_N
@@ -38,7 +38,7 @@ struct GwrArgs {
     int pt_norm_single;
     double* daily;             // [npts][ndays] chronological, or null
     double* out_month;         // [npts][D_m] month order, or null
-    int kmax;                  // hat outputs (null = off)
+    int kmax;                  // HAT instance: row length of hat_idx / hat_z
     int32_t* hat_k;
     int32_t* hat_idx;
     double* hat_z;
@@ -50,12 +50,13 @@ struct GwrArgs {
     const int32_t* xv_self;    // [npts] station index of the point, or null
     double* xv_out;            // [npts][xv_nc][12][3]
     int xv_nc, xv_ci;
-    double* hat_off;           // HAT instance: [npts][12] pt_norm - z . norm
+    double* hat_off;           // HAT instance: pt_norm - z . norm, or null
 };
 
-// HAT: hat rows of every (point, month) to hat_k / hat_off [npts][12] and hat_idx / hat_z [npts][12][kmax], no daily
-// values (the day windows of twxi_tile_days apply them).  A separate instance, so that the production kernel carries no
-// branch for it: z and the offset are bitwise what the production instance applies to the days.
+// HAT: hat rows of every (point, month) to hat_k / hat_off [npts][12] and hat_idx / hat_z [npts][12][kmax] ([npts] and
+// [npts][kmax] for a single month), no daily values (the day windows of twxi_tile_days apply them; twxi_gwr_hat returns
+// them).  A separate instance, so that the production kernel carries no branch for it: z and the offset are bitwise what
+// the production instance applies to the days.
 template <bool XVAL, bool PACKED, bool HAT = false>
 __global__ void __launch_bounds__(GWR_THREADS, TWXI_GWR_MINB) gwr_kernel(GwrArgs a) {
     __shared__ __align__(16) double s_z[GWR_WARPS][GWR_MAXK];
@@ -148,6 +149,7 @@ __global__ void __launch_bounds__(GWR_THREADS, TWXI_GWR_MINB) gwr_kernel(GwrArgs
 
     // ---- hat row z_j = w_j * (x_j . u) and offset pt_norm - z . norm -------------------------------------
     const size_t nd = (size_t)a.ob.ndays;
+    const size_t row = nm == 1 ? q : (size_t)q * 12 + m;     // HAT: hat row of (q, m)
     double zn = 0.0;
     for (int j = lane; j < k; j += 32) {
         const int s = s_off[warp][j];
@@ -171,26 +173,19 @@ __global__ void __launch_bounds__(GWR_THREADS, TWXI_GWR_MINB) gwr_kernel(GwrArgs
         s_off[warp][j] = s * (int)nd;
         zn += zj * nrm;
         if constexpr (HAT) {
-            const size_t o = ((size_t)q * 12 + m) * a.kmax + j;
-            a.hat_z[o] = zj;
-            a.hat_idx[o] = s;
-        } else if (a.hat_z && j < a.kmax) {                   // (device-resident overrides are not scanned on the host)
-            a.hat_z[(size_t)q * a.kmax + j] = zj;
-            a.hat_idx[(size_t)q * a.kmax + j] = s;
+            a.hat_z[row * a.kmax + j] = zj;
+            a.hat_idx[row * a.kmax + j] = s;
         }
     }
     zn = warp_sum(zn);
     if constexpr (HAT) {
         if (lane == 0) {
-            const double ptn = a.pt_norm[(size_t)q * 12 + m];
-            a.hat_k[(size_t)q * 12 + m] = k;
-            a.hat_off[(size_t)q * 12 + m] = ptn - zn;
+            a.hat_k[row] = k;
+            if (a.hat_off) a.hat_off[row] = a.pt_norm[(size_t)q * 12 + m] - zn;
         }
         return;
     }
-    if (a.hat_k && lane == 0) a.hat_k[q] = k;
     __syncwarp();
-    if (!XVAL && !a.daily && !a.out_month) return;
 
     // ---- daily values: lanes = days of the month, neighbours gathered from the station-major obs table ------------
     const int self = XVAL ? a.xv_self[q] : 0;
@@ -202,38 +197,7 @@ __global__ void __launch_bounds__(GWR_THREADS, TWXI_GWR_MINB) gwr_kernel(GwrArgs
         const int d = d0 + lane;
         const bool valid = d < D;
         const float* col = a.ob.obsT + p0 + (valid ? d : 0);
-        double acc0 = 0.0, acc1 = 0.0, acc2 = 0.0, acc3 = 0.0;
-        int j = 0;
-        for (; j + 7 < k; j += 8) {                           // eight gathers in flight per pass (same order of the sums)
-            const int4 o4 = *reinterpret_cast<const int4*>(&s_off[warp][j]);
-            const int4 o8 = *reinterpret_cast<const int4*>(&s_off[warp][j + 4]);
-            const float f0 = col[o4.x], f1 = col[o4.y], f2 = col[o4.z], f3 = col[o4.w];
-            const float f4 = col[o8.x], f5 = col[o8.y], f6 = col[o8.z], f7 = col[o8.w];
-            const double2 za = *reinterpret_cast<const double2*>(&s_z[warp][j]);
-            const double2 zb = *reinterpret_cast<const double2*>(&s_z[warp][j + 2]);
-            const double2 zc = *reinterpret_cast<const double2*>(&s_z[warp][j + 4]);
-            const double2 zd = *reinterpret_cast<const double2*>(&s_z[warp][j + 6]);
-            acc0 = fma(za.x, (double)f0, acc0);
-            acc1 = fma(za.y, (double)f1, acc1);
-            acc2 = fma(zb.x, (double)f2, acc2);
-            acc3 = fma(zb.y, (double)f3, acc3);
-            acc0 = fma(zc.x, (double)f4, acc0);
-            acc1 = fma(zc.y, (double)f5, acc1);
-            acc2 = fma(zd.x, (double)f6, acc2);
-            acc3 = fma(zd.y, (double)f7, acc3);
-        }
-        for (; j + 3 < k; j += 4) {                           // four gathers in flight per pass
-            const int4 o4 = *reinterpret_cast<const int4*>(&s_off[warp][j]);
-            const float f0 = col[o4.x], f1 = col[o4.y], f2 = col[o4.z], f3 = col[o4.w];
-            const double2 za = *reinterpret_cast<const double2*>(&s_z[warp][j]);
-            const double2 zb = *reinterpret_cast<const double2*>(&s_z[warp][j + 2]);
-            acc0 = fma(za.x, (double)f0, acc0);
-            acc1 = fma(za.y, (double)f1, acc1);
-            acc2 = fma(zb.x, (double)f2, acc2);
-            acc3 = fma(zb.y, (double)f3, acc3);
-        }
-        for (; j < k; ++j) acc0 = fma(s_z[warp][j], (double)col[s_off[warp][j]], acc0);
-        const double v = ((acc0 + acc1) + (acc2 + acc3)) + off;
+        const double v = hat_dot(col, s_z[warp], s_off[warp], k) + off;
         if (valid) {
             if (!XVAL && a.daily) a.daily[(size_t)q * nd + a.ob.day_of_pos[p0 + d]] = v;
             if (!XVAL && a.out_month) a.out_month[(size_t)q * D + d] = v;
@@ -287,8 +251,7 @@ static void gwr_fill(GwrArgs& a, Ctx& c, Batch& b, int mth) {
     a.k_fixed = 0; a.xv_self = nullptr; a.xv_out = nullptr; a.xv_nc = 0; a.xv_ci = 0; a.hat_off = nullptr;
 }
 
-int launch_gwr(Ctx& c, Batch& b, int mth, const double* pt_norm_override, int write_daily, double* out_month,
-               int kmax, int32_t* hat_k, int32_t* hat_idx, double* hat_z) {
+int launch_gwr(Ctx& c, Batch& b, int mth, const double* pt_norm_override, int write_daily, double* out_month) {
     if (b.npts <= 0) return TWXI_OK;
     GwrArgs a;
     gwr_fill(a, c, b, mth);
@@ -296,7 +259,6 @@ int launch_gwr(Ctx& c, Batch& b, int mth, const double* pt_norm_override, int wr
     a.pt_norm_single = pt_norm_override != nullptr;
     a.daily = write_daily ? b.daily : nullptr;
     a.out_month = out_month;
-    a.kmax = kmax; a.hat_k = hat_k; a.hat_idx = hat_idx; a.hat_z = hat_z;
     const long long items = (long long)b.npts * (mth >= 1 ? 1 : 12);
     const unsigned grid = (unsigned)((items + GWR_WARPS - 1) / GWR_WARPS);
     if (a.st.n > TWXI_GWR_PACKED_MIN_N) gwr_kernel<false, true><<<grid, GWR_THREADS, 0, c.stream>>>(a);
@@ -305,12 +267,12 @@ int launch_gwr(Ctx& c, Batch& b, int mth, const double* pt_norm_override, int wr
     return TWXI_OK;
 }
 
-int launch_gwr_hat_rows(Ctx& c, Batch& b, int kh, int32_t* hk, int32_t* hidx, double* hz, double* hoff) {
+int launch_gwr_hat_rows(Ctx& c, Batch& b, int mth, int kh, int32_t* hk, int32_t* hidx, double* hz, double* hoff) {
     if (b.npts <= 0) return TWXI_OK;
     GwrArgs a;
-    gwr_fill(a, c, b, 0);
+    gwr_fill(a, c, b, mth);
     a.kmax = kh; a.hat_k = hk; a.hat_idx = hidx; a.hat_z = hz; a.hat_off = hoff;
-    const long long items = (long long)b.npts * 12;
+    const long long items = (long long)b.npts * (mth >= 1 ? 1 : 12);
     const unsigned grid = (unsigned)((items + GWR_WARPS - 1) / GWR_WARPS);
     if (a.st.n > TWXI_GWR_PACKED_MIN_N) gwr_kernel<false, true, true><<<grid, GWR_THREADS, 0, c.stream>>>(a);
     else gwr_kernel<false, false, true><<<grid, GWR_THREADS, 0, c.stream>>>(a);

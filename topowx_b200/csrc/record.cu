@@ -3,12 +3,14 @@
 // twxi_interp_chunk holds a chunk's whole daily record on the device (f64 [ncell][ndays] per variable: 12.4 GB for a
 // 250 x 250 tile over 1948-2015).  Here the day-independent work (kNN, neighbour counts, kriging, GWR hat rows) runs once
 // at begin and the record is emitted in consecutive windows of any length; each window costs the GWR daily apply, the
-// Tmin >= Tmax fixer and the quantisation only.  The windows concatenate to exactly the bytes of twxi_interp_chunk:
-//  * apply  - gwr_kernel's day loop with the stored hat rows: same gathers, same order of the sums;
-//  * fixer  - fixer_kernel's sequential fixes over carry (the last 15 fixed days) + window + 15 unfixed look-ahead days:
-//             the fix of day x reads fixed days x-15..x-1 and unfixed days x..x+15, wherever the window boundaries are;
-//  * normals- the 1981-2010 (year, month) group means are reduced like fixer_kernel's (lane = day offset mod 32 in the
-//             group, warp_sum, accumulated year by year), with the lane partials of an unfinished group carried over.
+// Tmin >= Tmax fixer and the quantisation only.  The windows concatenate to exactly the bytes of twxi_interp_chunk, because
+// each step calls the helper its whole-record kernel calls (twxi_internal.cuh):
+//  * apply  - hat_dot with the stored hat rows, as gwr_kernel's day loop;
+//  * fixer  - fix_inverted over carry (the last 15 fixed days) + window + 15 unfixed look-ahead days, as fixer_kernel over
+//             the record: the fix of day x reads fixed days x-15..x-1 and unfixed days x..x+15, wherever the window
+//             boundaries are;
+//  * normals- group_lane_days over the window's part of each 1981-2010 (year, month) group, then warp_sum and the running
+//             sum over years as in fixer_kernel, with the lane partials of an unfinished group carried over.
 // A fixed day is valid (tavg -/+ half, half > 0), so only the fix of day 0 can find no valid day in its window; that
 // decision falls in the first window, which always computes days 1..15 as look-ahead.
 //
@@ -89,42 +91,10 @@ __global__ void __launch_bounds__(REC_THREADS, 4) tile_apply_kernel(ApplyArgs a)
     const double off = a.hoff[qm];
     const int p0 = a.p0[m];
     double* out = a.out + (size_t)q * a.wst + TAIL - a.w0;
-    for (int d0 = 0; d0 < D; d0 += 32) {                     // gwr_kernel's day loop, term for term
+    for (int d0 = 0; d0 < D; d0 += 32) {
         const int d = d0 + lane;
         const bool valid = d < D;
-        const float* col = a.obsT + p0 + (valid ? d : 0);
-        double acc0 = 0.0, acc1 = 0.0, acc2 = 0.0, acc3 = 0.0;
-        int j = 0;
-        for (; j + 7 < k; j += 8) {
-            const int4 o4 = *reinterpret_cast<const int4*>(&s_off[warp][j]);
-            const int4 o8 = *reinterpret_cast<const int4*>(&s_off[warp][j + 4]);
-            const float f0 = col[o4.x], f1 = col[o4.y], f2 = col[o4.z], f3 = col[o4.w];
-            const float f4 = col[o8.x], f5 = col[o8.y], f6 = col[o8.z], f7 = col[o8.w];
-            const double2 za = *reinterpret_cast<const double2*>(&s_z[warp][j]);
-            const double2 zb = *reinterpret_cast<const double2*>(&s_z[warp][j + 2]);
-            const double2 zc = *reinterpret_cast<const double2*>(&s_z[warp][j + 4]);
-            const double2 zd = *reinterpret_cast<const double2*>(&s_z[warp][j + 6]);
-            acc0 = fma(za.x, (double)f0, acc0);
-            acc1 = fma(za.y, (double)f1, acc1);
-            acc2 = fma(zb.x, (double)f2, acc2);
-            acc3 = fma(zb.y, (double)f3, acc3);
-            acc0 = fma(zc.x, (double)f4, acc0);
-            acc1 = fma(zc.y, (double)f5, acc1);
-            acc2 = fma(zd.x, (double)f6, acc2);
-            acc3 = fma(zd.y, (double)f7, acc3);
-        }
-        for (; j + 3 < k; j += 4) {
-            const int4 o4 = *reinterpret_cast<const int4*>(&s_off[warp][j]);
-            const float f0 = col[o4.x], f1 = col[o4.y], f2 = col[o4.z], f3 = col[o4.w];
-            const double2 za = *reinterpret_cast<const double2*>(&s_z[warp][j]);
-            const double2 zb = *reinterpret_cast<const double2*>(&s_z[warp][j + 2]);
-            acc0 = fma(za.x, (double)f0, acc0);
-            acc1 = fma(za.y, (double)f1, acc1);
-            acc2 = fma(zb.x, (double)f2, acc2);
-            acc3 = fma(zb.y, (double)f3, acc3);
-        }
-        for (; j < k; ++j) acc0 = fma(s_z[warp][j], (double)col[s_off[warp][j]], acc0);
-        const double v = ((acc0 + acc1) + (acc2 + acc3)) + off;
+        const double v = hat_dot(a.obsT + p0 + (valid ? d : 0), s_z[warp], s_off[warp], k) + off;
         if (valid) out[a.day_of_pos[p0 + d]] = v;
     }
 }
@@ -145,14 +115,13 @@ struct FixArgs {
     int16_t* qmax;
 };
 
-// The group sums of fixer_kernel for the part of group g inside the window: lane l adds the days at offsets = l mod 32 in
-// day order; the group's mean joins the running sum over years once its last day has been seen.
+// The part of group g inside the window (group_lane_days, as fixer_kernel sums whole groups); the group's mean joins the
+// running sum over years once its last day has been seen.
 __device__ __forceinline__ void group_part(const FixArgs& a, int g, int lane, const double* buf, double& part,
                                            double* acc) {
     const int gs = a.grp_start[g], len = a.grp_len[g];
     const int lo = max(gs, a.w0) - gs, hi = min(gs + len, a.w0 + a.nwin) - gs;
-    int o = lo + ((lane - lo) & 31);                          // first offset >= lo with o = lane (mod 32)
-    for (; o < hi; o += 32) part += buf[gs + o - a.w0 + TAIL];
+    group_lane_days(lo, hi, lane, [&](int o) { part += buf[gs + o - a.w0 + TAIL]; });
     if (gs + len <= a.w0 + a.nwin) {
         const double s = warp_sum(part);
         *acc += s / len;
@@ -174,34 +143,8 @@ __global__ void __launch_bounds__(128) tile_fix_kernel(FixArgs a) {
     if (st == TWXI_ST_OK) {
         if (lane < TAIL) { tmin[lane] = cmin[lane]; tmax[lane] = cmax[lane]; }
         __syncwarp();
-        const int wend = a.nwin + TAIL + a.la;                // columns computed: days up to w0 + nwin + la - 1
-        for (int d0 = 0; d0 < a.nwin && st == TWXI_ST_OK; d0 += 32) {
-            const int d = d0 + lane;
-            const bool inv = d < a.nwin && tmin[TAIL + d] >= tmax[TAIL + d];
-            unsigned mask = __ballot_sync(0xffffffffu, inv);
-            ninv += __popc(mask);
-            while (mask) {
-                const int x = TAIL + d0 + __ffs(mask) - 1;    // column of the day to fix
-                mask &= mask - 1;
-                const int dd = x - TAIL + lane;               // columns of days x-15 .. x+15
-                double diff = 0.0;
-                int ok = 0;
-                if (lane < 31 && a.w0 - TAIL + dd >= 0 && dd < wend) {
-                    const double lo = tmin[dd], hi = tmax[dd];
-                    if (lo < hi) { diff = hi - lo; ok = 1; }
-                }
-                const double sum = warp_sum(diff);
-                const int cnt = __popc(__ballot_sync(0xffffffffu, ok));
-                if (cnt == 0) { st = TWXI_ST_FIXER_EMPTY; break; }     // 'No valid tmin/tmax in window' :192
-                if (lane == 0) {
-                    const double tavg = (tmin[x] + tmax[x]) / 2.0;
-                    const double half = (sum / cnt) / 2.0;
-                    tmin[x] = tavg - half;
-                    tmax[x] = tavg + half;
-                }
-                __syncwarp();
-            }
-        }
+        // the window's days are columns TAIL .. TAIL + nwin - 1; columns up to nwin + TAIL + la - 1 are computed
+        ninv = fix_inverted(tmin, tmax, a.w0 - TAIL, TAIL, a.nwin, a.nwin + TAIL + a.la, lane, st);
     }
     const bool good = st == TWXI_ST_OK;
     if (good) {

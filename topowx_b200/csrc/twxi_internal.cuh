@@ -205,10 +205,10 @@ int launch_nngh_params(Ctx& c, Batch& b, const int32_t* norm_override, const int
                        int need_norm, int need_anom, int need_vario);
 int launch_krig(Ctx& c, Batch& b, int mth, const double* vario_override);
 int launch_vario_fit(Ctx& c, Batch& b, int mth);
-int launch_gwr(Ctx& c, Batch& b, int mth, const double* pt_norm_override, int write_daily,
-               double* out_month, int kmax, int32_t* hat_k, int32_t* hat_idx, double* hat_z);
-// hat rows of all 12 months with the arithmetic of launch_gwr: [ncell][12] k and offset, [ncell][12][kh] indices and z
-int launch_gwr_hat_rows(Ctx& c, Batch& b, int kh, int32_t* hk, int32_t* hidx, double* hz, double* hoff);
+int launch_gwr(Ctx& c, Batch& b, int mth, const double* pt_norm_override, int write_daily, double* out_month);
+// hat rows with the arithmetic of launch_gwr, of all 12 months (mth = 0: [npts][12] k and offset, [npts][12][kh] indices
+// and z) or of month mth ([npts], [npts][kh]); hoff may be null (no offset: b.mean is not read)
+int launch_gwr_hat_rows(Ctx& c, Batch& b, int mth, int kh, int32_t* hk, int32_t* hidx, double* hz, double* hoff);
 int launch_gwr_xval(Ctx& c, Batch& b, const int32_t* self, const int32_t* counts_host, int ncounts, double* out);
 int launch_station_points(Ctx& c, Batch& b, int npts, const int32_t* sidx);
 int launch_split3(cudaStream_t s, size_t n, const double* src, const int32_t* status, int per_point, double* a, double* b,
@@ -275,6 +275,92 @@ __device__ __forceinline__ int16_t quantize(double x) {
     const double r = rint(x * 100.0) / 100.0;
     const double v = r / (double)0.01f;
     return (int16_t)(int)v;
+}
+
+// The GWR daily value of one day before its offset: sum over j < k of z[j] * col[off[j]], col = the day's position in
+// the station-major obs table, off[j] = station * ndays.  Eight gathers in flight per pass, then four, then one, into
+// four accumulators.  z and off are 16-byte aligned rows (shared memory).  gwr_kernel and the day windows
+// (tile_apply_kernel) both use it, so their dailies are byte-identical.
+__device__ __forceinline__ double hat_dot(const float* col, const double* z, const int* off, int k) {
+    double acc0 = 0.0, acc1 = 0.0, acc2 = 0.0, acc3 = 0.0;
+    int j = 0;
+    for (; j + 7 < k; j += 8) {
+        const int4 o4 = *reinterpret_cast<const int4*>(&off[j]);
+        const int4 o8 = *reinterpret_cast<const int4*>(&off[j + 4]);
+        const float f0 = col[o4.x], f1 = col[o4.y], f2 = col[o4.z], f3 = col[o4.w];
+        const float f4 = col[o8.x], f5 = col[o8.y], f6 = col[o8.z], f7 = col[o8.w];
+        const double2 za = *reinterpret_cast<const double2*>(&z[j]);
+        const double2 zb = *reinterpret_cast<const double2*>(&z[j + 2]);
+        const double2 zc = *reinterpret_cast<const double2*>(&z[j + 4]);
+        const double2 zd = *reinterpret_cast<const double2*>(&z[j + 6]);
+        acc0 = fma(za.x, (double)f0, acc0);
+        acc1 = fma(za.y, (double)f1, acc1);
+        acc2 = fma(zb.x, (double)f2, acc2);
+        acc3 = fma(zb.y, (double)f3, acc3);
+        acc0 = fma(zc.x, (double)f4, acc0);
+        acc1 = fma(zc.y, (double)f5, acc1);
+        acc2 = fma(zd.x, (double)f6, acc2);
+        acc3 = fma(zd.y, (double)f7, acc3);
+    }
+    for (; j + 3 < k; j += 4) {
+        const int4 o4 = *reinterpret_cast<const int4*>(&off[j]);
+        const float f0 = col[o4.x], f1 = col[o4.y], f2 = col[o4.z], f3 = col[o4.w];
+        const double2 za = *reinterpret_cast<const double2*>(&z[j]);
+        const double2 zb = *reinterpret_cast<const double2*>(&z[j + 2]);
+        acc0 = fma(za.x, (double)f0, acc0);
+        acc1 = fma(za.y, (double)f1, acc1);
+        acc2 = fma(zb.x, (double)f2, acc2);
+        acc3 = fma(zb.y, (double)f3, acc3);
+    }
+    for (; j < k; ++j) acc0 = fma(z[j], (double)col[off[j]], acc0);
+    return (acc0 + acc1) + (acc2 + acc3);
+}
+
+// tmin_tmax_fixer (interp_tair.py:143-197) over one cell's series, one warp: column c holds record day day0 + c.  Fixes
+// the days at columns c0 .. c0 + n - 1 in day order: a day x with tmin >= tmax becomes tavg -/+ half the mean tmax - tmin
+// of the valid days at columns x-15 .. x+15 (tail = 15, :177-183), days fixed before it included; the window reads no
+// column before record day 0 and none from cend on.  Returns the number of such days; a day with no valid day in its
+// window sets st to TWXI_ST_FIXER_EMPTY ('No valid tmin/tmax in window' :192) and ends the fix.  fixer_kernel fixes the
+// whole record, tile_fix_kernel a window of it.
+__device__ __forceinline__ int fix_inverted(double* tmin, double* tmax, int day0, int c0, int n, int cend, int lane,
+                                            int& st) {
+    int ninv = 0;
+    for (int d0 = 0; d0 < n && st == TWXI_ST_OK; d0 += 32) {
+        const int d = d0 + lane;
+        const bool inv = d < n && tmin[c0 + d] >= tmax[c0 + d];
+        unsigned mask = __ballot_sync(0xffffffffu, inv);
+        ninv += __popc(mask);
+        while (mask) {
+            const int x = c0 + d0 + __ffs(mask) - 1;         // column of the day to fix
+            mask &= mask - 1;
+            const int dd = x - 15 + lane;                     // columns of days x-15 .. x+15
+            double diff = 0.0;
+            int ok = 0;
+            if (lane < 31 && day0 + dd >= 0 && dd < cend) {
+                const double lo = tmin[dd], hi = tmax[dd];
+                if (lo < hi) { diff = hi - lo; ok = 1; }
+            }
+            const double sum = warp_sum(diff);
+            const int cnt = __popc(__ballot_sync(0xffffffffu, ok));
+            if (cnt == 0) { st = TWXI_ST_FIXER_EMPTY; break; }
+            if (lane == 0) {
+                const double tavg = (tmin[x] + tmax[x]) / 2.0;
+                const double half = (sum / cnt) / 2.0;
+                tmin[x] = tavg - half;
+                tmax[x] = tavg + half;
+            }
+            __syncwarp();
+        }
+    }
+    return ninv;
+}
+
+// The days of a 1981-2010 (year, month) group that a lane adds to its partial sum: add(o) for the offsets lo <= o < hi in
+// the group with o = lane (mod 32), in day order.  fixer_kernel sums whole groups, tile_fix_kernel the part of a group
+// inside its window (carrying the partials to the next window), so the normals of both reduce in one order.
+template <typename F>
+__device__ __forceinline__ void group_lane_days(int lo, int hi, int lane, F&& add) {
+    for (int o = lo + ((lane - lo) & 31); o < hi; o += 32) add(o);   // first o >= lo with o = lane (mod 32)
 }
 
 // Haversine "a" term with the reference's operation order and no FMA contraction
