@@ -277,7 +277,8 @@ int twxi_interp_chunk(twxi_ctx* ctx_tmin, twxi_ctx* ctx_tmax, const double* wrk_
  * cycle through three sets of pinned buffers without ever calling the wait.  Submitting chunk t+1 guarantees nothing
  * about chunk t.  twxi_interp_chunk_wait(ctx_tmin, 0) only orders ctx_tmin's stream after the last copy (for event
  * timing); with host_sync != 0 it also blocks until everything submitted so far is complete.  The staging, the copy
- * streams and the events belong to ctx_tmin; one submitting thread per context pair.
+ * streams and the events belong to ctx_tmin; one submitting thread per context pair.  The wait also covers the
+ * asynchronous tile calls (twxi_tile_begin_async and the calls after it), which share this sequence of submissions.
  */
 int twxi_interp_chunk_async(twxi_ctx* ctx_tmin, twxi_ctx* ctx_tmax, const double* wrk_chk, int ny, int nx,
                             int16_t* tmin, int16_t* tmax, float* tmin_norm, float* tmax_norm,
@@ -334,6 +335,35 @@ int twxi_tile_end(twxi_ctx* ctx_tmin, twxi_ctx* ctx_tmax, float* tmin_norm, floa
  */
 int twxi_tile_days_mth(twxi_ctx* ctx_tmin, twxi_ctx* ctx_tmax, int ndays, int16_t* tmin, int16_t* tmax, int max_mth,
                        float* tmin_mth, float* tmax_mth, int32_t* nmth, int mem);
+
+/*
+ * The tile calls without the final wait, for drivers that hand each window to a writer while the next one is computed
+ * (the record counterpart of twxi_interp_chunk_async).  Each takes the arguments of its synchronous twin, checks them the
+ * same way before anything is enqueued, and computes the same bytes.  With host buffers:
+ *   twxi_tile_begin_async     stages wrk_chk host -> device on the h2d stream of ctx_tmin, like twxi_interp_chunk_async;
+ *   twxi_tile_days[_mth]_async, twxi_tile_end_async   stage their results on the device and copy them to the caller's
+ *                             buffers on ctx_tmin's copy stream, so the device -> host copy of window t overlaps the
+ *                             kernels of window t+1, and the copies of a tile's last windows overlap the kNN and kriging
+ *                             of the next tile's begin.
+ * Every successful such call takes the next slot of ctx_tmin's async sequence, which twxi_interp_chunk_async shares:
+ * chunks and tile calls count as one sequence of submissions.  The caller's buffers of submission t (wrk_chk of a begin,
+ * the outputs of a window or of an end) belong to the library until twxi_interp_chunk_wait(ctx_tmin, 1) returns, or until
+ * TWO further submissions have been made on the same context pair: submitting t+2 blocks the calling host thread until
+ * t's input has been read and t's results are complete in the caller's host buffers.  Three sets of pinned buffers
+ * therefore carry an endless stream.  Submitting t+1 guarantees nothing about t.  The buffers must be pinned for the
+ * overlap; pageable host buffers give the same results without it.
+ * The host-side tile state advances at submission: windows may be submitted back to back, *nmth is written before
+ * twxi_tile_days_mth_async returns, and twxi_tile_end_async closes the tile at once, so twxi_tile_begin_async of the next
+ * tile may follow immediately.  An error returns the code and message of the synchronous twin, takes no slot and leaves
+ * the tile as it was.  With device buffers (TWXI_MEM_DEVICE) the calls behave like their twins, which only enqueue, and
+ * take no slot.  Stage timing reports the slots of the synchronous calls.
+ */
+int twxi_tile_begin_async(twxi_ctx* ctx_tmin, twxi_ctx* ctx_tmax, const double* wrk_chk, int ny, int nx, int mem);
+int twxi_tile_days_async(twxi_ctx* ctx_tmin, twxi_ctx* ctx_tmax, int ndays, int16_t* tmin, int16_t* tmax, int mem);
+int twxi_tile_days_mth_async(twxi_ctx* ctx_tmin, twxi_ctx* ctx_tmax, int ndays, int16_t* tmin, int16_t* tmax,
+                             int max_mth, float* tmin_mth, float* tmax_mth, int32_t* nmth, int mem);
+int twxi_tile_end_async(twxi_ctx* ctx_tmin, twxi_ctx* ctx_tmax, float* tmin_norm, float* tmax_norm, float* tmin_se,
+                        float* tmax_se, int32_t* ninvalid, uint8_t* status, int mem);
 
 /*
  * Instrumentation for bench.py: number of kernels this library launched on the calling thread's contexts

@@ -77,6 +77,10 @@ def _load():
         "twxi_tile_days": (i32, [vp, vp, i32, vp, vp, i32]),
         "twxi_tile_days_mth": (i32, [vp, vp, i32, vp, vp, i32, vp, vp, vp, i32]),
         "twxi_tile_end": (i32, [vp, vp] + [vp] * 6 + [i32]),
+        "twxi_tile_begin_async": (i32, [vp, vp, vp, i32, i32, i32]),
+        "twxi_tile_days_async": (i32, [vp, vp, i32, vp, vp, i32]),
+        "twxi_tile_days_mth_async": (i32, [vp, vp, i32, vp, vp, i32, vp, vp, vp, i32]),
+        "twxi_tile_end_async": (i32, [vp, vp] + [vp] * 6 + [i32]),
         "twxi_measure_fp64_peak": (i32, [i32, vp, vp]),
     }
     for name, (res, args) in sig.items():

@@ -300,26 +300,54 @@ def _result_buffers(want, out, device, wrk_dev=None):
     return out, dev
 
 
-def tile_begin(ctx_tmin, ctx_tmax, wrk_chk):
+def _check_unpinned(bufs):
+    """Host torch tensors handed to an asynchronous call must be pinned: the copy stream reads or writes them after the call
+    returns."""
+    for k, b in bufs.items():
+        if b is not None and hasattr(b, "is_pinned") and not b.is_cuda and not b.is_pinned():
+            raise ValueError("%s is a torch host tensor that is not pinned: wait=False needs pinned host buffers "
+                             "(tensor.pin_memory())" % k)
+
+
+def _async_results(want, out, device, wait):
+    """_result_buffers for the tile calls.  wait=False with host results needs the caller's ``out``: the library owns those
+    buffers until two further submissions, so none is allocated behind the caller's back."""
+    if not wait:
+        if out is None and device is None:
+            raise ValueError("wait=False with host buffers needs `out`: the buffers belong to the library until two "
+                             "further submissions (or interp_chunk_wait), so the caller has to own them")
+        if out is not None:
+            _check_unpinned(out)
+    return _result_buffers(want, out, device)
+
+
+def tile_begin(ctx_tmin, ctx_tmax, wrk_chk, wait=True):
     """twxi_tile_begin: everything of interp_chunk that does not depend on the day (kNN, neighbour counts, kriging, GWR hat
-    rows) for the work chunk ``wrk_chk`` f8[32, ny, nx]; opens a tile on the context pair.  Returns (ny, nx)."""
+    rows) for the work chunk ``wrk_chk`` f8[32, ny, nx]; opens a tile on the context pair.  Returns (ny, nx).
+    ``wait=False`` submits it with twxi_tile_begin_async: a host ``wrk_chk`` (pinned, for the overlap) belongs to the
+    library until ``interp_chunk_wait`` returns or two further submissions have been made on the pair."""
     ny, nx = _check_wrk_chk(wrk_chk)
     if ctx_tmin.ndays != ctx_tmax.ndays:
         raise ValueError("tmin and tmax contexts hold observation records of different length")
-    check(lib.twxi_tile_begin(ctx_tmin.handle, ctx_tmax.handle, ptr(wrk_chk), ny, nx,
-                              MEM_DEVICE if _lib.is_device(wrk_chk) else MEM_HOST))
+    if not wait:
+        _check_unpinned(dict(wrk_chk=wrk_chk))
+    fn = lib.twxi_tile_begin if wait else lib.twxi_tile_begin_async
+    check(fn(ctx_tmin.handle, ctx_tmax.handle, ptr(wrk_chk), ny, nx, MEM_DEVICE if _lib.is_device(wrk_chk) else MEM_HOST))
     return ny, nx
 
 
-def tile_days(ctx_tmin, ctx_tmax, ndays, shape, out=None, device=None):
+def tile_days(ctx_tmin, ctx_tmax, ndays, shape, out=None, device=None, wait=True):
     """twxi_tile_days: the next ``ndays`` days of the open tile of ``shape`` = (ny, nx) -> {tmin, tmax} int16
     [ndays, ny, nx], byte-identical to the same days of interp_chunk.  ``out`` may carry the two buffers; otherwise they are
-    allocated on the host, or on the CUDA ``device`` (a torch device) when given."""
+    allocated on the host, or on the CUDA ``device`` (a torch device) when given.  ``wait=False`` submits the window with
+    twxi_tile_days_async; host buffers must then come in ``out`` (pinned torch tensors, or numpy arrays without overlap)
+    and belong to the library until ``interp_chunk_wait`` returns or two further submissions have been made on the pair."""
     ny, nx = shape
     want = dict(tmin=("int16", (int(ndays), ny, nx)), tmax=("int16", (int(ndays), ny, nx)))
-    out, dev = _result_buffers(want, out, device)
-    check(lib.twxi_tile_days(ctx_tmin.handle, ctx_tmax.handle, int(ndays), ptr(out["tmin"]), ptr(out["tmax"]),
-                             MEM_DEVICE if dev else MEM_HOST))
+    out, dev = _async_results(want, out, device, wait)
+    fn = lib.twxi_tile_days if wait else lib.twxi_tile_days_async
+    check(fn(ctx_tmin.handle, ctx_tmax.handle, int(ndays), ptr(out["tmin"]), ptr(out["tmax"]),
+             MEM_DEVICE if dev else MEM_HOST))
     return out
 
 
@@ -337,21 +365,23 @@ class MonthGroups(object):
         return int(np.searchsorted(ends, self.day0, side="right")), int(np.searchsorted(ends, self.day0 + n, side="right"))
 
 
-def tile_days_mth(ctx_tmin, ctx_tmax, ndays, shape, groups, out=None, device=None):
+def tile_days_mth(ctx_tmin, ctx_tmax, ndays, shape, groups, out=None, device=None, wait=True):
     """twxi_tile_days_mth: tile_days plus the monthly means of every month run that ends in the window ->
     {tmin, tmax} int16 [ndays, ny, nx], {tmin_mth, tmax_mth} float32 [nmth, ny, nx] and mth_groups, the (year, month,
     ndays) of each month, chronological.  ``groups`` is the MonthGroups of the tile (advanced by ndays); the month count
-    is exact, so ``out``'s month buffers must be [nmth, ny, nx]."""
+    is exact, so ``out``'s month buffers must be [nmth, ny, nx].  ``wait=False``: twxi_tile_days_mth_async, with the
+    buffer rules of tile_days; the month count and mth_groups are known at return."""
     ny, nx = shape
     g0, g1 = groups.completed(int(ndays))
     nm = g1 - g0
     want = dict(tmin=("int16", (int(ndays), ny, nx)), tmax=("int16", (int(ndays), ny, nx)),
                 tmin_mth=("float32", (nm, ny, nx)), tmax_mth=("float32", (nm, ny, nx)))
-    out, dev = _result_buffers(want, out, device)
+    out, dev = _async_results(want, out, device, wait)
     n = C.c_int32(-1)
-    check(lib.twxi_tile_days_mth(ctx_tmin.handle, ctx_tmax.handle, int(ndays), ptr(out["tmin"]), ptr(out["tmax"]), nm,
-                                 ptr(out["tmin_mth"]) if nm else None, ptr(out["tmax_mth"]) if nm else None, C.byref(n),
-                                 MEM_DEVICE if dev else MEM_HOST))
+    fn = lib.twxi_tile_days_mth if wait else lib.twxi_tile_days_mth_async
+    check(fn(ctx_tmin.handle, ctx_tmax.handle, int(ndays), ptr(out["tmin"]), ptr(out["tmax"]), nm,
+             ptr(out["tmin_mth"]) if nm else None, ptr(out["tmax_mth"]) if nm else None, C.byref(n),
+             MEM_DEVICE if dev else MEM_HOST))
     if n.value != nm:
         raise RuntimeError("twxi_tile_days_mth completed %d months, the days table %d" % (n.value, nm))
     groups.day0 += int(ndays)
@@ -359,15 +389,18 @@ def tile_days_mth(ctx_tmin, ctx_tmax, ndays, shape, groups, out=None, device=Non
     return out
 
 
-def tile_end(ctx_tmin, ctx_tmax, shape, out=None, device=None):
+def tile_end(ctx_tmin, ctx_tmax, shape, out=None, device=None, wait=True):
     """twxi_tile_end after the last day: {tmin_norm, tmax_norm, tmin_se, tmax_se, ninvalid, status} of interp_chunk
-    (normals recomputed from the fixed 1981-2010 dailies when a day was fixed); closes the tile."""
+    (normals recomputed from the fixed 1981-2010 dailies when a day was fixed); closes the tile.  ``wait=False``:
+    twxi_tile_end_async, with the buffer rules of tile_days; the tile is closed at return, so the next tile_begin may
+    follow at once."""
     ny, nx = shape
     want = dict(tmin_norm=("float32", (12, ny, nx)), tmax_norm=("float32", (12, ny, nx)),
                 tmin_se=("float32", (12, ny, nx)), tmax_se=("float32", (12, ny, nx)),
                 ninvalid=("int32", (ny, nx)), status=("uint8", (ny, nx)))
-    out, dev = _result_buffers(want, out, device)
-    check(lib.twxi_tile_end(ctx_tmin.handle, ctx_tmax.handle, ptr(out["tmin_norm"]), ptr(out["tmax_norm"]),
-                            ptr(out["tmin_se"]), ptr(out["tmax_se"]), ptr(out["ninvalid"]), ptr(out["status"]),
-                            MEM_DEVICE if dev else MEM_HOST))
+    out, dev = _async_results(want, out, device, wait)
+    fn = lib.twxi_tile_end if wait else lib.twxi_tile_end_async
+    check(fn(ctx_tmin.handle, ctx_tmax.handle, ptr(out["tmin_norm"]), ptr(out["tmax_norm"]),
+             ptr(out["tmin_se"]), ptr(out["tmax_se"]), ptr(out["ninvalid"]), ptr(out["status"]),
+             MEM_DEVICE if dev else MEM_HOST))
     return out

@@ -267,6 +267,57 @@ void AsyncOut::destroy() {
     *this = AsyncOut();
 }
 
+// The async calls of a pair (twxi_interp_chunk_async and the twxi_tile_*_async calls) share one sequence of two slots.
+// async_claim takes the next one: the call submitted two calls ago used it, so block the HOST until that call's input has
+// been read and its results are in the caller's buffers.  This is what makes "valid after two further submissions" true
+// (include/twxi.h).  The device still has the previous call queued, so no overlap is lost.
+static int async_claim(AsyncOut& ao) {
+    TWXI_TRY(ao.init());
+    const int sl = ao.slot;
+    if (ao.inflight_in[sl]) TWXI_CUDA(cudaEventSynchronize(ao.loaded[sl]));
+    ao.inflight_in[sl] = false;
+    if (ao.pending[sl]) TWXI_CUDA(cudaEventSynchronize(ao.copied[sl]));
+    ao.pending[sl] = false;
+    return TWXI_OK;
+}
+
+// The caller's work chunk into win[slot] on the h2d stream, ahead of the kernels; the compute stream s waits for it.
+static int async_load(AsyncOut& ao, cudaStream_t s, const double* wrk_chk, size_t bytes, const double** d_wrk) {
+    const int sl = ao.slot;
+    double* w;
+    TWXI_TRY(ao.win[sl].get((void**)&w, bytes));
+    if (ao.consumed[sl]) TWXI_CUDA(cudaStreamWaitEvent(ao.h2d, ao.unpacked[sl], 0));    // slot free again
+    TWXI_CUDA(cudaMemcpyAsync(w, wrk_chk, bytes, cudaMemcpyHostToDevice, ao.h2d));
+    TWXI_CUDA(cudaEventRecord(ao.loaded[sl], ao.h2d));
+    ao.inflight_in[sl] = true;
+    TWXI_CUDA(cudaStreamWaitEvent(s, ao.loaded[sl], 0));
+    *d_wrk = w;
+    return TWXI_OK;
+}
+
+// After the kernel that reads win[slot]: the h2d stream may overwrite it from here on.
+static int async_unpacked(AsyncOut& ao, cudaStream_t s) {
+    TWXI_CUDA(cudaEventRecord(ao.unpacked[ao.slot], s));
+    ao.consumed[ao.slot] = true;
+    return TWXI_OK;
+}
+
+// Ends a submission: with results, the copies of the staging d (stage[slot], written on the compute stream s) to the
+// caller's buffers o go on the copy stream; then the next call takes the other slot.
+static int async_next(AsyncOut& ao, cudaStream_t s, const ChunkOut* o = nullptr, const ChunkOut* d = nullptr) {
+    if (o) {
+        TWXI_CUDA(cudaEventRecord(ao.done, s));
+        TWXI_CUDA(cudaStreamWaitEvent(ao.copy, ao.done, 0));
+        TWXI_TRY(copy_out(ao.copy, *o, *d));
+        TWXI_CUDA(cudaEventRecord(ao.copied[ao.slot], ao.copy));
+        ao.pending[ao.slot] = true;
+        ao.last = ao.slot;
+    }
+    ao.slot ^= 1;
+    ++ao.submitted;
+    return TWXI_OK;
+}
+
 // Lay out the per-tile arrays of TileState in one allocation (256-byte aligned pieces).
 static int tile_alloc(TileState& t) {
     const size_t nc = (size_t)t.ncell, nh = (size_t)2 * nc * 12 * t.kh;
@@ -917,23 +968,8 @@ static int interp_chunk_impl(twxi_ctx* cmin, twxi_ctx* cmax, const double* wrk_c
     const bool acopy = async && host;                    // chunk and results travel on the copy streams
     AsyncOut& ao = cmin->async;
     if (acopy) {
-        TWXI_TRY(ao.init());
-        const int sl = ao.slot;
-        // The chunk submitted two calls ago used this slot.  Block the HOST until its work chunk has been read and its
-        // results are in the caller's buffers: this is what makes "valid after two further submissions" true
-        // (include/twxi.h).  The device still has the previous chunk queued, so no overlap is lost.
-        if (ao.inflight_in[sl]) TWXI_CUDA(cudaEventSynchronize(ao.loaded[sl]));
-        ao.inflight_in[sl] = false;
-        if (ao.pending[sl]) TWXI_CUDA(cudaEventSynchronize(ao.copied[sl]));
-        ao.pending[sl] = false;
-        double* w;
-        TWXI_TRY(ao.win[sl].get((void**)&w, wrk_bytes));
-        if (ao.consumed[sl]) TWXI_CUDA(cudaStreamWaitEvent(ao.h2d, ao.unpacked[sl], 0));    // slot free again
-        TWXI_CUDA(cudaMemcpyAsync(w, wrk_chk, wrk_bytes, cudaMemcpyHostToDevice, ao.h2d));
-        TWXI_CUDA(cudaEventRecord(ao.loaded[sl], ao.h2d));
-        ao.inflight_in[sl] = true;
-        TWXI_CUDA(cudaStreamWaitEvent(cmin->stream, ao.loaded[sl], 0));
-        d_wrk = w;
+        TWXI_TRY(async_claim(ao));
+        TWXI_TRY(async_load(ao, cmin->stream, wrk_chk, wrk_bytes, &d_wrk));
     } else if (host) {
         double* w;
         TWXI_TRY(cmin->scratch[2].get((void**)&w, wrk_bytes));
@@ -948,10 +984,7 @@ static int interp_chunk_impl(twxi_ctx* cmin, twxi_ctx* cmax, const double* wrk_c
     ta.begin(cmin->stream);
     TWXI_TRY(launch_unpack_chunk(cmin->stream, d_wrk, ny, nx, cmin->climdivs, cmin->n_climdivs, cmax->climdivs,
                                  cmax->n_climdivs, cmin->b, cmax->b));
-    if (acopy) {
-        TWXI_CUDA(cudaEventRecord(ao.unpacked[ao.slot], cmin->stream));
-        ao.consumed[ao.slot] = true;
-    }
+    if (acopy) TWXI_TRY(async_unpacked(ao, cmin->stream));
     TWXI_TRY(run_variable(*cmin, daily, ta));
     ta.mark(5);
     tb.begin(cmin->stream);
@@ -959,14 +992,7 @@ static int interp_chunk_impl(twxi_ctx* cmin, twxi_ctx* cmax, const double* wrk_c
     TWXI_TRY(launch_fixer(*cmin, *cmax, ncell, 1, daily ? 1 : 0, d));
     tb.mark(5);
     if (acopy) {
-        TWXI_CUDA(cudaEventRecord(ao.done, cmin->stream));
-        TWXI_CUDA(cudaStreamWaitEvent(ao.copy, ao.done, 0));
-        TWXI_TRY(copy_out(ao.copy, o, d));
-        TWXI_CUDA(cudaEventRecord(ao.copied[ao.slot], ao.copy));
-        ao.pending[ao.slot] = true;
-        ao.last = ao.slot;
-        ao.slot ^= 1;
-        ++ao.submitted;
+        TWXI_TRY(async_next(ao, cmin->stream, &o, &d));
     } else if (host) {
         TWXI_TRY(copy_out(cmin->stream, o, d));
     }
@@ -989,7 +1015,8 @@ int twxi_interp_chunk_async(twxi_ctx* cmin, twxi_ctx* cmax, const double* wrk_ch
                              status, mem, true);
 }
 
-int twxi_tile_begin(twxi_ctx* cmin, twxi_ctx* cmax, const double* wrk_chk, int ny, int nx, int mem) {
+// twxi_tile_begin[_async]: with `async` and a host wrk_chk, the chunk goes to the device through the pair's async slots.
+static int tile_begin_impl(twxi_ctx* cmin, twxi_ctx* cmax, const double* wrk_chk, int ny, int nx, int mem, bool async) {
     TWXI_ARG(wrk_chk, "null argument");
     TWXI_ARG(ny >= 1 && nx >= 1 && (long long)ny * nx <= (1 << 24), "bad chunk size");
     TWXI_TRY(check_pair(cmin, cmax, true));
@@ -999,9 +1026,14 @@ int twxi_tile_begin(twxi_ctx* cmin, twxi_ctx* cmax, const double* wrk_chk, int n
     const int ncell = ny * nx;
     TWXI_TRY(chunk_batches(*cmin, *cmax, ny, nx, false));
     const double* d_wrk = wrk_chk;
-    if (mem != TWXI_MEM_DEVICE) {
+    const bool acopy = async && mem != TWXI_MEM_DEVICE;
+    AsyncOut& ao = cmin->async;
+    const size_t wrk_bytes = (size_t)32 * ncell * 8;
+    if (acopy) {
+        TWXI_TRY(async_claim(ao));
+        TWXI_TRY(async_load(ao, cmin->stream, wrk_chk, wrk_bytes, &d_wrk));
+    } else if (mem != TWXI_MEM_DEVICE) {
         double* w;
-        const size_t wrk_bytes = (size_t)32 * ncell * 8;
         TWXI_TRY(cmin->scratch[2].get((void**)&w, wrk_bytes));
         TWXI_CUDA(cudaMemcpyAsync(w, wrk_chk, wrk_bytes, cudaMemcpyHostToDevice, cmin->stream));
         d_wrk = w;
@@ -1014,6 +1046,7 @@ int twxi_tile_begin(twxi_ctx* cmin, twxi_ctx* cmax, const double* wrk_chk, int n
     ta.begin(cmin->stream);
     TWXI_TRY(launch_unpack_chunk(cmin->stream, d_wrk, ny, nx, cmin->climdivs, cmin->n_climdivs, cmax->climdivs,
                                  cmax->n_climdivs, cmin->b, cmax->b));
+    if (acopy) TWXI_TRY(async_unpacked(ao, cmin->stream));
     TWXI_TRY(run_variable(*cmin, true, ta, &t, 0));
     ta.mark(5);
     tb.begin(cmin->stream);
@@ -1027,9 +1060,18 @@ int twxi_tile_begin(twxi_ctx* cmin, twxi_ctx* cmax, const double* wrk_chk, int n
     t.ndays = cmin->ob.ndays;
     t.next_day = 0;
     t.plain_days = false;
-    TWXI_TRY(finish(*cmin, mem));
+    if (acopy) TWXI_TRY(async_next(ao, cmin->stream));
+    if (!async) TWXI_TRY(finish(*cmin, mem));
     t.open = true;
     return TWXI_OK;
+}
+
+int twxi_tile_begin(twxi_ctx* cmin, twxi_ctx* cmax, const double* wrk_chk, int ny, int nx, int mem) {
+    return tile_begin_impl(cmin, cmax, wrk_chk, ny, nx, mem, false);
+}
+
+int twxi_tile_begin_async(twxi_ctx* cmin, twxi_ctx* cmax, const double* wrk_chk, int ny, int nx, int mem) {
+    return tile_begin_impl(cmin, cmax, wrk_chk, ny, nx, mem, true);
 }
 
 static int tile_check(twxi_ctx* cmin, twxi_ctx* cmax) {
@@ -1066,9 +1108,9 @@ static MonthSpan month_span(const Ctx& c, int w0, int w1) {
 }
 
 // One window of the open tile into o.q; with `mth`, also the monthly means of the runs that end in it into o.mth
-// (twxi_tile_days_mth).
-static int tile_days_impl(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, ChunkOut o, int mem,
-                          const MonthSpan* mth = nullptr) {
+// (twxi_tile_days_mth).  With `async` and host buffers the results leave through the pair's async slots.
+static int tile_days_impl(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, ChunkOut o, int mem, const MonthSpan* mth,
+                          bool async) {
     TileState& t = cmin->tile;
     WindowSpan w;
     w.w0 = t.next_day; w.nwin = ndays;
@@ -1085,8 +1127,11 @@ static int tile_days_impl(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, ChunkOut o,
         w.g1 = g + 1;
     }
     o.ncell = t.ncell; o.ndays = ndays; o.nmth = mth ? mth->nmth : 0;
+    const bool acopy = async && mem != TWXI_MEM_DEVICE;
+    AsyncOut& ao = cmin->async;
+    if (acopy) TWXI_TRY(async_claim(ao));
     ChunkOut d = o;
-    if (mem != TWXI_MEM_DEVICE) TWXI_TRY(stage_out(t.out, o, &d));
+    if (mem != TWXI_MEM_DEVICE) TWXI_TRY(stage_out(acopy ? ao.stage[ao.slot] : t.out, o, &d));
     StageTimer tm;
     tm.begin(cmin->stream, 3);                                // stage slots 3 (GWR daily apply) and 4 (fixer / quantise)
     TWXI_TRY(launch_tile_apply(cmin->stream, t, *cmin, *cmax, w));
@@ -1095,22 +1140,31 @@ static int tile_days_impl(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, ChunkOut o,
     tm.mark(5);
     tm.end(false);
     if (mth) TWXI_TRY(launch_tile_month(cmin->stream, t, *cmin, w, *mth, d.q[0], d.q[1], d.mth[0], d.mth[1]));
-    if (mem != TWXI_MEM_DEVICE) TWXI_TRY(copy_out(cmin->stream, o, d));
+    if (acopy) TWXI_TRY(async_next(ao, cmin->stream, &o, &d));
+    else if (mem != TWXI_MEM_DEVICE) TWXI_TRY(copy_out(cmin->stream, o, d));
     t.next_day = w1;
-    return finish(*cmin, mem);
+    return async ? TWXI_OK : finish(*cmin, mem);
 }
 
-int twxi_tile_days(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, int16_t* tmin, int16_t* tmax, int mem) {
+static int tile_days_call(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, int16_t* tmin, int16_t* tmax, int mem, bool async) {
     TWXI_TRY(tile_check(cmin, cmax));
     TWXI_ARG(tmin && tmax, "null argument");
     TWXI_ARG(ndays >= 1 && ndays <= cmin->tile.ndays - cmin->tile.next_day, "ndays must be 1 .. the days that remain");
     TWXI_CUDA(cudaSetDevice(cmin->device));
     cmin->tile.plain_days = true;
-    return tile_days_impl(cmin, cmax, ndays, ChunkOut{{tmin, tmax}}, mem);
+    return tile_days_impl(cmin, cmax, ndays, ChunkOut{{tmin, tmax}}, mem, nullptr, async);
 }
 
-int twxi_tile_days_mth(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, int16_t* tmin, int16_t* tmax, int max_mth,
-                       float* tmin_mth, float* tmax_mth, int32_t* nmth, int mem) {
+int twxi_tile_days(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, int16_t* tmin, int16_t* tmax, int mem) {
+    return tile_days_call(cmin, cmax, ndays, tmin, tmax, mem, false);
+}
+
+int twxi_tile_days_async(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, int16_t* tmin, int16_t* tmax, int mem) {
+    return tile_days_call(cmin, cmax, ndays, tmin, tmax, mem, true);
+}
+
+static int tile_days_mth_call(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, int16_t* tmin, int16_t* tmax, int max_mth,
+                              float* tmin_mth, float* tmax_mth, int32_t* nmth, int mem, bool async) {
     TWXI_TRY(tile_check(cmin, cmax));
     TWXI_ARG(tmin && tmax && nmth, "null argument");
     TWXI_ARG(ndays >= 1 && ndays <= cmin->tile.ndays - cmin->tile.next_day, "ndays must be 1 .. the days that remain");
@@ -1131,13 +1185,23 @@ int twxi_tile_days_mth(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, int16_t* tmin,
     TWXI_CUDA(cudaSetDevice(cmin->device));
     ChunkOut o{{tmin, tmax}};
     o.mth[0] = tmin_mth; o.mth[1] = tmax_mth;
-    TWXI_TRY(tile_days_impl(cmin, cmax, ndays, o, mem, &m));
+    TWXI_TRY(tile_days_impl(cmin, cmax, ndays, o, mem, &m, async));
     *nmth = m.nmth;
     return TWXI_OK;
 }
 
-int twxi_tile_end(twxi_ctx* cmin, twxi_ctx* cmax, float* tmin_norm, float* tmax_norm, float* tmin_se, float* tmax_se,
-                  int32_t* ninvalid, uint8_t* status, int mem) {
+int twxi_tile_days_mth(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, int16_t* tmin, int16_t* tmax, int max_mth,
+                       float* tmin_mth, float* tmax_mth, int32_t* nmth, int mem) {
+    return tile_days_mth_call(cmin, cmax, ndays, tmin, tmax, max_mth, tmin_mth, tmax_mth, nmth, mem, false);
+}
+
+int twxi_tile_days_mth_async(twxi_ctx* cmin, twxi_ctx* cmax, int ndays, int16_t* tmin, int16_t* tmax, int max_mth,
+                             float* tmin_mth, float* tmax_mth, int32_t* nmth, int mem) {
+    return tile_days_mth_call(cmin, cmax, ndays, tmin, tmax, max_mth, tmin_mth, tmax_mth, nmth, mem, true);
+}
+
+static int tile_end_call(twxi_ctx* cmin, twxi_ctx* cmax, float* tmin_norm, float* tmax_norm, float* tmin_se,
+                         float* tmax_se, int32_t* ninvalid, uint8_t* status, int mem, bool async) {
     TWXI_TRY(tile_check(cmin, cmax));
     TWXI_ARG(tmin_norm && tmax_norm && tmin_se && tmax_se && ninvalid && status, "null argument");
     TileState& t = cmin->tile;
@@ -1148,12 +1212,26 @@ int twxi_tile_end(twxi_ctx* cmin, twxi_ctx* cmax, float* tmin_norm, float* tmax_
     TWXI_CUDA(cudaSetDevice(cmin->device));
     const ChunkOut o{{nullptr, nullptr}, {tmin_norm, tmax_norm}, {tmin_se, tmax_se}, ninvalid, status, {nullptr, nullptr},
                      (size_t)t.ncell};
+    const bool acopy = async && mem != TWXI_MEM_DEVICE;
+    AsyncOut& ao = cmin->async;
+    if (acopy) TWXI_TRY(async_claim(ao));
     ChunkOut d = o;
-    if (mem != TWXI_MEM_DEVICE) TWXI_TRY(stage_out(t.out, o, &d));
+    if (mem != TWXI_MEM_DEVICE) TWXI_TRY(stage_out(acopy ? ao.stage[ao.slot] : t.out, o, &d));
     TWXI_TRY(launch_tile_end(cmin->stream, t, *cmin, d));
-    if (mem != TWXI_MEM_DEVICE) TWXI_TRY(copy_out(cmin->stream, o, d));
+    if (acopy) TWXI_TRY(async_next(ao, cmin->stream, &o, &d));
+    else if (mem != TWXI_MEM_DEVICE) TWXI_TRY(copy_out(cmin->stream, o, d));
     t.open = false;
-    return finish(*cmin, mem);
+    return async ? TWXI_OK : finish(*cmin, mem);
+}
+
+int twxi_tile_end(twxi_ctx* cmin, twxi_ctx* cmax, float* tmin_norm, float* tmax_norm, float* tmin_se, float* tmax_se,
+                  int32_t* ninvalid, uint8_t* status, int mem) {
+    return tile_end_call(cmin, cmax, tmin_norm, tmax_norm, tmin_se, tmax_se, ninvalid, status, mem, false);
+}
+
+int twxi_tile_end_async(twxi_ctx* cmin, twxi_ctx* cmax, float* tmin_norm, float* tmax_norm, float* tmin_se,
+                        float* tmax_se, int32_t* ninvalid, uint8_t* status, int mem) {
+    return tile_end_call(cmin, cmax, tmin_norm, tmax_norm, tmin_se, tmax_se, ninvalid, status, mem, true);
 }
 
 int twxi_interp_chunk_wait(twxi_ctx* cmin, int host_sync) {

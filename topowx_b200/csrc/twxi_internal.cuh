@@ -114,9 +114,10 @@ struct Scratch {
     void release() { if (p) cudaFree(p); p = nullptr; bytes = 0; }
 };
 
-// State of the asynchronous work-chunk call (twxi_interp_chunk_async), owned by the tmin context of the pair: results
-// leave the device on a copy stream from double-buffered staging, so that the device -> host copy of chunk t overlaps the
-// kernels of chunk t+1; work chunks go host -> device on their own stream into double-buffered staging, ahead of the kernels.
+// State of the asynchronous calls (twxi_interp_chunk_async and the twxi_tile_*_async calls, one sequence of submissions),
+// owned by the tmin context of the pair: results leave the device on a copy stream from double-buffered staging, so that
+// the device -> host copy of call t overlaps the kernels of call t+1; work chunks go host -> device on their own stream
+// into double-buffered staging, ahead of the kernels.
 struct AsyncOut {
     cudaStream_t copy = nullptr;
     cudaEvent_t done = nullptr;                   // compute stream: staging of the current call written
@@ -130,7 +131,7 @@ struct AsyncOut {
     bool inflight_in[2] = {false, false};         // loaded[slot] recorded and not yet waited for on the host
     Scratch win[2];
     int slot = 0, last = -1;
-    long long submitted = 0;                      // chunks submitted so far
+    long long submitted = 0;                      // calls submitted so far
     int init();
     void destroy();
 };

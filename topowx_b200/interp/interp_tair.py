@@ -321,18 +321,22 @@ class PtInterpTair(object):
         return _context.interp_chunk(self.ctx_tmin, self.ctx_tmax, wrk_chk, out=out, daily=not self.norms_only, wait=wait)
 
     def interp_chunk_wait(self):
-        '''Completion of the chunks submitted with interp_chunk(..., wait=False).'''
+        '''Completion of the chunks and record streams submitted with wait=False.'''
         _context.interp_chunk_wait(self.ctx_tmin)
 
-    def interp_chunk_stream(self, wrk_chk, months=False):
+    def interp_chunk_stream(self, wrk_chk, months=False, wait=True):
         '''
         New: interp_chunk over a long record in day windows (twxi_tile_begin / _days / _end).  The kriging and the GWR hat
         rows run once here; the returned RecordStream emits the record window by window, so the device holds one window of
         dailies instead of the whole record.  The windows concatenate to exactly the bytes interp_chunk returns.  One
         stream per context pair at a time: a new stream discards an open one.  months=True: every window also returns the
         monthly means of the months it completes (twxi_tile_days_mth), so one pass emits dailies, normals and monthly grids.
+        wait=False submits the begin, every window and the finish without waiting (twxi_tile_*_async): with host buffers
+        the windows and the finish need `out` (pinned), and each submission's buffers (wrk_chk's too) are valid once two
+        further submissions have been made on the pair, chunks included, or after interp_chunk_wait.  The stream is
+        closed at finish, so the next stream may start while this one's last copies drain.
         '''
-        return RecordStream(self, wrk_chk, months)
+        return RecordStream(self, wrk_chk, months, wait)
 
 
 class RecordStream(object):
@@ -342,23 +346,26 @@ class RecordStream(object):
     year of the remaining days; `finish()` returns the normals, se, ninvalid and status of interp_chunk and closes the
     stream.  Buffers live where wrk_chk lives (numpy on the host, torch tensors on its CUDA device).  With months=True
     each window's dict also holds tmin_mth, tmax_mth float32 [nmth, ny, nx] and mth_groups [(year, month, ndays)] of the
-    months that end in it (context.tile_days_mth).
+    months that end in it (context.tile_days_mth).  With wait=False every call only submits (see
+    PtInterpTair.interp_chunk_stream); `years()` allocates its buffers, so it needs wait=True or device buffers.
     '''
 
-    def __init__(self, pt_interp, wrk_chk, months=False):
+    def __init__(self, pt_interp, wrk_chk, months=False, wait=True):
         self.ctx_tmin, self.ctx_tmax = pt_interp.ctx_tmin, pt_interp.ctx_tmax
         self.days_meta = pt_interp.days
         self.device = wrk_chk.device if _lib.is_device(wrk_chk) else None
-        self.shape = _context.tile_begin(self.ctx_tmin, self.ctx_tmax, wrk_chk)
+        self.wait = wait
+        self.shape = _context.tile_begin(self.ctx_tmin, self.ctx_tmax, wrk_chk, wait=wait)
         self.groups = _context.MonthGroups(self.days_meta) if months else None
         self.day0 = 0
 
     def days(self, n, out=None):
         if self.groups is None:
-            o = _context.tile_days(self.ctx_tmin, self.ctx_tmax, n, self.shape, out=out, device=self.device)
+            o = _context.tile_days(self.ctx_tmin, self.ctx_tmax, n, self.shape, out=out, device=self.device,
+                                   wait=self.wait)
         else:
             o = _context.tile_days_mth(self.ctx_tmin, self.ctx_tmax, n, self.shape, self.groups, out=out,
-                                       device=self.device)
+                                       device=self.device, wait=self.wait)
         self.day0 += int(n)
         return o
 
@@ -370,7 +377,7 @@ class RecordStream(object):
             yield d0, self.days(n)
 
     def finish(self, out=None):
-        return _context.tile_end(self.ctx_tmin, self.ctx_tmax, self.shape, out=out, device=self.device)
+        return _context.tile_end(self.ctx_tmin, self.ctx_tmax, self.shape, out=out, device=self.device, wait=self.wait)
 
 
 class StationDataWrkChk(StationSerialDataDb):
