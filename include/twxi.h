@@ -237,6 +237,25 @@ int twxi_xval_anom(twxi_ctx* ctx, int npts, const int32_t* stn_idx, int n_counts
                    double* bias, double* mae, double* r2, uint8_t* status, int mem);
 
 /*
+ * a15 with its skill figures: the leave-one-out cross validation of the whole interpolation (kriged normal + GWR daily
+ * anomaly) that XvalTairOverall / step 24 run (optimize.py:547-604), for npts stations at once.  Points are stations of
+ * the context (stn_idx int32 [npts], context indices, as in twxi_xval_anom); each is left out of its own neighbour search
+ * together with any co-located station (rm_zero_dist = 1, optimize.py:569).  Neighbour search, smoothed counts, kriging
+ * and GWR run as in twxi_interp_points, so daily [npts][ndays], norms and se [npts][12] (float64) are byte-identical to
+ * what twxi_interp_points returns for the same stations and leave-outs.  `daily` may be NULL: the series are then built
+ * on the device, used for the statistics and never copied.
+ * bias, mae, r2 float64 [npts][12] compare, over every record day of month m, x = the interpolated daily value with
+ * y = the station's own observation (float32 widened to float64):
+ *     bias = mean(x - y), mae = mean(|x - y|), r2 = Pearson r^2 (= scipy.stats.linregress(x, y)[2]**2),
+ * the definitions of XvalTairAnom.run_xval (optimize.py:520-531) applied to the full series instead of the anomalies.
+ * NaN for a station whose status is not TWXI_ST_OK, for a month without a day in the record, and in r2 when either
+ * series is constant over the month (as np.corrcoef).  Failed stations keep fill values in daily / norms / se; an
+ * stn_idx outside the table gives TWXI_ST_TOO_FEW_STNS for that point.  TWXI_ERR_STATE before twxi_ctx_set_obs.
+ */
+int twxi_xval_overall(twxi_ctx* ctx, int npts, const int32_t* stn_idx, double* daily, double* norms, double* se,
+                      double* bias, double* mae, double* r2, uint8_t* status, int mem);
+
+/*
  * a11 / a12: Tmin and Tmax at ncells points with the Tmin>=Tmax fixer.  Replaces PtInterpTair.interp_pt
  * (interp_tair.py:526-592) incl. tmin_tmax_fixer (:143-197) and the 1981-2010 normals recomputation
  * (:583-590).  lst_tmin / lst_tmax [ncells][12] are the "tminMM"/"tmaxMM" LST planes; climdiv may be NULL

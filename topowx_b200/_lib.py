@@ -68,6 +68,7 @@ def _load():
         "twxi_gwr_hat": (i32, [vp, C.POINTER(Points), i32, vp, i32, vp, vp, vp, vp, i32]),
         "twxi_gwr_mth": (i32, [vp, C.POINTER(Points), i32, vp, vp, vp, vp, i32]),
         "twxi_xval_anom": (i32, [vp, i32, vp, i32, vp, vp, vp, vp, vp, i32]),
+        "twxi_xval_overall": (i32, [vp, i32] + [vp] * 8 + [i32]),
         "twxi_interp_points": (i32, [vp, C.POINTER(Points), vp, vp, vp, vp, vp, i32]),
         "twxi_interp_cells": (i32, [vp, vp, i32] + [vp] * 9 + [i32, i32, i32] + [vp] * 8 + [i32]),
         "twxi_interp_chunk": (i32, [vp, vp, vp, i32, i32] + [vp] * 8 + [i32]),

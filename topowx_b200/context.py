@@ -193,6 +193,20 @@ class TwxiContext(object):
         check(lib.twxi_xval_anom(self._h, n, ptr(stn_idx), nc, ptr(nnghs), ptr(bias), ptr(mae), ptr(r2), ptr(st), MEM_HOST))
         return bias, mae, r2, st
 
+    def xval_overall(self, stn_idx, daily=False):
+        """twxi_xval_overall: leave-one-out interpolation (kriged normal + GWR daily anomaly) at the stations ``stn_idx``
+        (context indices), each left out with any co-located station, and its skill against the station's own
+        observations.  Returns bias, mae, r2, norms, se [n, 12], status [n] and, with ``daily``, the dailies [n, ndays]
+        (otherwise None: they stay on the device)."""
+        stn_idx = np.ascontiguousarray(stn_idx, dtype=np.int32)
+        n = stn_idx.size
+        dly = np.empty((n, self.ndays)) if daily else None
+        bias, mae, r2, norms, se = (np.empty((n, 12)) for _ in range(5))
+        st = np.empty(n, dtype=np.uint8)
+        check(lib.twxi_xval_overall(self._h, n, ptr(stn_idx), ptr(dly), ptr(norms), ptr(se), ptr(bias), ptr(mae), ptr(r2),
+                                    ptr(st), MEM_HOST))
+        return bias, mae, r2, norms, se, st, dly
+
     def interp_points(self, lat, lon, elev, tdi, lst, rm_idx=None, rm_zero=False, daily=True):
         p, keep = self._points(lat, lon, elev=elev, tdi=tdi, lst=lst, rm_idx=rm_idx, rm_zero=rm_zero)
         n = p.npts

@@ -877,6 +877,47 @@ int twxi_interp_points(twxi_ctx* c, const twxi_points* pts, double* daily, doubl
     return finish(*c, mem);
 }
 
+int twxi_xval_overall(twxi_ctx* c, int npts, const int32_t* stn_idx, double* daily, double* norms, double* se,
+                      double* bias, double* mae, double* r2, uint8_t* status, int mem) {
+    TWXI_ARG(c && stn_idx && norms && se && bias && mae && r2 && status, "null argument");
+    TWXI_ARG(npts >= 0, "bad sizes");
+    if (!c->has_obs) { set_error("twxi_ctx_set_obs has not been called"); return TWXI_ERR_STATE; }
+    TWXI_CUDA(cudaSetDevice(c->device));
+    if (npts == 0) return TWXI_OK;
+    // the dailies are built on the device whether or not the caller takes them: the statistics read them there
+    TWXI_TRY(ensure_batch(*c, npts, default_k1(*c), true));
+    Batch& b = c->b;
+    b.n_rm = 1; b.rm_zero = 1; b.gy = b.gx = 0;                // optimize.py:569: rm_zero_dist_stns=True, stns_rm = the station
+    int32_t* d_idx;
+    TWXI_TRY(c->scratch[2].get((void**)&d_idx, (size_t)npts * 4));
+    TWXI_CUDA(cudaMemcpyAsync(d_idx, stn_idx, (size_t)npts * 4, cudaMemcpyDefault, c->stream));
+    TWXI_TRY(launch_station_points(*c, b, npts, d_idx));
+    StageTimer t;
+    t.begin(c->stream);
+    TWXI_TRY(run_variable(*c, true, t));
+    const size_t cnt = (size_t)npts * 12;
+    char* tmp;
+    TWXI_TRY(c->scratch[0].get((void**)&tmp, cnt * 8 * (2 + 3 + 3) + (size_t)npts));
+    double* d_norms = reinterpret_cast<double*>(tmp);
+    double* d_se = d_norms + cnt;
+    double* d_stats = d_se + cnt;                              // [npts][12][3]
+    double* d_split = d_stats + cnt * 3;                       // bias, mae, r2 [npts][12] each
+    uint8_t* st8 = reinterpret_cast<uint8_t*>(d_split + cnt * 3);
+    TWXI_TRY(launch_finalize_points(*c, b, b.daily, d_norms, d_se, nullptr, st8));
+    TWXI_TRY(launch_xval_stats(*c, b, d_idx, d_stats));
+    TWXI_TRY(launch_split3(c->stream, cnt, d_stats, b.status, 12, d_split, d_split + cnt, d_split + 2 * cnt));
+    t.mark(5);
+    TWXI_TRY(copy_out(c->stream, norms, d_norms, cnt));
+    TWXI_TRY(copy_out(c->stream, se, d_se, cnt));
+    TWXI_TRY(copy_out(c->stream, bias, d_split, cnt));
+    TWXI_TRY(copy_out(c->stream, mae, d_split + cnt, cnt));
+    TWXI_TRY(copy_out(c->stream, r2, d_split + 2 * cnt, cnt));
+    TWXI_TRY(copy_out(c->stream, status, st8, (size_t)npts));
+    if (daily) TWXI_TRY(copy_out(c->stream, daily, b.daily, (size_t)npts * c->ob.ndays));
+    t.end(false);
+    return finish(*c, mem);
+}
+
 static int check_pair(twxi_ctx* a, twxi_ctx* b, bool daily) {
     TWXI_ARG(a && b, "null ctx");
     TWXI_ARG(a->device == b->device, "tmin and tmax contexts must be on the same device");

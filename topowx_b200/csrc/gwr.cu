@@ -321,4 +321,63 @@ int launch_split3(cudaStream_t s, size_t n, const double* src, const int32_t* st
     return TWXI_OK;
 }
 
+// Skill of the full leave-one-out interpolation (twxi_xval_overall): bias, MAE and r^2 of the dailies that the production
+// gwr_kernel has written to `daily` against the held-out station's own observations, the definitions of
+// XvalTairAnom.run_xval (optimize.py:520-531) over every record day of the month.  One warp per (station, month),
+// month-major like gwr_kernel; lanes walk the month's positions p0 + d, so the station's obsT row is read coalesced.
+// Both series are summed as anomalies from the station's normal n_s: bias and MAE are the same, r^2 is invariant to the
+// shift, and the centred sums no longer cancel ~20 C means over the ~2 100 days a month has in a 68-year record.
+// A series that is constant over the month gives r^2 = NaN, as np.corrcoef does.
+constexpr int XSTAT_WARPS = 8;
+__global__ void __launch_bounds__(XSTAT_WARPS * 32) xval_stats_kernel(StnTable st, ObsTable ob, int npts,
+                                                                    const int32_t* self, const int32_t* status,
+                                                                    const double* daily, double* out) {
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const long long item = (long long)blockIdx.x * XSTAT_WARPS + warp;
+    if (item >= (long long)npts * 12) return;
+    const int q = (int)(item % npts), m = (int)(item / npts);
+    if (status[q] != TWXI_ST_OK) return;
+    const int s = self[q];
+    const size_t nd = (size_t)ob.ndays;
+    const double ns = st.norm[(size_t)m * st.n + s];
+    int p0 = 0, p1 = 0;
+#pragma unroll
+    for (int i = 0; i < 12; ++i)                              // constant indices: moff stays in the parameter space
+        if (i == m) { p0 = ob.moff[i]; p1 = ob.moff[i + 1]; }
+    const int D = p1 - p0;
+    const double* xq = daily + (size_t)q * nd;
+    const float* yq = ob.obsT + (size_t)s * nd + p0;
+    const double x0 = D > 0 ? xq[ob.day_of_pos[p0]] : 0.0;
+    const float y0 = D > 0 ? yq[0] : 0.0f;
+    bool xvar = false, yvar = false;
+    double sd = 0.0, sad = 0.0, sx = 0.0, sy = 0.0, sxx = 0.0, syy = 0.0, sxy = 0.0;
+    for (int d = lane; d < D; d += 32) {
+        const double xv = xq[ob.day_of_pos[p0 + d]];
+        const float yv = yq[d];
+        xvar |= xv != x0; yvar |= yv != y0;
+        const double x = xv - ns, y = (double)yv - ns;
+        const double dif = x - y;
+        sd += dif; sad += fabs(dif); sx += x; sy += y; sxx += x * x; syy += y * y; sxy += x * y;
+    }
+    // the reduction and the statistics of gwr_kernel's XVAL instance (twxi_xval_anom), term for term
+    sd = warp_sum(sd); sad = warp_sum(sad); sx = warp_sum(sx); sy = warp_sum(sy);
+    sxx = warp_sum(sxx); syy = warp_sum(syy); sxy = warp_sum(sxy);
+    const bool constant = !__any_sync(0xffffffffu, xvar) || !__any_sync(0xffffffffu, yvar);
+    if (lane == 0) {
+        const double n = (double)D;
+        const double cxy = sxy - sx * sy / n, cxx = sxx - sx * sx / n, cyy = syy - sy * sy / n;
+        const double r = cxy / sqrt(cxx * cyy);               // = scipy.stats.linregress(x, y)[2]
+        double* o = out + ((size_t)q * 12 + m) * 3;
+        o[0] = sd / n; o[1] = sad / n; o[2] = constant ? __longlong_as_double(0x7ff8000000000000ll) : r * r;
+    }
+}
+int launch_xval_stats(Ctx& c, Batch& b, const int32_t* self, double* out) {
+    if (b.npts <= 0) return TWXI_OK;
+    const long long items = (long long)b.npts * 12;
+    const unsigned grid = (unsigned)((items + XSTAT_WARPS - 1) / XSTAT_WARPS);
+    xval_stats_kernel<<<grid, XSTAT_WARPS * 32, 0, c.stream>>>(c.st, c.ob, b.npts, self, b.status, b.daily, out);
+    TWXI_LAUNCH_CHECK();
+    return TWXI_OK;
+}
+
 }  // namespace twxi

@@ -214,6 +214,9 @@ int launch_gwr_xval(Ctx& c, Batch& b, const int32_t* self, const int32_t* counts
 int launch_station_points(Ctx& c, Batch& b, int npts, const int32_t* sidx);
 int launch_split3(cudaStream_t s, size_t n, const double* src, const int32_t* status, int per_point, double* a, double* b,
                   double* c);
+// twxi_xval_overall: (bias, MAE, r^2) [npts][12][3] of b.daily against the own observations of the stations self[npts],
+// written for the points whose status is TWXI_ST_OK
+int launch_xval_stats(Ctx& c, Batch& b, const int32_t* self, double* out);
 int launch_build_dist_table(cudaStream_t s, int n, const double* lon, const double* lat, double* H);
 int launch_station_trig(cudaStream_t s, int n, const double* lon, const double* lat, double* lonrad,
                         double* latrad, double* coslat);

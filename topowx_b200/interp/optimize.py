@@ -60,6 +60,30 @@ class XvalTairOverall():
                                                                  daily=daily)
         return dly, norms, se, st
 
+    def run_xval(self, stn_id):
+        '''
+        Leave-one-out skill at one station: (bias, mae, r2), each [12], of the interpolated daily series against the
+        station's own observations (the statistics of XvalTairAnom.run_xval, optimize.py:520-531, over the full series).
+        '''
+        bias, mae, r2, norms, se, st = self.run_xval_batch([stn_id])
+        _raise_status(st[0])
+        return bias[0], mae[0], r2[0]
+
+    def run_xval_batch(self, stn_ids, daily=False):
+        '''
+        Batch form (new): leave-one-out interpolation and its skill at every station of `stn_ids` in one library call
+        (twxi_xval_overall: the statistics are computed on the device, and the daily series leave it only with `daily`).
+        Returns (bias, mae, r2, norms, se [n, 12], status [n]) and, with `daily`, the dailies [n, ndays] of
+        run_interp_batch; failed stations have NaN statistics and fill values elsewhere.
+        '''
+        ctx = self.interp_tair.gwr_tair.stn_slct.ctx
+        rows = np.array([self.stn_da.stn_idxs[s] for s in stn_ids], dtype=np.int64)
+        loc = ctx.local_of_db[rows]
+        if np.any(loc < 0):
+            raise KeyError("station is not among the selected (good) stations")
+        bias, mae, r2, norms, se, st, dly = ctx.xval_overall(loc.astype(np.int32), daily=daily)
+        return (bias, mae, r2, norms, se, st, dly) if daily else (bias, mae, r2, norms, se, st)
+
 
 def build_nstn_bandwidths(rng_min, rng_max, pct_step):
     '''
